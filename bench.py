@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- propagated frames/s of the label-propagation hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload = "davis2017_vos"): BASELINE config 2 -- VOS-style mask
 propagation on a synthetic DAVIS-2017-shaped clip: 480x854 frames, random-init ResNet-18
@@ -21,6 +21,9 @@ N > 1    : one process per GPU (torchrun), one clip per rank per step (weak scal
            NCCL all_gather inside the timed region; time = max over ranks.
 --impl reference : the oracle port of the reference's op sequence (torch CPU, all host
            threads) on a bounded sample of the same workload: one full-memory frame per step.
+--dump-outputs DIR : after the timed steps, what the last timed step returned to its caller, as DIR/<name>.npy
+           (float32 / float64; see dump_outputs).  The inputs are seeded, so two builds run with the same
+           arguments can be compared output for output.
 """
 import argparse
 import json
@@ -192,6 +195,28 @@ def build_inputs(device, seed):
     return feats, onehot
 
 
+DUMP_BYTES = 64 * 1000 * 1000          # all arrays of one --dump-outputs directory together
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Write each tensor of ``arrays`` (name -> tensor) as ``out_dir/<name>.npy``: float64 stays float64, every other
+    dtype becomes float32.  An array larger than its even share of DUMP_BYTES is replaced by a sample of its flattened
+    elements: the positions are drawn without replacement from a generator seeded with ``seed`` and kept in ascending
+    order, so they are the same in every run that dumps an array of that size."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays)) - 4096           # room for the .npy header
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+        n_max = share // a.itemsize
+        if a.size > n_max:
+            pos = np.random.default_rng(seed).choice(a.size, n_max, replace=False)
+            pos.sort()
+            a = a.reshape(-1)[pos]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 CONFIG_NOTES = dict(l2="inputs (420 MB features + 840 MB feature bank per clip) exceed the 126 MB L2",
                     clips_per_step_per_gpu=1, parallelism="videos sharded (one clip per GPU per step), results gathered "
                     "to rank 0")
@@ -317,6 +342,9 @@ def run_ours(args):
     frames_per_step = (T - 1) * world
     value = frames_per_step * args.steps / (ms / 1e3)
 
+    if args.dump_outputs and rank == 0:
+        # [T, 480, 854] object id per pixel of every frame; written before the e2e steps reuse the buffer
+        dump_outputs(args.dump_outputs, dict(masks=clip.masks))
     if args.profile:      # under ncu: kernels only, no e2e / CPU legs, no JSON line worth keeping
         if rank == 0:
             print(json.dumps(dict(profile_run=True, ms_per_step=ms / args.steps, k1_ms=k1_ms, plan=repr(clip.plan))))
@@ -622,7 +650,8 @@ def _sample_frames(n):
 def _cpu_sample(n_frames, warmup=1):
     """Reference CPU path (oracle port of the reference's op sequence, all host threads) on n_frames query frames of
     the bench clip.  The neighbourhood mask is built once per video by the reference (affinity_utils.py:75-112): its
-    build time is measured and charged at 1/63 per propagated frame.  Returns (frames/s, description)."""
+    build time is measured and charged at 1/63 per propagated frame.  Returns (frames/s, ms per frame, cores,
+    description, propagated labels of the last frame)."""
     from oracle import oracle as O        # the CPU legs of bench.py are the one place it runs the oracle
     cores = os.cpu_count()
     torch.set_num_threads(cores)
@@ -635,17 +664,17 @@ def _cpu_sample(n_frames, warmup=1):
         _cpu_frame(O, feats, labels, mask, ts[i % len(ts)])
     s = time.perf_counter()
     for t in ts:
-        _cpu_frame(O, feats, labels, mask, t)
+        out = _cpu_frame(O, feats, labels, mask, t)
     dt = time.perf_counter() - s + t_mask * len(ts) / (WORK["clip_frames"] - 1)
     entries = [min(t, WORK["precede_frames"]) + 1 for t in ts]
     desc = (f"{len(ts)} propagated frames of the same clip (query frames {ts}, memory entries {entries}: the clip's "
             f"mean is 18.0), oracle port of the reference op sequence (genuine functions are not on the GPU box), "
             f"torch CPU fp32, {cores} threads; the per-video mask build ({t_mask:.2f} s) is charged at 1/63 per frame")
-    return len(ts) / dt, dt / len(ts) * 1e3, cores, desc
+    return len(ts) / dt, dt / len(ts) * 1e3, cores, desc, out
 
 
 def cpu_baseline_sample(frames=3):
-    value, _, cores, desc = _cpu_sample(frames)
+    value, _, cores, desc, _ = _cpu_sample(frames)
     return dict(value=value, unit="frames/s", cores=cores, kind="port", sample=desc)
 
 
@@ -653,7 +682,9 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    value, ms, cores, desc = _cpu_sample(args.steps, warmup=max(1, args.warmup))
+    value, ms, cores, desc, labels = _cpu_sample(args.steps, warmup=max(1, args.warmup))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(labels=labels))       # [1, L, 60, 107] propagated soft labels
     print(json.dumps(dict(impl="reference", metric="propagated frames/sec", value=value, unit="frames/s",
                           n_gpus=int(os.environ.get("WORLD_SIZE", "1")), steps=args.steps, warmup=max(1, args.warmup),
                           ms_per_step=ms, higher_is_better=True, scaling="weak", vs_baseline=None,
@@ -674,7 +705,11 @@ def main():
     ap.add_argument("--profile", action="store_true", help="kernels only (for ncu): no e2e, no CPU baseline")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary block (BASELINE configs 3, 4, 5)")
     ap.add_argument("--only", nargs="*", default=None, help="secondary configs to run (cfg3 cfg4 cfg5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         if args.steps is None:
             args.steps = 3

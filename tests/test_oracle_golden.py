@@ -139,21 +139,6 @@ def test_memory_multiset_duplicates_frame0():
     assert O.memory_frames(3, 5, with_first=False) == [0, 1, 2]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present")
-def test_live_reference_agrees_with_port():
-    """In the build container also execute the genuine function on fresh seeded inputs."""
-    from oracle import ref_loader
-    ref = ref_loader.load_functions()
-    g = torch.Generator().manual_seed(99)
-    q = torch.randn(1, 48, 11, 13, generator=g)
-    k = torch.randn(1, 48, 3, 11, 13, generator=g)
-    v = torch.rand(1, 4, 3, 11, 13, generator=g)
-    m = ref.spatial_neighbor(1, 11, 13, neighbor_range=8, device="cpu", dtype=torch.float32)
-    want = ref.masked_attention_efficient(q, k, v, m, temperature=0.07, topk=10, step=50)
-    got = O.propagate_port(q, k, v, mask=O.neighbor_mask(11, 13, 8), temperature=0.07, topk=10, step=50)
-    assert torch.allclose(got, want, atol=2e-6, rtol=0)
-
-
 @pytest.mark.parametrize("mode", ["first", "strided"])
 def test_tapvid_metrics_match_reference(golden_dir, mode):
     d = _load(golden_dir, "tapvid_metrics.npz")
