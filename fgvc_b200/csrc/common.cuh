@@ -107,12 +107,19 @@ struct TopK {
   }
   // caller guarantees x > thr().  Select form of the sorted insert: K compares, then every slot
   // takes its left neighbour, the new element or itself (equal values keep arrival order).
+  // The last slot is written without its compare (x > v[K-1] holds): with the compare in the
+  // expression, nvcc 12.9 compiled TopK<4> in gather_labels_kernel to take the new index but keep
+  // the old value there, which dropped the K-th winner (tests/test_gpu_label_kernels.py, K = 4).
   __device__ __forceinline__ void push(float x, int i) {
     bool c[K];
 #pragma unroll
     for (int j = 0; j < K; ++j) c[j] = x > v[j];
+    if (K > 1) {
+      v[K - 1] = c[K - 2] ? v[K - 2] : x;
+      id[K - 1] = c[K - 2] ? id[K - 2] : i;
+    }
 #pragma unroll
-    for (int j = K - 1; j > 0; --j) {
+    for (int j = K - 2; j > 0; --j) {
       v[j] = c[j - 1] ? v[j - 1] : (c[j] ? x : v[j]);
       id[j] = c[j - 1] ? id[j - 1] : (c[j] ? i : id[j]);
     }

@@ -224,7 +224,9 @@ gather_chain_kernel(const float* __restrict__ cw, const int32_t* __restrict__ cr
   const int per = (n_pix + gridDim.x - 1) / gridDim.x;
   const int q_lo = blockIdx.x * per, q_hi = min(n_pix, q_lo + per);
   // single-pass slices (the usual case: the grid is sized for it): the label-independent (weight, row) pairs of job
-  // j + 1 are fetched into registers while job j is gathered, so the only loads after a grid barrier are the label rows
+  // j + 1 are fetched into registers while job j is gathered, so the only loads after a grid barrier are the label rows.
+  // With L <= 4 (one float4 per label row) the launch sizes the grid at ceil(n_pix / 64) CTAs or fewer, so every map
+  // of more than 32 pixels takes the multi-pass branch; so does any map of more than 32 x (resident CTAs) pixels.
   const bool one_pass = q_hi - q_lo <= CH_Q;
   constexpr int PRE = (CH_Q * K + 255) / 256;
   float pw[PRE];
