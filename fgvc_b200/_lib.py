@@ -36,6 +36,12 @@ class Job(ctypes.Structure):
     _fields_ = [("q_slot", c_int32), ("mem_begin", c_int32), ("mem_end", c_int32), ("out_slot", c_int32)]
 
 
+class Lane(ctypes.Structure):
+    """fgvc_lane: one recurrence of fgvc_point_clip_tail_lanes (offsets in floats)"""
+    _fields_ = [("job_begin", c_int32), ("job_end", c_int32), ("L", c_int32), ("Lp", c_int32),
+                ("lab_offset", c_int64), ("coord_offset", c_int64)]
+
+
 P = c_void_p
 I = c_int32
 L64 = c_int64
@@ -70,6 +76,7 @@ SIGNATURES = {
     "fgvc_mask_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, P, P, P, P, L64, P]),
     "fgvc_point_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, I, P, P, P, L64, P]),
     "fgvc_point_clip_tail_shared": (I, [P, P, I, P, P, P, I, I, P, I, I, F, I, P, I, I, I, I, I, P, P, P, L64, P]),
+    "fgvc_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, P, I, P, I, I, F, I, P, I, I, I, P, P, P, L64, P]),
     "fgvc_c2f_scratch_elems": (L64, [I, I]),
     "fgvc_c2f_propagate": (I, [P, I, I, I, I, I, P, I, I, I, P, P, P, P, I, I, I, I, F, P, I, P, P, P, L64, I, P]),
 }

@@ -67,10 +67,20 @@ extern "C" int fgvc_mask_clip_tail(const float* topk_val, const int32_t* topk_id
                             reinterpret_cast<uint32_t*>(scratch_minmax), masks, st);
 }
 
+// Lowest out_slot of jobs [job_begin, job_end) when their out_slots run consecutively up (a forward track) or down (a
+// track run backwards in time), else -1.  The K3 launch of a point tail covers the slots [lowest, lowest + n).
+static int consecutive_slots(const fgvc_job* jobs_host, int job_begin, int job_end) {
+  const int s0 = jobs_host[job_begin].out_slot, n = job_end - job_begin;
+  const int dir = (n > 1 && jobs_host[job_begin + 1].out_slot < s0) ? -1 : 1;
+  for (int j = job_begin; j < job_end; ++j)
+    if (jobs_host[j].out_slot != s0 + dir * (j - job_begin)) return -1;
+  return dir > 0 ? s0 : s0 - (n - 1);
+}
+
 // Point tracking tail: the gather chain over jobs [job_begin, job_end) with an NCHW copy of every
 // propagated frame into maps_nchw[slot][L][H*W], then ONE K3 launch (fused up-sample / soft-argmax)
 // over all (frame, point) maps of the range: coords[slot][L][2].  The out_slots of the range must
-// be consecutive (they are frame indices).
+// be consecutive (they are frame indices), ascending or descending.
 static int point_clip_tail_impl(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
                                     const fgvc_job* jobs_dev, const fgvc_job* jobs_host, int32_t job_begin,
                                     int32_t job_end, const int32_t* mem_label_slot, int32_t H, int32_t W,
@@ -80,9 +90,8 @@ static int point_clip_tail_impl(const float* topk_val, const int32_t* topk_idx, 
   FGVC_CHECK_ARG(jobs_dev && jobs_host && maps_nchw && coords && lab_bank, "fgvc_point_clip_tail: null pointer");
   FGVC_CHECK_ARG(job_end > job_begin, "fgvc_point_clip_tail: empty job range");
   const int n_pix = H * W;
-  const int slot0 = jobs_host[job_begin].out_slot;
-  for (int j = job_begin; j < job_end; ++j)
-    FGVC_CHECK_ARG(jobs_host[j].out_slot == slot0 + (j - job_begin), "fgvc_point_clip_tail: out_slots must be consecutive");
+  const int slot0 = consecutive_slots(jobs_host, job_begin, job_end);
+  FGVC_CHECK_ARG(slot0 >= 0, "fgvc_point_clip_tail: out_slots must be consecutive");
   FGVC_CHECK_ARG(pair_ref == nullptr || chain_ws != nullptr, "fgvc_point_clip_tail_shared: needs the chain workspace");
   if (chain_ws != nullptr && (job_end - job_begin > 1 || pair_ref != nullptr)) {
     cudaStream_t st = (cudaStream_t)stream;
@@ -130,4 +139,48 @@ extern "C" int fgvc_point_clip_tail_shared(const float* topk_val, const int32_t*
   return point_clip_tail_impl(topk_val, topk_idx, K, 1, jobs_dev, jobs_host, job_begin, job_end, mem_label_slot, H, W,
                               temperature, flags, lab_bank, Lp, L, out_h, out_w, coord_topk, maps_nchw, coords, chain_ws,
                               chain_ws_bytes, pair_ref, stream);
+}
+
+// Several independent point tails of one clip (bidirectional tracking: the forward and the backward track of every
+// point group), each lane bit for bit its own point_clip_tail_impl: one multi-lane gather chain for all of them
+// (gather.cu), then per lane the NCHW copies and one K3 launch -- bandwidth work, where one launch per lane costs
+// nothing worth saving.
+extern "C" int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
+                                          const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
+                                          const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int32_t n_lanes,
+                                          const int32_t* mem_label_slot, int32_t H, int32_t W, float temperature,
+                                          int32_t flags, float* lab_bank, int32_t out_h, int32_t out_w,
+                                          int32_t coord_topk, float* maps_nchw, float* coords, void* chain_ws,
+                                          int64_t chain_ws_bytes, void* stream) {
+  FGVC_CHECK_ARG(topk_val && topk_idx && jobs_dev && jobs_host && lanes_dev && lanes_host && mem_label_slot && lab_bank &&
+                     maps_nchw && coords && chain_ws, "fgvc_point_clip_tail_lanes: null pointer");
+  FGVC_CHECK_ARG(K >= 1 && K <= 16, "fgvc_point_clip_tail_lanes: topk=%d not in [1,16]", K);
+  FGVC_CHECK_ARG(n_lanes >= 1 && H > 0 && W > 0 && groups >= 1, "fgvc_point_clip_tail_lanes: bad sizes");
+  FGVC_CHECK_ARG(pair_ref == nullptr || groups == 1, "fgvc_point_clip_tail_lanes: shared lists need groups == 1");
+  FGVC_CHECK_ARG(temperature > 0.f, "fgvc_point_clip_tail_lanes: temperature must be > 0");
+  for (int i = 0; i < n_lanes; ++i) {
+    const fgvc_lane& ln = lanes_host[i];
+    FGVC_CHECK_ARG(ln.job_begin >= 0 && ln.job_end > ln.job_begin, "fgvc_point_clip_tail_lanes: lane %d is empty", i);
+    FGVC_CHECK_ARG(ln.L > 0 && ln.Lp >= ln.L && ln.Lp % 4 == 0 && ln.lab_offset >= 0 && ln.lab_offset % 4 == 0 &&
+                       ln.coord_offset >= 0, "fgvc_point_clip_tail_lanes: bad label sizes or offsets in lane %d", i);
+    FGVC_CHECK_ARG(consecutive_slots(jobs_host, ln.job_begin, ln.job_end) >= 0,
+                   "fgvc_point_clip_tail_lanes: out_slots of lane %d must be consecutive", i);
+  }
+  const int n_pix = H * W;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = launch_gather_chain_lanes(topk_val, topk_idx, K, groups, jobs_dev, lanes_dev, lanes_host, n_lanes,
+                                     mem_label_slot, pair_ref, n_pix, temperature, flags, lab_bank, chain_ws,
+                                     chain_ws_bytes, st);
+  if (rc) return rc;
+  for (int i = 0; i < n_lanes; ++i) {
+    const fgvc_lane& ln = lanes_host[i];
+    rc = launch_labels_to_nchw_jobs(lab_bank + ln.lab_offset, jobs_dev, ln.job_begin, ln.job_end, ln.Lp, ln.L, n_pix,
+                                    maps_nchw, st);
+    if (rc) return rc;
+    const int slot0 = consecutive_slots(jobs_host, ln.job_begin, ln.job_end);
+    rc = fgvc_heatmap_coords(maps_nchw + (int64_t)slot0 * ln.L * n_pix, (ln.job_end - ln.job_begin) * ln.L, H, W, out_h,
+                             out_w, coord_topk, coords + ln.coord_offset + (int64_t)slot0 * ln.L * 2, stream);
+    if (rc) return rc;
+  }
+  return FGVC_OK;
 }

@@ -167,6 +167,10 @@ int64_t chain_workspace_bytes(int n_jobs, int n_pix, int K);
 int launch_gather_chain(const float* tv, const int32_t* ti, int K, int groups, const fgvc_job* jobs, int job_begin,
                         int job_end, const int32_t* mem_label, const int32_t* pair_ref, int n_pix, float temperature,
                         int flags, float* lab, int Lp, void* ws, int64_t ws_bytes, cudaStream_t st);
+int launch_gather_chain_lanes(const float* tv, const int32_t* ti, int K, int groups, const fgvc_job* jobs,
+                              const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int n_lanes,
+                              const int32_t* mem_label, const int32_t* pair_ref, int n_pix, float temperature, int flags,
+                              float* lab, void* ws, int64_t ws_bytes, cudaStream_t st);
 int launch_labels_to_nchw_jobs(const float* lab, const fgvc_job* jobs_dev, int job_begin, int job_end, int Lp, int L,
                                int n_pix, float* maps_nchw, cudaStream_t st);
 void packed_tile_shape(int H, int W, int reach, int jobs_per_tile, int* QH, int* QW, int* BH, int* ncta);

@@ -323,37 +323,203 @@ gather_chain_kernel(const float* __restrict__ cw, const int32_t* __restrict__ cr
   }
 }
 
+// ------------------------------------------------------------------ the multi-lane gather chain
+// Several independent recurrences of one clip (lanes: the forward and backward tracks of every point group) in ONE
+// cooperative kernel.  Step s gathers job s of every lane that is still running, then all CTAs meet at the grid
+// barrier, so a clip pays the longest lane's length in barriers instead of the sum over its lanes.  Each CTA owns the
+// same fixed query slice in every lane; per (query, channel) the FMA sequence is gather_chain_kernel's, so every lane
+// is bit for bit the single-lane chain over its jobs.  The (weight, row) pairs of all jobs come from ONE
+// gather_weights_kernel launch over the job range [job_base, ...) holding every lane; rows are relative to the lane's
+// bank.  In the one-pass branch the CTA walks its work items (step, lane) in order and copies the pairs of the next
+// item into a second shared buffer (cp.async, no registers held) while it gathers the current one: they are
+// label-independent, so this holds across barriers and lanes, and the shared memory does not grow with the lanes.
+
+// first lane >= l that still runs at step s (n_lanes: none)
+__device__ __forceinline__ int next_lane(const fgvc_lane* __restrict__ lanes, int n_lanes, int s, int l) {
+  while (l < n_lanes && __ldg(&lanes[l].job_end) - __ldg(&lanes[l].job_begin) <= s) ++l;
+  return l;
+}
+
+// index in the chain workspace of the (weight, row) pair of query q of job s of lane l
+template <int K>
+__device__ __forceinline__ int64_t lane_pairs(const fgvc_lane* __restrict__ lanes, int l, int s, int job_base, int n_pix,
+                                              int q) {
+  return ((int64_t)(__ldg(&lanes[l].job_begin) + s - job_base) * n_pix + q) * K;
+}
+
+// queries of a lane-chain CTA's one-pass slice.  The kernel is bounded to 2 resident CTAs per SM, where it needs no
+// spill at any K (64 to 88 registers: the K label rows of a query are loaded at once); at 2 to 4 CTAs per SM a
+// slice of 64 keeps 128 x 128 maps in the one-pass branch.
+constexpr int CH_QL = 64;
+
+// 4-byte global -> shared copy that holds no register until it lands (cp.async, sm_80+)
+__device__ __forceinline__ void cp_async4(void* smem, const void* gmem) {
+  const unsigned int d = (unsigned int)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(gmem) : "memory");
+}
+
+template <int K>
+__global__ void __launch_bounds__(256, 2)
+gather_chain_lanes_kernel(const float* __restrict__ cw, const int32_t* __restrict__ crow,
+                          const fgvc_job* __restrict__ jobs, int job_base, const fgvc_lane* __restrict__ lanes,
+                          int n_lanes, int n_steps, int n_pix, float* lab, unsigned int* barrier) {
+  // two buffers of (weight, row) pairs: the current work item's and the next one's, in flight
+  __shared__ float sw[2][CH_QL][K];
+  __shared__ int srow[2][CH_QL][K];
+  const int tid = threadIdx.x;
+  const int per = (n_pix + gridDim.x - 1) / gridDim.x;
+  const int q_lo = blockIdx.x * per, q_hi = min(n_pix, q_lo + per);
+  const bool one_pass = q_hi - q_lo <= CH_QL;
+  const int nq1 = max(q_hi - q_lo, 0);
+  int l = next_lane(lanes, n_lanes, 0, 0), b = 0;
+  if (one_pass && l < n_lanes) {
+    const int64_t o = lane_pairs<K>(lanes, l, 0, job_base, n_pix, q_lo);
+    for (int i = tid; i < nq1 * K; i += 256) {
+      (&sw[0][0][0])[i] = __ldg(cw + o + i);
+      (&srow[0][0][0])[i] = __ldg(crow + o + i);
+    }
+    __syncthreads();
+  }
+  for (int s = 0; s < n_steps; ++s) {
+    for (; l < n_lanes; l = next_lane(lanes, n_lanes, s, l + 1)) {
+      const int l4n = __ldg(&lanes[l].Lp) / 4;
+      float4* bank = reinterpret_cast<float4*>(lab + __ldg(&lanes[l].lab_offset));
+      const int out_slot = jobs[__ldg(&lanes[l].job_begin) + s].out_slot;
+      if (one_pass) {
+        // the next work item: the next running lane of this step, else the first lane of the next step
+        int ns = s, nl = next_lane(lanes, n_lanes, s, l + 1);
+        if (nl == n_lanes) {
+          ns = s + 1;
+          nl = ns < n_steps ? next_lane(lanes, n_lanes, ns, 0) : n_lanes;
+        }
+        const bool more = nl < n_lanes;
+        if (more) {
+          const int64_t o = lane_pairs<K>(lanes, nl, ns, job_base, n_pix, q_lo);
+          for (int i = tid; i < nq1 * K; i += 256) {
+            cp_async4(&sw[b ^ 1][0][0] + i, cw + o + i);
+            cp_async4(&srow[b ^ 1][0][0] + i, crow + o + i);
+          }
+          asm volatile("cp.async.commit_group;" ::: "memory");
+        }
+        for (int i = tid; i < nq1 * l4n; i += 256) {
+          const int q = i / l4n, c = i - q * l4n;
+          float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+          for (int k = 0; k < K; ++k) {
+            const float w = sw[b][q][k];
+            if (w != 0.f) {
+              const float4 v = __ldcg(bank + (int64_t)srow[b][q][k] * l4n + c);   // may have been written by another CTA
+              acc.x = fmaf(w, v.x, acc.x); acc.y = fmaf(w, v.y, acc.y);
+              acc.z = fmaf(w, v.z, acc.z); acc.w = fmaf(w, v.w, acc.w);
+            }
+          }
+          bank[((int64_t)out_slot * n_pix + q_lo + q) * l4n + c] = acc;
+        }
+        if (more) {
+          asm volatile("cp.async.wait_all;" ::: "memory");
+          __syncthreads();                             // the next item's pairs have landed, this item's are done
+          b ^= 1;
+        }
+      } else {
+        const int64_t o0 = lane_pairs<K>(lanes, l, s, job_base, n_pix, 0);
+        for (int q0 = q_lo; q0 < q_hi; q0 += CH_QL) {
+          const int nq = min(CH_QL, q_hi - q0);
+          __syncthreads();
+          for (int i = tid; i < nq * K; i += 256) {
+            const int64_t o = o0 + (int64_t)q0 * K + i;
+            (&sw[0][0][0])[i] = __ldg(cw + o);
+            (&srow[0][0][0])[i] = __ldg(crow + o);
+          }
+          __syncthreads();
+          for (int i = tid; i < nq * l4n; i += 256) {
+            const int q = i / l4n, c = i - q * l4n;
+            float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+              const float w = sw[0][q][k];
+              if (w != 0.f) {
+                const float4 v = __ldcg(bank + (int64_t)srow[0][q][k] * l4n + c);   // may have been written by another CTA
+                acc.x = fmaf(w, v.x, acc.x); acc.y = fmaf(w, v.y, acc.y);
+                acc.z = fmaf(w, v.z, acc.z); acc.w = fmaf(w, v.w, acc.w);
+              }
+            }
+            bank[((int64_t)out_slot * n_pix + q0 + q) * l4n + c] = acc;
+          }
+        }
+      }
+    }
+    // grid barrier: every CTA's stores of step s are visible before anyone starts step s + 1
+    if (s + 1 < n_steps) {
+      __syncthreads();
+      if (tid == 0) {
+        __threadfence();
+        atomicAdd(barrier, 1u);
+        const unsigned int want = (unsigned int)(s + 1) * gridDim.x;
+        unsigned int seen;
+        do {
+          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(barrier) : "memory");
+        } while (seen < want);
+      }
+      __syncthreads();
+    }
+    l = next_lane(lanes, n_lanes, s + 1, 0);
+  }
+}
+
 int64_t chain_workspace_bytes(int n_jobs, int n_pix, int K) {
   const int Kt = K <= 4 ? 4 : (K <= 10 ? 10 : 16);
   return (int64_t)n_jobs * n_pix * Kt * 8 + 256;
+}
+
+// the label-independent (weight, row) pairs of jobs [job_begin, job_begin + n) into the chain workspace (cw, crow),
+// and the grid barrier's counter reset; returns the counter
+template <int K>
+static int launch_weights_t(const float* tv, const int32_t* ti, int k_in, int groups, const fgvc_job* jobs, int job_begin,
+                            int n, const int32_t* mem_label, const int32_t* pair_ref, int n_pix, float temperature,
+                            int flags, void* ws, float** cw, int32_t** crow, unsigned int** barrier, cudaStream_t st) {
+  const int64_t cells = (int64_t)n * n_pix * K;
+  *cw = reinterpret_cast<float*>(ws);
+  *crow = reinterpret_cast<int32_t*>(reinterpret_cast<uint8_t*>(ws) + cells * 4);
+  *barrier = reinterpret_cast<unsigned int*>(reinterpret_cast<uint8_t*>(ws) + cells * 8);
+  FGVC_CUDA(cudaMemsetAsync(*barrier, 0, 256, st));
+  dim3 gw(cdiv(n_pix, 256), n);
+  gather_weights_kernel<K><<<gw, 256, 0, st>>>(tv, ti, k_in, groups, jobs, job_begin, mem_label, pair_ref, n_pix,
+                                               temperature, flags, *cw, *crow);
+  FGVC_LAUNCH_CHECK();
+  return FGVC_OK;
+}
+
+// co-resident CTAs of a 256-thread chain kernel on the calling thread's device (they spin on the grid barrier:
+// cooperative launch, sized from the occupancy; cached per device index, written once with the same value by any
+// thread)
+static int resident_ctas(const void* kernel, std::atomic<int>* cached, int* max_ctas) {
+  int dev = 0;
+  FGVC_CUDA(cudaGetDevice(&dev));
+  *max_ctas = (dev >= 0 && dev < 64) ? cached[dev].load(std::memory_order_relaxed) : 0;
+  if (*max_ctas == 0) {
+    int sms = 0, occ = 0;
+    FGVC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    FGVC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, 256, 0));
+    *max_ctas = sms * (occ < 1 ? 1 : occ);
+    if (dev >= 0 && dev < 64) cached[dev].store(*max_ctas, std::memory_order_relaxed);
+  }
+  return FGVC_OK;
 }
 
 template <int K>
 static int launch_chain_t(const float* tv, const int32_t* ti, int k_in, int groups, const fgvc_job* jobs, int job_begin,
                           int n, const int32_t* mem_label, const int32_t* pair_ref, int n_pix, float temperature,
                           int flags, float* lab, int Lp, void* ws, cudaStream_t st) {
-  const int64_t cells = (int64_t)n * n_pix * K;
-  float* cw = reinterpret_cast<float*>(ws);
-  int32_t* crow = reinterpret_cast<int32_t*>(reinterpret_cast<uint8_t*>(ws) + cells * 4);
-  unsigned int* barrier = reinterpret_cast<unsigned int*>(reinterpret_cast<uint8_t*>(ws) + cells * 8);
-  FGVC_CUDA(cudaMemsetAsync(barrier, 0, 256, st));
-  dim3 gw(cdiv(n_pix, 256), n);
-  gather_weights_kernel<K><<<gw, 256, 0, st>>>(tv, ti, k_in, groups, jobs, job_begin, mem_label, pair_ref, n_pix,
-                                               temperature, flags, cw, crow);
-  FGVC_LAUNCH_CHECK();
-  // all CTAs must be co-resident (they spin on the grid barrier): cooperative launch, sized from the occupancy
-  // (per device of the calling thread; cached per device index, written once with the same value by any thread)
+  float* cw;
+  int32_t* crow;
+  unsigned int* barrier;
+  int rc = launch_weights_t<K>(tv, ti, k_in, groups, jobs, job_begin, n, mem_label, pair_ref, n_pix, temperature, flags,
+                               ws, &cw, &crow, &barrier, st);
+  if (rc) return rc;
   static std::atomic<int> cached[64];
-  int dev = 0;
-  FGVC_CUDA(cudaGetDevice(&dev));
-  int max_ctas = (dev >= 0 && dev < 64) ? cached[dev].load(std::memory_order_relaxed) : 0;
-  if (max_ctas == 0) {
-    int sms = 0, occ = 0;
-    FGVC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    FGVC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_chain_kernel<K>, 256, 0));
-    max_ctas = sms * (occ < 1 ? 1 : occ);
-    if (dev >= 0 && dev < 64) cached[dev].store(max_ctas, std::memory_order_relaxed);
-  }
+  int max_ctas = 0;
+  rc = resident_ctas((const void*)gather_chain_kernel<K>, cached, &max_ctas);
+  if (rc) return rc;
   const int l4n = Lp / 4;
   // latency-bound (a few microseconds per frame): as many CTAs as can be co-resident, so that a CTA's slice is
   // one pass of <= CH_Q queries whenever possible
@@ -380,6 +546,54 @@ int launch_gather_chain(const float* tv, const int32_t* ti, int K, int groups, c
   if (K <= 4) return launch_chain_t<4>(tv, ti, K, groups, jobs, job_begin, n, mem_label, pair_ref, n_pix, temperature, flags, lab, Lp, ws, st);
   if (K <= 10) return launch_chain_t<10>(tv, ti, K, groups, jobs, job_begin, n, mem_label, pair_ref, n_pix, temperature, flags, lab, Lp, ws, st);
   return launch_chain_t<16>(tv, ti, K, groups, jobs, job_begin, n, mem_label, pair_ref, n_pix, temperature, flags, lab, Lp, ws, st);
+}
+
+template <int K>
+static int launch_chain_lanes_t(const float* tv, const int32_t* ti, int k_in, int groups, const fgvc_job* jobs,
+                                int job_base, int n, const fgvc_lane* lanes_dev, int n_lanes, int n_steps, int max_l4n,
+                                const int32_t* mem_label, const int32_t* pair_ref, int n_pix, float temperature,
+                                int flags, float* lab, void* ws, cudaStream_t st) {
+  float* cw;
+  int32_t* crow;
+  unsigned int* barrier;
+  int rc = launch_weights_t<K>(tv, ti, k_in, groups, jobs, job_base, n, mem_label, pair_ref, n_pix, temperature, flags,
+                               ws, &cw, &crow, &barrier, st);
+  if (rc) return rc;
+  static std::atomic<int> cached[64];
+  int max_ctas = 0;
+  rc = resident_ctas((const void*)gather_chain_lanes_kernel<K>, cached, &max_ctas);
+  if (rc) return rc;
+  // the grid rule of the single-lane chain, for the lane with the longest rows
+  const int ctas = (int)min((int64_t)max_ctas, max((int64_t)1, ((int64_t)n_pix * max_l4n + 63) / 64));
+  int jb = job_base, nl = n_lanes, ns = n_steps, npx = n_pix;
+  void* args[] = {(void*)&cw, (void*)&crow, (void*)&jobs, (void*)&jb, (void*)&lanes_dev, (void*)&nl, (void*)&ns,
+                  (void*)&npx, (void*)&lab, (void*)&barrier};
+  FGVC_CUDA(cudaLaunchCooperativeKernel((const void*)gather_chain_lanes_kernel<K>, dim3(ctas), dim3(256), args, 0, st));
+  fgvc::g_launches.fetch_add(1);
+  return FGVC_OK;
+}
+
+// K1b for every lane of lanes_host[0, n_lanes) as one multi-lane chain (see gather_chain_lanes_kernel); the lanes are
+// validated by the caller
+int launch_gather_chain_lanes(const float* tv, const int32_t* ti, int K, int groups, const fgvc_job* jobs,
+                              const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int n_lanes,
+                              const int32_t* mem_label, const int32_t* pair_ref, int n_pix, float temperature, int flags,
+                              float* lab, void* ws, int64_t ws_bytes, cudaStream_t st) {
+  int jb = lanes_host[0].job_begin, je = lanes_host[0].job_end, n_steps = 0, max_l4n = 1;
+  for (int i = 0; i < n_lanes; ++i) {
+    jb = min(jb, lanes_host[i].job_begin);
+    je = max(je, lanes_host[i].job_end);
+    n_steps = max(n_steps, lanes_host[i].job_end - lanes_host[i].job_begin);
+    max_l4n = max(max_l4n, lanes_host[i].Lp / 4);
+  }
+  const int n = je - jb;
+  FGVC_CHECK_ARG(n <= 65535, "gather chain lanes: %d jobs in the lanes' range, at most 65535", n);
+  FGVC_CHECK_ARG(ws != nullptr && ws_bytes >= chain_workspace_bytes(n, n_pix, K),
+                 "gather chain lanes: workspace of %lld bytes needed (fgvc_chain_workspace_bytes)",
+                 (long long)chain_workspace_bytes(n, n_pix, K));
+  if (K <= 4) return launch_chain_lanes_t<4>(tv, ti, K, groups, jobs, jb, n, lanes_dev, n_lanes, n_steps, max_l4n, mem_label, pair_ref, n_pix, temperature, flags, lab, ws, st);
+  if (K <= 10) return launch_chain_lanes_t<10>(tv, ti, K, groups, jobs, jb, n, lanes_dev, n_lanes, n_steps, max_l4n, mem_label, pair_ref, n_pix, temperature, flags, lab, ws, st);
+  return launch_chain_lanes_t<16>(tv, ti, K, groups, jobs, jb, n, lanes_dev, n_lanes, n_steps, max_l4n, mem_label, pair_ref, n_pix, temperature, flags, lab, ws, st);
 }
 
 }  // namespace fgvc

@@ -81,10 +81,15 @@ class FeatureBank:
 class LabelBank:
     """lab[slot][H*W][Lp], Lp = L padded to a multiple of 4."""
 
-    def __init__(self, n_slots, L, H, W, device):
+    def __init__(self, n_slots, L, H, W, device, buf=None):
+        """``buf``: a flat fp32 CUDA tensor of n_slots * H*W * Lp elements to hold the bank (several banks carved out of
+        one allocation); default: a new one."""
         _lib.require_cuda()
         self.n_slots, self.L, self.Lp, self.H, self.W = n_slots, L, pad4(L), H, W
-        self.buf = torch.empty(n_slots, H * W, self.Lp, dtype=torch.float32, device=device)
+        if buf is None:
+            self.buf = torch.empty(n_slots, H * W, self.Lp, dtype=torch.float32, device=device)
+        else:
+            self.buf = buf.view(n_slots, H * W, self.Lp)
 
     def put_nchw(self, src, slot, chan_stride=None):
         """src: [L,H,W] view whose pixels are contiguous; chan_stride in floats."""
@@ -396,30 +401,41 @@ def pick_packing(table, j0, j1, H, W, radius, mode):
     return best
 
 
+def pair_key(table, job):
+    """(query frame, backward) of a job of ``table``: the memory frames of a job run backwards in time (the forward
+    tracker on the time-reversed clip) all lie after its query frame, those of a forward job before it."""
+    q_slot, b = job[0], job[1]
+    return q_slot, (table.mem_feat[b] & ~_lib.MEM_UNMASKED) > q_slot
+
+
 def shared_pair_table(table, spans, T):
     """Several ``with_first`` groups of one clip: the jobs (group g, query frame t) of different groups see the same
     memory frames except their first one, so the label-independent K1 work is shared -- run it once per query frame
-    over the UNION of the groups' memory entries, one list per (query frame, memory entry) pair, and let the tail
-    merge each job's lists.  Returns (utable, Gmax, pair_ref) or None when sharing would not pay:
-      utable   : JobTable with one job per query frame t, entries = sorted unique (frame, mask flag) of all groups;
+    and direction over the UNION of the groups' memory entries, one list per (query frame, direction, memory entry),
+    and let the tail merge each job's lists.  Forward and backward jobs of a query frame are not merged: their
+    memories have no frame in common, and the list floor of the shared launch needs one.  Returns (utable, Gmax,
+    pair_ref) or None when sharing would not pay:
+      utable   : JobTable with one job per (query frame, direction), entries = sorted unique (frame, mask flag) of all
+                 groups;
       pair_ref : for every memory entry of ``table`` the index (u_job * Gmax + position in the union) of its list."""
-    by_t = {}
-    for j, (q_slot, b, e, _) in enumerate(table.jobs):
-        by_t.setdefault(q_slot, set()).update(table.mem_feat[b:e])
-    if len(table) < 1.8 * len(by_t):
+    by_key = {}
+    for job in table.jobs:
+        by_key.setdefault(pair_key(table, job), set()).update(table.mem_feat[job[1]:job[2]])
+    if len(table) < 1.8 * len(by_key):
         return None
-    gmax = max(len(v) for v in by_t.values())
+    gmax = max(len(v) for v in by_key.values())
     if gmax > 64:
         return None
     utable, where = JobTable(), {}
-    for u, t in enumerate(sorted(by_t)):
-        ent = sorted(by_t[t], key=lambda r: (r & ~_lib.MEM_UNMASKED, 0 if (r & _lib.MEM_UNMASKED) else 1))
-        utable.add_raw(t, ent, t)
+    for u, key in enumerate(sorted(by_key)):
+        ent = sorted(by_key[key], key=lambda r: (r & ~_lib.MEM_UNMASKED, 0 if (r & _lib.MEM_UNMASKED) else 1))
+        utable.add_raw(key[0], ent, key[0])
         for i, r in enumerate(ent):
-            where[(t, r)] = u * gmax + i
+            where[(key, r)] = u * gmax + i
     pair_ref = []
-    for (q_slot, b, e, _) in table.jobs:
-        pair_ref.extend(where[(q_slot, r)] for r in table.mem_feat[b:e])
+    for job in table.jobs:
+        key = pair_key(table, job)
+        pair_ref.extend(where[(key, r)] for r in table.mem_feat[job[1]:job[2]])
     return utable, gmax, pair_ref
 
 
@@ -452,6 +468,23 @@ def chain_workspace(dev, n_jobs, n_pix, K, flags=0, force=False):
         ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         _CHAIN_WS[_ws_key(dev)] = ws
     return ptr(ws), nbytes
+
+
+def point_tail_lanes(lists, pair_ref, table, lanes, lab, maps, coords, H, W, out_hw, temperature, flags, coord_topk=5):
+    """fgvc_point_clip_tail_lanes: the point tails of several independent recurrences of a clip in one multi-lane
+    gather chain.  ``lanes``: list of (job_begin, job_end, L, lab_offset, coord_offset), offsets in floats into the
+    flat tensors ``lab`` (label banks) and ``coords`` (tracks); ``maps``: NCHW scratch of every lane;
+    ``pair_ref``: device int32 tensor of the shared lists or None."""
+    dev = lab.device
+    jobs_dev, _, mem_label = table.device(dev)
+    jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4).contiguous()
+    host = (_lib.Lane * len(lanes))(*[_lib.Lane(jb, je, L, pad4(L), lo, co) for (jb, je, L, lo, co) in lanes])
+    lanes_dev = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(dev)
+    jb, je = min(ln[0] for ln in lanes), max(ln[1] for ln in lanes)
+    call("fgvc_point_clip_tail_lanes", ptr(lists.val), ptr(lists.idx), lists.K, 1 if pair_ref is not None else lists.groups,
+         ptr(pair_ref) if pair_ref is not None else None, ptr(jobs_dev), ptr(jobs_host), ptr(lanes_dev), ctypes.c_void_p(ctypes.addressof(host)), len(lanes),
+         ptr(mem_label), H, W, float(temperature), int(flags), ptr(lab), int(out_hw[0]), int(out_hw[1]), int(coord_topk),
+         ptr(maps), ptr(coords), *chain_workspace(dev, je - jb, H * W, lists.K, flags, force=True), stream_ptr())
 
 
 K1_TIMING = None       # bench.py: a list -> affinity_topk appends (start, end) CUDA events of every K1 launch

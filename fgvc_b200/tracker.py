@@ -12,6 +12,7 @@ What changes relative to the reference loop (results identical, see tests):
   * heat-maps are never up-sampled into a [T,P,h,w] tensor nor shipped to the host:
     K3 fuses the bilinear up-sampling with the top-5 soft-argmax (:396-406, :172-191).
 """
+import ctypes
 import os
 
 import torch
@@ -217,18 +218,26 @@ class VanillaTracker(nn.Module):
             if not host_feats and (shard is None or shard[1] == 1):
                 bank.load_frames(feats, 0, normalize=normalize)
 
+        bidirectional = bool(cfg.get("bidirectional", False))
         table = JobTable()
-        spans = []   # per group: (first job, t0)
+        spans = []   # per group: (first job, t0); forward jobs t0+1 .. T-1, then (bidirectional) backward jobs t0-1 .. 0
         for t0, _ in groups:
             spans.append((len(table), t0))
             for t in range(t0 + 1, T):
                 mem = engine.memory_frames(t, precede, with_first_mem, first=t0)
                 table.add(t, mem, mem, t, unmasked=len(mem) if nr is None else unmasked_first)
+            if bidirectional:
+                # the forward tracker on the time-reversed clip (query frame T-1-t0), mapped back to frame indices:
+                # memory [t0] + [min(t0, t + precede), ..., t + 1]
+                for t in range(t0 - 1, -1, -1):
+                    mem = [T - 1 - r for r in engine.memory_frames(T - 1 - t, precede, with_first_mem, first=T - 1 - t0)]
+                    table.add(t, mem, mem, t, unmasked=len(mem) if nr is None else unmasked_first)
         outs = []
         radius = (nr // 2) if nr is not None else 1
         shared = None
         rank, world = shard if shard is not None else (0, 1)
-        streamed = host_feats and len(groups) == 1 and world == 1 and len(table) > 0
+        # (the streamed path needs every job to read only earlier frames: forward jobs only)
+        streamed = host_feats and len(groups) == 1 and world == 1 and len(table) > 0 and not bidirectional
         if host_feats and not streamed and world == 1:
             bank.load_frames(feats.to(dev, non_blocking=True), 0, normalize=normalize)
         if streamed:
@@ -265,16 +274,21 @@ class VanillaTracker(nn.Module):
             if shared is not None:
                 utable, gmax, pair_ref = shared
                 # every list of a query frame t starts from the K-th best of the query's 5 x 5 neighbourhood in frame
-                # t - 1, which is in the memory of every group that is alive at t: without it the per-pair lists start
-                # cold and half of the launch is list insertion
+                # t - 1 (t + 1 for the backward jobs), which is in the memory of every group that is alive at t: without
+                # it the per-pair lists start cold and half of the launch is list insertion
                 floor = None
                 if os.environ.get("FGVC_NO_FLOOR") != "1" and radius >= 3:
-                    # the newest frame that EVERY job of a query frame has in its memory (-1: none, no floor)
+                    # the frame nearest to t that EVERY job of a (query frame, direction) has in its memory (-1: none,
+                    # no floor)
                     common = {}
-                    for (q_slot, b, e, _) in table.jobs:
-                        mem = {r & ~_lib.MEM_UNMASKED for r in table.mem_feat[b:e]}
-                        common[q_slot] = mem if q_slot not in common else (common[q_slot] & mem)
-                    seeds = [max(common.get(j[0], set()), default=-1) for j in utable.jobs]
+                    for job in table.jobs:
+                        key = engine.pair_key(table, job)
+                        mem = {r & ~_lib.MEM_UNMASKED for r in table.mem_feat[job[1]:job[2]]}
+                        common[key] = mem if key not in common else (common[key] & mem)
+                    seeds = []
+                    for job in utable.jobs:
+                        key = engine.pair_key(utable, job)
+                        seeds.append((min if key[1] else max)(common.get(key, set()), default=-1))
                     floor = engine.topk_floor(bank, utable, seeds, radius, cfg.topk, mask_mode)
                 lists = engine.affinity_topk(bank, utable, radius, cfg.topk, mask_mode, groups=gmax,
                                              engine=self.engine_id, pack=False, floor=floor)
@@ -288,36 +302,41 @@ class VanillaTracker(nn.Module):
         all_c0 = engine.gaussian_coords(all_pts, (h, w)) if groups and all_pts.shape[0] else None
         p_off = 0
         sizes = [int(pts.shape[0]) for _, pts in groups]
-        for (j0, t0), (_, pts) in zip(spans, groups):
-            P_all = pts.shape[0]
-            lo_p, hi_p = (0, P_all) if world == 1 else ((P_all * rank) // world, (P_all * (rank + 1)) // world)
-            P = hi_p - lo_p
-            pts = all_pts[p_off + lo_p:p_off + hi_p]
-            c0 = all_c0[p_off + lo_p:p_off + hi_p] if all_c0 is not None else None
-            p_off += P_all
-            if P == 0:
-                outs.append(torch.zeros(T, 0, 2, dtype=torch.float64, device=dev))
-                continue
-            labels = LabelBank(T, P, Hf, Wf, dev)
-            labels.put_gaussians(pts, t0, stride)
-            coords = torch.zeros(T, P, 2, dtype=torch.float32, device=dev)
-            coords[t0] = c0
-            if T - t0 > 1:
-                scratch = torch.empty(T, P, Hf, Wf, dtype=torch.float32, device=dev)   # NCHW maps of every frame
-                if shared is not None:
-                    _lib.call("fgvc_point_clip_tail_shared", _lib.ptr(lists.val), _lib.ptr(lists.idx), lists.K,
-                              _lib.ptr(pair_ref), _lib.ptr(jobs_dev), _lib.ptr(jobs_host), j0, j0 + (T - t0 - 1),
-                              _lib.ptr(mem_label), Hf, Wf, temperature, flags, _lib.ptr(labels.buf), labels.Lp, P, h, w, 5,
-                              _lib.ptr(scratch), _lib.ptr(coords),
-                              *engine.chain_workspace(dev, T - t0 - 1, Hf * Wf, lists.K, flags, force=True),
-                              _lib.stream_ptr())
-                else:
-                    _lib.call("fgvc_point_clip_tail", _lib.ptr(lists.val), _lib.ptr(lists.idx), lists.K, lists.groups,
-                              _lib.ptr(jobs_dev), _lib.ptr(jobs_host), j0, j0 + (T - t0 - 1), _lib.ptr(mem_label), Hf, Wf,
-                              temperature, flags, _lib.ptr(labels.buf), labels.Lp, P, h, w, 5, _lib.ptr(scratch),
-                              _lib.ptr(coords), *engine.chain_workspace(dev, T - t0 - 1, Hf * Wf, lists.K, flags),
-                              _lib.stream_ptr())
-            outs.append(coords.double())
+        if bidirectional:
+            outs = self._bidirectional_tail(lists, shared, pair_ref if shared is not None else None, table, spans, groups,
+                                            all_pts, all_c0, rank, world, T, Hf, Wf, (h, w), stride, temperature, flags,
+                                            dev)
+        else:
+            for (j0, t0), (_, pts) in zip(spans, groups):
+                P_all = pts.shape[0]
+                lo_p, hi_p = (0, P_all) if world == 1 else ((P_all * rank) // world, (P_all * (rank + 1)) // world)
+                P = hi_p - lo_p
+                pts = all_pts[p_off + lo_p:p_off + hi_p]
+                c0 = all_c0[p_off + lo_p:p_off + hi_p] if all_c0 is not None else None
+                p_off += P_all
+                if P == 0:
+                    outs.append(torch.zeros(T, 0, 2, dtype=torch.float64, device=dev))
+                    continue
+                labels = LabelBank(T, P, Hf, Wf, dev)
+                labels.put_gaussians(pts, t0, stride)
+                coords = torch.zeros(T, P, 2, dtype=torch.float32, device=dev)
+                coords[t0] = c0
+                if T - t0 > 1:
+                    scratch = torch.empty(T, P, Hf, Wf, dtype=torch.float32, device=dev)   # NCHW maps of every frame
+                    if shared is not None:
+                        _lib.call("fgvc_point_clip_tail_shared", _lib.ptr(lists.val), _lib.ptr(lists.idx), lists.K,
+                                  _lib.ptr(pair_ref), _lib.ptr(jobs_dev), _lib.ptr(jobs_host), j0, j0 + (T - t0 - 1),
+                                  _lib.ptr(mem_label), Hf, Wf, temperature, flags, _lib.ptr(labels.buf), labels.Lp, P, h, w, 5,
+                                  _lib.ptr(scratch), _lib.ptr(coords),
+                                  *engine.chain_workspace(dev, T - t0 - 1, Hf * Wf, lists.K, flags, force=True),
+                                  _lib.stream_ptr())
+                    else:
+                        _lib.call("fgvc_point_clip_tail", _lib.ptr(lists.val), _lib.ptr(lists.idx), lists.K, lists.groups,
+                                  _lib.ptr(jobs_dev), _lib.ptr(jobs_host), j0, j0 + (T - t0 - 1), _lib.ptr(mem_label), Hf, Wf,
+                                  temperature, flags, _lib.ptr(labels.buf), labels.Lp, P, h, w, 5, _lib.ptr(scratch),
+                                  _lib.ptr(coords), *engine.chain_workspace(dev, T - t0 - 1, Hf * Wf, lists.K, flags),
+                                  _lib.stream_ptr())
+                outs.append(coords.double())
         if world > 1:
             from . import apis
             pads = [-(-n // world) for n in sizes]
@@ -328,6 +347,60 @@ class VanillaTracker(nn.Module):
                 off += pad
             outs = apis.gather_point_tracks(local, sizes, rank, world)
         return outs
+
+    def _bidirectional_tail(self, lists, shared, pair_ref, table, spans, groups, all_pts, all_c0, rank, world, T, Hf, Wf,
+                            image_hw, stride, temperature, flags, dev):
+        """Recurrent tail of ``test_cfg.bidirectional``: every group of this rank's points is tracked forward from its
+        query frame and backward to frame 0 -- two lanes over the group's label bank (both read slot t0 and write
+        disjoint slots).  All banks and tracks are carved out of one allocation each, and every lane runs in ONE
+        multi-lane gather chain (engine.point_tail_lanes); FGVC_NO_LANES=1 runs each lane through its own point tail
+        instead (same results, one chain launch per lane).  Returns per group the [T, P_rank, 2] float64 tracks."""
+        n_pix = Hf * Wf
+        parts, p_off = [], 0               # per group: (first job, t0, first point in all_pts, points of this rank)
+        for (j0, t0), (_, pts) in zip(spans, groups):
+            P_all = int(pts.shape[0])
+            lo_p, hi_p = (0, P_all) if world == 1 else ((P_all * rank) // world, (P_all * (rank + 1)) // world)
+            parts.append((j0, t0, p_off + lo_p, hi_p - lo_p))
+            p_off += P_all
+        lab = torch.empty(sum(T * n_pix * engine.pad4(P) for *_, P in parts), dtype=torch.float32, device=dev)
+        coords = torch.zeros(sum(T * P * 2 for *_, P in parts), dtype=torch.float32, device=dev)
+        lanes, outs, lab_off, c_off = [], [], 0, 0
+        for j0, t0, a, P in parts:
+            track = coords[c_off:c_off + T * P * 2].view(T, P, 2)
+            outs.append(track)
+            if P:
+                labels = LabelBank(T, P, Hf, Wf, dev, buf=lab[lab_off:lab_off + T * n_pix * engine.pad4(P)])
+                labels.put_gaussians(all_pts[a:a + P], t0, stride)
+                track[t0] = all_c0[a:a + P]
+                n_fw = T - t0 - 1
+                for jb, je in ((j0, j0 + n_fw), (j0 + n_fw, j0 + T - 1)):      # forward lane, backward lane
+                    if je > jb:
+                        lanes.append((jb, je, P, lab_off, c_off))
+            lab_off += T * n_pix * engine.pad4(P)
+            c_off += T * P * 2
+        if lanes:
+            maps = torch.empty(T * max(ln[2] for ln in lanes) * n_pix, dtype=torch.float32, device=dev)   # NCHW scratch
+            if os.environ.get("FGVC_NO_LANES") == "1":
+                jobs_dev, _, mem_label = table.device(dev)
+                jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4).contiguous()
+                for jb, je, P, lo, co in lanes:
+                    lab_ptr = ctypes.c_void_p(lab.data_ptr() + 4 * lo)
+                    crd_ptr = ctypes.c_void_p(coords.data_ptr() + 4 * co)
+                    if shared is not None:
+                        _lib.call("fgvc_point_clip_tail_shared", _lib.ptr(lists.val), _lib.ptr(lists.idx), lists.K,
+                                  _lib.ptr(pair_ref), _lib.ptr(jobs_dev), _lib.ptr(jobs_host), jb, je, _lib.ptr(mem_label),
+                                  Hf, Wf, temperature, flags, lab_ptr, engine.pad4(P), P, *image_hw, 5, _lib.ptr(maps),
+                                  crd_ptr, *engine.chain_workspace(dev, je - jb, n_pix, lists.K, flags, force=True),
+                                  _lib.stream_ptr())
+                    else:
+                        _lib.call("fgvc_point_clip_tail", _lib.ptr(lists.val), _lib.ptr(lists.idx), lists.K, lists.groups,
+                                  _lib.ptr(jobs_dev), _lib.ptr(jobs_host), jb, je, _lib.ptr(mem_label), Hf, Wf,
+                                  temperature, flags, lab_ptr, engine.pad4(P), P, *image_hw, 5, _lib.ptr(maps), crd_ptr,
+                                  *engine.chain_workspace(dev, je - jb, n_pix, lists.K, flags), _lib.stream_ptr())
+            else:
+                engine.point_tail_lanes(lists, pair_ref, table, lanes, lab, maps, coords, Hf, Wf, image_hw, temperature,
+                                        flags)
+        return [o.double() for o in outs]
 
     def forward_test(self, rgbs, query_points, trajectories, visibilities, save_image=False, save_path=None,
                      iteration=None, shard=None):

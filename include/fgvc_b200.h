@@ -84,6 +84,19 @@ typedef struct fgvc_job {
   int32_t out_slot;   /* label-bank slot written by fgvc_gather_labels */
 } fgvc_job;
 
+/* One lane of fgvc_point_clip_tail_lanes: one recurrence of a clip (the forward or the backward track of a point group)
+ * = the consecutive jobs [job_begin, job_end) in recurrence order, with their out_slots running consecutively up or
+ * down, over its own label bank lab_bank + lab_offset ([slot][H*W][Lp]) and its own tracks coords + coord_offset
+ * ([slot][L][2]).  Two lanes may share a bank when neither reads a slot the other writes. */
+typedef struct fgvc_lane {
+  int32_t job_begin;
+  int32_t job_end;
+  int32_t L;             /* label channels (points) of the lane's bank */
+  int32_t Lp;            /* bank row length: L rounded up to a multiple of 4 */
+  int64_t lab_offset;    /* floats from lab_bank to the lane's bank */
+  int64_t coord_offset;  /* floats from coords to the lane's tracks */
+} fgvc_lane;
+
 /* Job-packed query tiles of the fp16 tensor engine (fgvc_affinity_topk_packed): a tile group = up to 4 jobs that
  * share most of their memory frames (consecutive query frames of a clip) and are multiplied against each key box
  * together.  Memory entries [u_begin, u_end) of the union tables list every (frame, mask flag) any job of the group
@@ -252,7 +265,8 @@ FGVC_API int fgvc_decode_masks_pixmajor(const float* lab_bank, int32_t slot, int
  *              masks[slot][out_h][out_w]; scratch_minmax: (job_end - job_begin) * 2 * L words;
  *  point tail: the K1b gather chain over jobs [job_begin, job_end) with an NCHW copy of every frame
  *              into maps_nchw[slot][L][H*W], then ONE K3 launch over all their (frame, point) maps
- *              into coords[slot][L][2]; the out_slots of the range must be consecutive. */
+ *              into coords[slot][L][2]; the out_slots of the range must be consecutive (ascending, or descending
+ *              for a track run backwards in time). */
 /* chain_ws (optional, fgvc_chain_workspace_bytes(job_end - job_begin, H*W, K) bytes): with it the gather chain of a
  * range runs as ONE persistent cooperative kernel (label-independent weights for all frames first, then one grid
  * barrier per frame) instead of one launch per frame; NULL keeps the per-frame launches.  Same results. */
@@ -282,6 +296,23 @@ FGVC_API int fgvc_point_clip_tail_shared(const float* topk_val, const int32_t* t
                          int32_t job_begin, int32_t job_end, const int32_t* mem_label_slot, int32_t H, int32_t W,
                          float temperature, int32_t flags, float* lab_bank, int32_t Lp, int32_t L,
                          int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
+                         float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream);
+
+/* Point tail of SEVERAL independent recurrences of one clip (bidirectional tracking: every point group is tracked
+ * forward from its query frame and, on the time-reversed clip, backward to frame 0).  Each lane (fgvc_lane) is the
+ * point tail above over its own job range, bank and tracks, and gives bit for bit what that tail gives; but the
+ * chains of all lanes run together: ONE weight launch over the jobs of every lane, then ONE cooperative kernel whose
+ * step s gathers job s of every lane still running, with one grid barrier per step -- the longest lane's length of
+ * barriers instead of the sum over the lanes.  The NCHW copies and K3 then run per lane.  pair_ref: NULL (lists of
+ * `groups` parts per job) or the shared lists of fgvc_point_clip_tail_shared (groups must be 1).
+ * lanes_dev / lanes_host: the lane table in device and host memory.  maps_nchw: scratch of (largest out_slot + 1) x
+ * (largest L) x H*W floats, reused lane after lane.  chain_ws (required): fgvc_chain_workspace_bytes(je - jb, H*W, K)
+ * bytes, [jb, je) = the smallest job range holding every lane. */
+FGVC_API int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
+                         const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
+                         const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int32_t n_lanes,
+                         const int32_t* mem_label_slot, int32_t H, int32_t W, float temperature, int32_t flags,
+                         float* lab_bank, int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
                          float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream);
 
 /* K2 -- coarse-to-fine propagation (local_attention.py:721-880), single query frame.

@@ -46,6 +46,12 @@ def main():
         a = trk.propagate_points(feats.cpu().pin_memory(), grp, (h, w), shard=(rank, world))[0]
         b = trk.propagate_points(feats, grp, (h, w))[0]
     err = max(err, (a - b).abs().max().item())
+    # bidirectional tracking (points queried at several frames, tracked both ways): same split, direction-agnostic
+    trk.test_cfg = type(trk.test_cfg)(dict(cfg, bidirectional=True))
+    with torch.no_grad():
+        got3 = apis.sharded_forward_test(trk, rgbs, qp, traj, vis)
+        want3 = trk(test_mode=True, rgbs=rgbs, query_points=qp, trajectories=traj, visibilities=vis)
+    err = max(err, (got3[2].double() - want3[2].double()).abs().max().item())
     trk.test_cfg = type(trk.test_cfg)(cfg)
     # video-sharded driver + typed NCCL gather
     ds = [dict(rgbs=S.synthetic_video(4, 32, 48, seed=10 + i)[None], query_points=S.query_points(3, 4, 32, 48, seed=i)[None],
