@@ -42,6 +42,12 @@ class Lane(ctypes.Structure):
                 ("lab_offset", c_int64), ("coord_offset", c_int64)]
 
 
+class C2FLane(ctypes.Structure):
+    """fgvc_c2f_lane: one recurrence of fgvc_c2f_point_clip_tail_lanes (offsets in floats)"""
+    _fields_ = [("job_begin", c_int32), ("job_end", c_int32), ("L", c_int32), ("Lp", c_int32),
+                ("lab_offset", c_int64), ("out_offset", c_int64), ("coord_offset", c_int64)]
+
+
 P = c_void_p
 I = c_int32
 L64 = c_int64
@@ -79,6 +85,9 @@ SIGNATURES = {
     "fgvc_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, P, I, P, I, I, F, I, P, I, I, I, P, P, P, L64, P]),
     "fgvc_c2f_scratch_elems": (L64, [I, I]),
     "fgvc_c2f_propagate": (I, [P, I, I, I, I, I, P, I, I, I, P, P, P, P, I, I, I, I, F, P, I, P, P, P, L64, I, P]),
+    "fgvc_c2f_clip_workspace_bytes": (L64, [P, I, I, I, I, I]),
+    "fgvc_c2f_clip_weights": (I, [P, I, I, I, I, I, P, I, I, I, P, I, I, P, P, I, I, I, I, F, P, P, P, L64, I, P]),
+    "fgvc_c2f_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, I, I, I, I, I, P, P, I, I, I, P, P, P, P]),
 }
 
 _lib = None

@@ -17,15 +17,21 @@ Everything stays resident in HBM across frames: both feature banks are built onc
 label bank holds every frame, a frame costs one coarse K1 (k = 1 per memory frame), one window-mode K1 on the tensor
 cores, the c2f tail, one up-sampling kernel and K3.
 """
+import ctypes
+
 import torch
 
 from . import _lib, engine
 from .engine import FeatureBank, JobTable, LabelBank
 
+# bound of the list workspace of one fgvc_c2f_clip_weights call (the host calls it in job slices beyond): ~1.5 MB per
+# job at 32^2 coarse / 128^2 fine, precede 5, K 10 -- a strided 50-frame clip tracked both ways fits one slice
+_CLIP_WS_BUDGET = 2 << 30
+
 
 class C2FPointTracker:
     """cfg keys: precede_frames, topk, temperature, neighbor_range (coarse), radius_fine, with_first (memory),
-    with_first_neighbor, with_norm, split, mask_mode."""
+    with_first_neighbor, with_norm, split, mask_mode; bidirectional (track_queries only)."""
 
     def __init__(self, cfg, engine_id=_lib.ENGINE_AUTO):
         self.cfg = cfg
@@ -130,3 +136,109 @@ class C2FPointTracker:
             outs.append(out)
         landed(T - 1)            # (a one-frame clip: the banks must not be released under the staging stream)
         return traj, outs
+
+    @torch.no_grad()
+    def track_queries(self, feats_coarse, feats_fine, query_points, image_hw):
+        """TAP-Vid queries: query_points [P, 3] (t, x, y) as ``forward_test``'s ``query_points[0]`` (and
+        ``metrics.tapvid_sample``).  Returns traj [T, P, 2] float32 CUDA in the input point order.
+
+        The points are grouped by query frame t0.  Frames t >= t0 of a group are what ``track(feats_coarse[t0:],
+        feats_fine[t0:], points)`` gives; with the cfg key ``bidirectional`` frames t < t0 are what ``track()`` gives on
+        the time-reversed prefix ``feats[:t0 + 1].flip(0)``, mapped back (memory [t0] + [min(t0, t + precede) .. t + 1]),
+        else they are zero.  The label-independent stages of every job of the clip (coarse arg-max, fine window top-K,
+        zero-padded candidates, soft-max weights) run in a few launches whose number does not grow with the groups
+        (fgvc_c2f_clip_weights), and every forward and backward recurrence runs as a lane of one cooperative chain
+        (fgvc_c2f_point_clip_tail_lanes).  Host features (pinned) are uploaded whole, then take the same path."""
+        _lib.require_cuda()
+        cfg = self.cfg
+        T, C, Hc, Wc = feats_coarse.shape
+        Tf, Cf, Hf, Wf = feats_fine.shape
+        assert T == Tf and Hf % Hc == 0 and Wf % Wc == 0 and Hf // Hc == Wf // Wc, "fine grid must be s x the coarse grid"
+        h, w = image_hw
+        dev = feats_coarse.device if feats_coarse.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        stride_f = h // Hf
+        split = cfg.get("split") or ("f16" if (engine.default_split(C) == "f16" and Cf % 4 == 0) else "tf32")
+        normalize = cfg.get("with_norm", True)
+        coarse = FeatureBank(T, C, Hc, Wc, dev, split=split)
+        fine = FeatureBank(T, Cf, Hf, Wf, dev, split=split)
+        coarse.load_frames(feats_coarse.to(dev, non_blocking=True).float(), 0, normalize=normalize)
+        fine.load_frames(feats_fine.to(dev, non_blocking=True).float(), 0, normalize=normalize)
+
+        qp = query_points.to(device=dev, dtype=torch.float32)
+        qt = qp[:, 0].round().long()
+        t0s = torch.unique(qt).tolist()
+        order = [torch.nonzero(qt == t).flatten() for t in t0s]
+        bidirectional = bool(cfg.get("bidirectional", False))
+        unmasked_first = 0 if cfg.get("with_first_neighbor", True) else 1
+        table, spans = engine.query_job_table(t0s, T, cfg["precede_frames"], cfg.get("with_first", True), bidirectional,
+                                              lambda mem: unmasked_first)
+        K = int(cfg["topk"])
+        n_c, n_f = Hc * Wc, Hf * Wf
+        sizes = [int(o.numel()) for o in order]
+        lab = torch.empty(sum(T * n_f * engine.pad4(P) for P in sizes), dtype=torch.float32, device=dev)
+        cout = torch.empty(sum(T * n_c * engine.pad4(P) for P in sizes), dtype=torch.float32, device=dev)
+        coords = torch.zeros(sum(T * P * 2 for P in sizes), dtype=torch.float32, device=dev)
+        perm = torch.cat(order) if order else torch.zeros(0, dtype=torch.long, device=dev)
+        pts_all = qp[perm, 1:].contiguous()
+        c0_all = engine.gaussian_coords(pts_all, (h, w)) if pts_all.shape[0] else None
+        lanes, tracks = [], []
+        lab_off = out_off = c_off = p_off = 0
+        for (j0, t0), P in zip(spans, sizes):
+            track = coords[c_off:c_off + T * P * 2].view(T, P, 2)
+            tracks.append(track)
+            labels = LabelBank(T, P, Hf, Wf, dev, buf=lab[lab_off:lab_off + T * n_f * engine.pad4(P)])
+            labels.put_gaussians(pts_all[p_off:p_off + P], t0, stride_f)
+            track[t0] = c0_all[p_off:p_off + P]
+            n_fw, n_bw = T - t0 - 1, (t0 if bidirectional else 0)
+            # forward lane, backward lane: they share the group's banks (both read slot t0, they write disjoint slots)
+            for jb, je in ((j0, j0 + n_fw), (j0 + n_fw, j0 + n_fw + n_bw)):
+                if je > jb:
+                    lanes.append(_lib.C2FLane(jb, je, P, engine.pad4(P), lab_off, out_off, c_off))
+            lab_off += T * n_f * engine.pad4(P)
+            out_off += T * n_c * engine.pad4(P)
+            c_off += T * P * 2
+            p_off += P
+        if lanes:
+            self._clip_weights_and_chain(coarse, fine, table, lanes, lab, cout, coords, K, (h, w), dev)
+        traj = torch.zeros(T, qp.shape[0], 2, dtype=torch.float32, device=dev)
+        if perm.numel():
+            traj[:, perm] = torch.cat(tracks, dim=1)
+        return traj
+
+    def _clip_weights_and_chain(self, coarse, fine, table, lanes, lab, cout, coords, K, image_hw, dev):
+        """fgvc_c2f_clip_weights over every job of ``table`` (in job slices of bounded workspace), then
+        fgvc_c2f_point_clip_tail_lanes over ``lanes``."""
+        cfg = self.cfg
+        n_c = coarse.H * coarse.W
+        jobs_dev, mem_feat, mem_label = table.device(dev)
+        jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4).contiguous()
+        n = len(table)
+        weights = torch.empty(n, n_c, K, dtype=torch.float32, device=dev)
+        rows = torch.empty(n, n_c, K, dtype=torch.int32, device=dev)
+        lib = _lib.load()
+        total = int(lib.fgvc_c2f_clip_workspace_bytes(_lib.ptr(jobs_host), 0, n, coarse.H, coarse.W, K))
+        # slices: bounded workspace, and at most 65535 window CTAs per coarse tile (<= 4 per memory entry)
+        n_mem = sum(j[2] - j[1] for j in table.jobs)
+        n_slices = max(-(-total // _CLIP_WS_BUDGET), -(-4 * n_mem // 65535), -(-n // 65535))
+        mode = _lib.MASK_CIRCLE if cfg.get("mask_mode", "circle") == "circle" else _lib.MASK_SQUARE
+        ws = None
+        for i in range(n_slices):
+            a, b = (n * i) // n_slices, (n * (i + 1)) // n_slices
+            need = int(lib.fgvc_c2f_clip_workspace_bytes(_lib.ptr(jobs_host), a, b, coarse.H, coarse.W, K))
+            if ws is None or ws.numel() < need:
+                ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            _lib.call("fgvc_c2f_clip_weights", _lib.ptr(coarse.buf), coarse.fmt, coarse.n_slots, coarse.H, coarse.W,
+                      coarse.C, _lib.ptr(fine.buf), fine.H, fine.W, fine.C, _lib.ptr(jobs_host), a, b, _lib.ptr(mem_feat),
+                      _lib.ptr(mem_label), int(cfg["neighbor_range"] // 2), mode, int(cfg.get("radius_fine", 12)), K,
+                      float(cfg["temperature"]), ctypes.c_void_p(weights.data_ptr() + 4 * a * n_c * K),
+                      ctypes.c_void_p(rows.data_ptr() + 4 * a * n_c * K), _lib.ptr(ws), need, int(self.engine_id),
+                      _lib.stream_ptr())
+        host = (_lib.C2FLane * len(lanes))(*lanes)
+        lanes_dev = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(dev)
+        maps = torch.empty(coarse.n_slots * max(ln.L for ln in lanes) * n_c, dtype=torch.float32, device=dev)  # NCHW scratch
+        barrier = torch.empty(256, dtype=torch.uint8, device=dev)
+        _lib.call("fgvc_c2f_point_clip_tail_lanes", _lib.ptr(weights), _lib.ptr(rows), K, 0, _lib.ptr(jobs_dev),
+                  _lib.ptr(jobs_host), _lib.ptr(lanes_dev), ctypes.c_void_p(ctypes.addressof(host)), len(lanes),
+                  coarse.H, coarse.W, fine.H, fine.W, _lib.ptr(lab), _lib.ptr(cout), int(image_hw[0]), int(image_hw[1]), 5,
+                  _lib.ptr(maps), _lib.ptr(coords), _lib.ptr(barrier), _lib.stream_ptr())
+

@@ -184,3 +184,45 @@ extern "C" int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* 
   }
   return FGVC_OK;
 }
+
+// The coarse-to-fine point tails of several recurrences of a clip (C2FPointTracker.track_queries): one multi-lane c2f
+// chain (c2f.cu), then per lane the NCHW copies of its coarse outputs and one K3 launch.
+extern "C" int fgvc_c2f_point_clip_tail_lanes(const float* weights, const int32_t* rows, int32_t K, int32_t job_base,
+                                              const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
+                                              const fgvc_c2f_lane* lanes_dev, const fgvc_c2f_lane* lanes_host,
+                                              int32_t n_lanes, int32_t Hc, int32_t Wc, int32_t Hf, int32_t Wf,
+                                              float* fine_lab, float* coarse_out, int32_t out_h, int32_t out_w,
+                                              int32_t coord_topk, float* maps_nchw, float* coords, void* barrier_ws,
+                                              void* stream) {
+  FGVC_CHECK_ARG(weights && rows && jobs_dev && jobs_host && lanes_dev && lanes_host && fine_lab && coarse_out &&
+                     maps_nchw && coords && barrier_ws, "fgvc_c2f_point_clip_tail_lanes: null pointer");
+  FGVC_CHECK_ARG(K >= 1 && K <= 16, "fgvc_c2f_point_clip_tail_lanes: topk=%d not in [1,16]", K);
+  FGVC_CHECK_ARG(n_lanes >= 1 && Hc > 0 && Wc > 0 && Hf > 0 && Wf > 0 && job_base >= 0,
+                 "fgvc_c2f_point_clip_tail_lanes: bad sizes");
+  for (int i = 0; i < n_lanes; ++i) {
+    const fgvc_c2f_lane& ln = lanes_host[i];
+    FGVC_CHECK_ARG(ln.job_begin >= job_base && ln.job_end > ln.job_begin,
+                   "fgvc_c2f_point_clip_tail_lanes: lane %d is empty or starts before job_base", i);
+    FGVC_CHECK_ARG(ln.L > 0 && ln.Lp >= ln.L && ln.Lp % 4 == 0 && ln.lab_offset >= 0 && ln.lab_offset % 4 == 0 &&
+                       ln.out_offset >= 0 && ln.out_offset % 4 == 0 && ln.coord_offset >= 0,
+                   "fgvc_c2f_point_clip_tail_lanes: bad label sizes or offsets in lane %d", i);
+    FGVC_CHECK_ARG(consecutive_slots(jobs_host, ln.job_begin, ln.job_end) >= 0,
+                   "fgvc_c2f_point_clip_tail_lanes: out_slots of lane %d must be consecutive", i);
+  }
+  const int nc = Hc * Wc;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = launch_c2f_chain_lanes(weights, rows, K, job_base, jobs_dev, lanes_dev, lanes_host, n_lanes, Hc, Wc, Hf, Wf,
+                                  fine_lab, coarse_out, reinterpret_cast<unsigned int*>(barrier_ws), st);
+  if (rc) return rc;
+  for (int i = 0; i < n_lanes; ++i) {
+    const fgvc_c2f_lane& ln = lanes_host[i];
+    rc = launch_labels_to_nchw_jobs(coarse_out + ln.out_offset, jobs_dev, ln.job_begin, ln.job_end, ln.Lp, ln.L, nc,
+                                    maps_nchw, st);
+    if (rc) return rc;
+    const int slot0 = consecutive_slots(jobs_host, ln.job_begin, ln.job_end);
+    rc = fgvc_heatmap_coords(maps_nchw + (int64_t)slot0 * ln.L * nc, (ln.job_end - ln.job_begin) * ln.L, Hc, Wc, out_h,
+                             out_w, coord_topk, coords + ln.coord_offset + (int64_t)slot0 * ln.L * 2, stream);
+    if (rc) return rc;
+  }
+  return FGVC_OK;
+}

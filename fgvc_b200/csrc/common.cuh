@@ -148,6 +148,63 @@ __device__ __forceinline__ bool in_mask(int dy, int dx, int r, int mode) {
 // largest |d| that can be in-mask
 __host__ __device__ inline int mask_reach(int r, int mode) { return mode == FGVC_MASK_CIRCLE ? r - 1 : r; }
 
+// grid barrier of a cooperative launch over a counter zeroed before the launch: the n-th barrier of every CTA
+// (n = 1, 2, ...) returns once all CTAs reached their n-th.  The caller's stores before it are visible after it to
+// ld.global.cg loads (the stores are fenced before the arrival).
+__device__ __forceinline__ void grid_barrier(unsigned int* counter, unsigned int n) {
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    atomicAdd(counter, 1u);
+    const unsigned int want = n * gridDim.x;
+    unsigned int seen;
+    do {
+      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(counter) : "memory");
+    } while (seen < want);
+  }
+  __syncthreads();
+}
+
+// F.interpolate(mode='bilinear', align_corners=False) taps of destination pixel (y, x) of an Hd x Wd map from an
+// Hs x Ws one: src = max((dst + 0.5) * in / out - 0.5, 0), second tap clamped to the last row / column
+struct BilinearTaps {
+  int p00, p01, p10, p11;     // source pixels (y0, x0), (y0, x1), (y1, x0), (y1, x1)
+  float ly, lx;
+};
+__device__ __forceinline__ BilinearTaps bilinear_taps(int y, int x, int Hs, int Ws, int Hd, int Wd) {
+  const float fy = fmaxf(((float)y + 0.5f) * ((float)Hs / (float)Hd) - 0.5f, 0.f);
+  const float fx = fmaxf(((float)x + 0.5f) * ((float)Ws / (float)Wd) - 0.5f, 0.f);
+  const int y0 = min((int)fy, Hs - 1), x0 = min((int)fx, Ws - 1);
+  const int y1 = min(y0 + 1, Hs - 1), x1 = min(x0 + 1, Ws - 1);
+  BilinearTaps t;
+  t.p00 = y0 * Ws + x0; t.p01 = y0 * Ws + x1; t.p10 = y1 * Ws + x0; t.p11 = y1 * Ws + x1;
+  t.ly = fy - (float)y0; t.lx = fx - (float)x0;
+  return t;
+}
+// same association as ATen's upsample_bilinear2d: (1-ly) * ((1-lx) * a + lx * b) + ly * ((1-lx) * c + lx * d)
+__device__ __forceinline__ float4 bilinear_mix(const BilinearTaps& t, const float4& a, const float4& b, const float4& c,
+                                               const float4& d) {
+  const float ly = t.ly, lx = t.lx, hy = 1.f - ly, hx = 1.f - lx;
+  float4 o;
+  o.x = hy * (hx * a.x + lx * b.x) + ly * (hx * c.x + lx * d.x);
+  o.y = hy * (hx * a.y + lx * b.y) + ly * (hx * c.y + lx * d.y);
+  o.z = hy * (hx * a.z + lx * b.z) + ly * (hx * c.z + lx * d.z);
+  o.w = hy * (hx * a.w + lx * b.w) + ly * (hx * c.w + lx * d.w);
+  return o;
+}
+
+// One job of a clip-level c2f fine stage (fgvc_c2f_clip_weights): where its coarse arg-max table, its floors and its
+// fine top-K lists live in the workspace, and which CTAs of the window-mode K1 launch are its (grid.y indices
+// [y_begin, y_begin + n_mem * chunks), entry-major).
+struct c2f_wjob {
+  fgvc_job job;
+  int32_t chunks;       // CTAs per (coarse tile, memory entry): c2f_window_chunks(Hc, Wc, n_mem)
+  int32_t y_begin;
+  int64_t best_off;     // elements: arg-max table [n_mem][Hc * Wc]
+  int64_t floor_off;    // elements: floors [Hc * Wc]
+  int64_t list_off;     // elements: lists [Hc * Wc][n_mem * chunks][K]
+};
+
 // host launchers implemented in the .cu files -------------------------------------------
 int launch_affinity_topk_simt(const void* bank, int fmt, int H, int W, int C, const fgvc_job* jobs, int n_jobs,
                               const int32_t* mem_feat, int radius, int mode, int K, int groups,
@@ -182,7 +239,16 @@ bool c2f_window_supported(int Hf, int Wf, int Cf, int K, int n_mem);
 int launch_c2f_window_tc16(const void* fine_bank, int n_slots, int Hc, int Wc, int Hf, int Wf, int Cf, int scale,
                            const fgvc_job& job, const int32_t* mem_feat, const int32_t* best, int rf, int K, int chunks,
                            float* floor_ws, float* tv, int32_t* ti, cudaStream_t st);
+int launch_c2f_window_tc16_jobs(const void* fine_bank, int n_slots, int Hc, int Wc, int Hf, int Wf, int Cf, int scale,
+                                const c2f_wjob* wjobs_dev, int n_wjobs, int n_y, const int32_t* mem_feat,
+                                const int32_t* best, int rf, int K, float* floor_ws, float* tv, int32_t* ti,
+                                cudaStream_t st);
 int c2f_window_chunks(int Hc, int Wc, int n_mem);
+bool c2f_use_window(int engine, int bank_format, int Hf, int Wf, int Cf, int K, int n_mem);
+int resident_ctas(const void* kernel, std::atomic<int>* cached, int* max_ctas);
+int launch_c2f_chain_lanes(const float* cw, const int32_t* crow, int K, int job_base, const fgvc_job* jobs_dev,
+                           const fgvc_c2f_lane* lanes_dev, const fgvc_c2f_lane* lanes_host, int n_lanes, int Hc, int Wc,
+                           int Hf, int Wf, float* fine_lab, float* coarse_out, unsigned int* barrier, cudaStream_t st);
 int launch_decode_jobs(const float* lab, const fgvc_job* jobs_dev, int job_begin, int job_end, int L, int Lp, int H,
                        int W, int out_h, int out_w, uint32_t* minmax, uint8_t* masks, cudaStream_t st);
 int launch_labels_harden(float* lab_slot, int n_pix, int L, int Lp, cudaStream_t st);

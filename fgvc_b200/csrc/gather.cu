@@ -307,19 +307,7 @@ gather_chain_kernel(const float* __restrict__ cw, const int32_t* __restrict__ cr
       }
     }
     // grid barrier: every CTA's stores of job j are visible before anyone starts job j + 1
-    if (j + 1 < n_jobs) {
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicAdd(barrier, 1u);
-        const unsigned int want = (unsigned int)(j + 1) * gridDim.x;
-        unsigned int seen;
-        do {
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(barrier) : "memory");
-        } while (seen < want);
-      }
-      __syncthreads();
-    }
+    if (j + 1 < n_jobs) grid_barrier(barrier, (unsigned int)(j + 1));
   }
 }
 
@@ -449,19 +437,7 @@ gather_chain_lanes_kernel(const float* __restrict__ cw, const int32_t* __restric
       }
     }
     // grid barrier: every CTA's stores of step s are visible before anyone starts step s + 1
-    if (s + 1 < n_steps) {
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicAdd(barrier, 1u);
-        const unsigned int want = (unsigned int)(s + 1) * gridDim.x;
-        unsigned int seen;
-        do {
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(barrier) : "memory");
-        } while (seen < want);
-      }
-      __syncthreads();
-    }
+    if (s + 1 < n_steps) grid_barrier(barrier, (unsigned int)(s + 1));
     l = next_lane(lanes, n_lanes, s + 1, 0);
   }
 }
@@ -492,7 +468,7 @@ static int launch_weights_t(const float* tv, const int32_t* ti, int k_in, int gr
 // co-resident CTAs of a 256-thread chain kernel on the calling thread's device (they spin on the grid barrier:
 // cooperative launch, sized from the occupancy; cached per device index, written once with the same value by any
 // thread)
-static int resident_ctas(const void* kernel, std::atomic<int>* cached, int* max_ctas) {
+int resident_ctas(const void* kernel, std::atomic<int>* cached, int* max_ctas) {
   int dev = 0;
   FGVC_CUDA(cudaGetDevice(&dev));
   *max_ctas = (dev >= 0 && dev < 64) ? cached[dev].load(std::memory_order_relaxed) : 0;

@@ -189,8 +189,8 @@ gaussian_labels_kernel(const float* __restrict__ pts, int P, int H, int W, int s
   dst[i] = v;
 }
 
-// bilinear up-sampling of a pixel-major label map (F.interpolate(mode='bilinear', align_corners=False) semantics:
-// src = max((dst + 0.5) * in / out - 0.5, 0), second tap clamped to the last row / column); one thread per
+// bilinear up-sampling of a pixel-major label map (F.interpolate(mode='bilinear', align_corners=False) semantics,
+// bilinear_taps / bilinear_mix in common.cuh); one thread per
 // (destination pixel, 4 channels): float4 loads and stores along the channel dimension are coalesced
 __global__ void __launch_bounds__(256)
 upsample_labels_kernel(const float* __restrict__ src, int Hs, int Ws, int Lp, float* __restrict__ dst, int Hd, int Wd) {
@@ -200,22 +200,11 @@ upsample_labels_kernel(const float* __restrict__ src, int Hs, int Ws, int Lp, fl
   const int l4 = (int)(i % l4n);
   const int pix = (int)(i / l4n);
   const int y = pix / Wd, x = pix - y * Wd;
-  const float fy = fmaxf(((float)y + 0.5f) * ((float)Hs / (float)Hd) - 0.5f, 0.f);
-  const float fx = fmaxf(((float)x + 0.5f) * ((float)Ws / (float)Wd) - 0.5f, 0.f);
-  const int y0 = min((int)fy, Hs - 1), x0 = min((int)fx, Ws - 1);
-  const int y1 = min(y0 + 1, Hs - 1), x1 = min(x0 + 1, Ws - 1);
-  const float ly = fy - (float)y0, lx = fx - (float)x0;
+  const BilinearTaps t = bilinear_taps(y, x, Hs, Ws, Hd, Wd);
   const float4* s4 = reinterpret_cast<const float4*>(src);
-  const float4 a = __ldg(s4 + (int64_t)(y0 * Ws + x0) * l4n + l4), b = __ldg(s4 + (int64_t)(y0 * Ws + x1) * l4n + l4);
-  const float4 c = __ldg(s4 + (int64_t)(y1 * Ws + x0) * l4n + l4), d = __ldg(s4 + (int64_t)(y1 * Ws + x1) * l4n + l4);
-  // same association as ATen's upsample_bilinear2d: (1-ly) * ((1-lx) * a + lx * b) + ly * ((1-lx) * c + lx * d)
-  const float hy = 1.f - ly, hx = 1.f - lx;
-  float4 o;
-  o.x = hy * (hx * a.x + lx * b.x) + ly * (hx * c.x + lx * d.x);
-  o.y = hy * (hx * a.y + lx * b.y) + ly * (hx * c.y + lx * d.y);
-  o.z = hy * (hx * a.z + lx * b.z) + ly * (hx * c.z + lx * d.z);
-  o.w = hy * (hx * a.w + lx * b.w) + ly * (hx * c.w + lx * d.w);
-  reinterpret_cast<float4*>(dst)[i] = o;
+  const float4 a = __ldg(s4 + (int64_t)t.p00 * l4n + l4), b = __ldg(s4 + (int64_t)t.p01 * l4n + l4);
+  const float4 c = __ldg(s4 + (int64_t)t.p10 * l4n + l4), d = __ldg(s4 + (int64_t)t.p11 * l4n + l4);
+  reinterpret_cast<float4*>(dst)[i] = bilinear_mix(t, a, b, c, d);
 }
 
 // hard propagation (vanilla_tracker.py:762-767): replace the soft labels of a slot by one_hot(argmax)

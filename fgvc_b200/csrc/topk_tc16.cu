@@ -64,6 +64,8 @@ struct Params {
   // window mode (K2 fine stage)
   int HQ, WQ, scale, rf, chunks;
   fgvc_job job;
+  const c2f_wjob* wjobs;            // several jobs in one launch (grid.y = their (entry, chunk) CTAs) or nullptr: `job`
+  int n_wjobs;
   const int32_t* best;              // [n_mem][HQ * WQ] coarse arg-max key pixel per memory entry
   const float* floor;               // [HQ * WQ] lower bound of the query's final K-th value (accumulator units) or nullptr
   float* tv;
@@ -233,9 +235,33 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
   // ---- this CTA's jobs and memory entries
   fgvc_tile_group tg;
   int e_lo, e_hi, og = 0;
+  // window mode: this CTA's job, memory entry (position in the job's list), chunk of the entry's boxes, and the
+  // job's arg-max table, floors and lists -- from the job table when the launch has several jobs
+  fgvc_job wjob = p.job;
+  int went = blockIdx.y, wchunk = blockIdx.z, wchunks = p.chunks;
+  const int32_t* wbest = p.best;
+  const float* wfloor = p.floor;
+  float* wtv = p.tv;
+  int32_t* wti = p.ti;
+  if (WIN && p.wjobs != nullptr) {
+    int lo = 0, hi = p.n_wjobs - 1;
+    while (lo < hi) {                                        // last job with y_begin <= blockIdx.y
+      const int mid = (lo + hi + 1) >> 1;
+      if (__ldg(&p.wjobs[mid].y_begin) <= (int)blockIdx.y) lo = mid; else hi = mid - 1;
+    }
+    const c2f_wjob& wj = p.wjobs[lo];
+    wjob = wj.job;
+    wchunks = wj.chunks;
+    went = ((int)blockIdx.y - wj.y_begin) / wchunks;
+    wchunk = ((int)blockIdx.y - wj.y_begin) - went * wchunks;
+    wbest = p.best + wj.best_off;
+    wfloor = p.floor != nullptr ? p.floor + wj.floor_off : nullptr;
+    wtv = p.tv + wj.list_off;
+    wti = p.ti + wj.list_off;
+  }
   if (WIN) {
     tg.job[0] = 0; tg.n_jobs = 1;
-    e_lo = p.job.mem_begin + blockIdx.y; e_hi = e_lo + 1;
+    e_lo = wjob.mem_begin + went; e_hi = e_lo + 1;
   } else {
     if (p.tgroups) {
       // heaviest groups first: in clip order the late jobs have the longest memory lists, and a launch that ends
@@ -373,7 +399,7 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
     int cy_lo = 1 << 30, cy_hi = -1, cx_lo = 1 << 30, cx_hi = -1;
     int my_cy = 0, my_cx = 0;
     if (qvalid) {
-      const int b = max(__ldg(p.best + (int64_t)blockIdx.y * nq_c + qy * p.WQ + qx), 0) % nq_c;
+      const int b = max(__ldg(wbest + (int64_t)went * nq_c + qy * p.WQ + qx), 0) % nq_c;
       my_cy = cy_lo = cy_hi = (b / p.WQ) * p.scale;
       my_cx = cx_lo = cx_hi = (b % p.WQ) * p.scale;
     }
@@ -413,7 +439,7 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
         int kept = 0;
         for (int i = lane; i < words; i += 32) kept += __popc(cover[i]);
         kept = __reduce_add_sync(0xffffffffu, kept);
-        const int k_lo = (int)((int64_t)kept * blockIdx.z / p.chunks), k_hi = (int)((int64_t)kept * (blockIdx.z + 1) / p.chunks);
+        const int k_lo = (int)((int64_t)kept * wchunk / wchunks), k_hi = (int)((int64_t)kept * (wchunk + 1) / wchunks);
         int seen = 0;
         for (int base = 0; base < total; base += 32) {
           const int i = base + lane;
@@ -540,7 +566,7 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
       // both query parts -> tensor memory, two fp16 channels per 32-bit cell (lower channel in the low half).  The four
       // warps that share a TMEM lane quarter split the channels: 16 cells (64 B of the row) per tcgen05.st.
       // Window mode: the row is the FINE query feature at (scale * qy, scale * qx)   (local_attention.py:785)
-      const int q_slot = WIN ? p.job.q_slot : (jb >= 0 ? p.jobs[jb].q_slot : 0);
+      const int q_slot = WIN ? wjob.q_slot : (jb >= 0 ? p.jobs[jb].q_slot : 0);
       const int qpix = !qvalid ? 0 : (WIN ? (qy * p.scale) * p.W + qx * p.scale : qy * p.W + qx);
       const int64_t part = (int64_t)p.n_pix * p.C;
       const __half* row = bank + (int64_t)q_slot * 2 * part + (int64_t)qpix * p.C;
@@ -565,8 +591,8 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
     volatile float* thr_mine = thr_sh + m * EPI_WG + wg;
     // every list of this query may start from a floor that K genuine candidates are known to reach (the caller's
     // guarantee): [coarse query] in window mode, [job][query pixel] otherwise
-    *thr_mine = (p.floor != nullptr && qvalid)
-                    ? __ldg(p.floor + (WIN ? (int64_t)qy * p.WQ + qx : (int64_t)jb * p.n_pix + qy * p.W + qx))
+    *thr_mine = (wfloor != nullptr && qvalid)
+                    ? __ldg(wfloor + (WIN ? (int64_t)qy * p.WQ + qx : (int64_t)jb * p.n_pix + qy * p.W + qx))
                     : -INFINITY;
     asm volatile("bar.sync 1, %0;" ::"n"(128 * EPI_WG) : "memory");
     // Warpgroup wg owns the key rows wg (and wg + 4 when a box has 8 rows) of every box: a static assignment, so the
@@ -679,10 +705,10 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
         const uint32_t* blist = boxes + li * MAX_BOXES;
         int upos_e, cy = qy, cx = qx;
         if constexpr (WIN) {
-          upos_e = qvalid ? e - p.job.mem_begin : -1;
+          upos_e = qvalid ? e - wjob.mem_begin : -1;
           // this lane's window centre in this memory entry: scale * (coarse arg-max key)   (local_attention.py:835-845)
           if (qvalid) {
-            const int bq = max(__ldg(p.best + (int64_t)(e - p.job.mem_begin) * nq_c + qy * p.WQ + qx), 0) % nq_c;
+            const int bq = max(__ldg(wbest + (int64_t)(e - wjob.mem_begin) * nq_c + qy * p.WQ + qx), 0) % nq_c;
             cy = (bq / p.WQ) * p.scale;
             cx = (bq % p.WQ) * p.scale;
           }
@@ -727,11 +753,11 @@ affinity_topk_tc16_kernel(const __grid_constant__ CUtensorMap tmap_k, const __ha
         }
       const int q = qy * qW + qx;
       int64_t o;
-      if (WIN) o = ((int64_t)q * ((p.job.mem_end - p.job.mem_begin) * p.chunks) + (blockIdx.y * p.chunks + blockIdx.z)) * p.k_out;
+      if (WIN) o = ((int64_t)q * ((wjob.mem_end - wjob.mem_begin) * wchunks) + (went * wchunks + wchunk)) * p.k_out;
       else o = (((int64_t)jb * p.lists_per_job + og) * p.n_pix + q) * p.k_out;
 #pragma unroll
       for (int i = 0; i < K; ++i)
-        if (i < p.k_out) { p.tv[o + i] = top.v[i] * FGVC_F16_ACC_INV; p.ti[o + i] = top.id[i]; }
+        if (i < p.k_out) { wtv[o + i] = top.v[i] * FGVC_F16_ACC_INV; wti[o + i] = top.id[i]; }
     }
   }
   tc_fence_before();
@@ -1041,14 +1067,20 @@ bool c2f_window_supported(int Hf, int Wf, int Cf, int K, int n_mem) {
 constexpr int FLOOR_SAMPLES = 5;
 __global__ void __launch_bounds__(256)
 c2f_floor_kernel(const __half* __restrict__ bank, int Hf, int Wf, int Cf, int HQ, int WQ, int scale, int rf,
-                 fgvc_job job, const int32_t* __restrict__ ent, const int32_t* __restrict__ best, int K,
-                 float* __restrict__ floor_out) {
+                 fgvc_job job, const c2f_wjob* __restrict__ wjobs, const int32_t* __restrict__ ent,
+                 const int32_t* __restrict__ best, int K, float* __restrict__ floor_out) {
+  // several jobs (wjobs): job = blockIdx.y of the table
   // one CTA per coarse query, one warp per memory entry (8 at a time), the 5 samples of an entry in flight together
   __shared__ float samp[tc16::TW_MAX_MEM * FLOOR_SAMPLES];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int q = blockIdx.x, nq = HQ * WQ;
   const int qy = q / WQ, qx = q - qy * WQ;
   const int64_t n_pix = (int64_t)Hf * Wf;
+  if (wjobs != nullptr) {
+    job = wjobs[blockIdx.y].job;
+    best += wjobs[blockIdx.y].best_off;
+    floor_out += wjobs[blockIdx.y].floor_off;
+  }
   const __half* qrow = bank + ((int64_t)job.q_slot * 2 * n_pix + (int64_t)(qy * scale) * Wf + qx * scale) * Cf;
   const __half* qlo = qrow + n_pix * Cf;
   const int n_mem = job.mem_end - job.mem_begin;
@@ -1121,9 +1153,12 @@ int c2f_window_chunks(int Hc, int Wc, int n_mem) {
 
 // fine stage of c2f as a window-mode K1: top-K lists tv / ti [Hc * Wc][n_mem * chunks][K] over the in-window, in-image
 // fine keys (idx = memory position * Hf * Wf + fine key pixel).  best: [n_mem][Hc * Wc] coarse arg-max keys.
-int launch_c2f_window_tc16(const void* fine_bank, int n_slots, int Hc, int Wc, int Hf, int Wf, int Cf, int scale,
-                           const fgvc_job& job, const int32_t* mem_feat, const int32_t* best, int rf, int K, int chunks,
-                           float* floor_ws, float* tv, int32_t* ti, cudaStream_t st) {
+// wjobs_dev == nullptr: the one job `job`, grid (tiles, n_mem, chunks); else the n_wjobs jobs of the table (the device
+// copy of wjobs_host), grid (tiles, n_y): best / floor_ws / tv / ti are then bases that the table's offsets add to.
+static int launch_window(const void* fine_bank, int n_slots, int Hc, int Wc, int Hf, int Wf, int Cf, int scale,
+                         const fgvc_job& job, const c2f_wjob* wjobs_dev, int n_wjobs, int n_y, const int32_t* mem_feat,
+                         const int32_t* best, int rf, int K, int chunks, float* floor_ws, float* tv, int32_t* ti,
+                         cudaStream_t st) {
   using namespace tc16;
   Params p = {};
   p.H = Hf; p.W = Wf; p.C = Cf; p.n_pix = Hf * Wf;
@@ -1139,6 +1174,7 @@ int launch_c2f_window_tc16(const void* fine_bank, int n_slots, int Hc, int Wc, i
   p.chunks = chunks;
   p.tiles_x = cdiv(Wc, p.QW);
   p.job = job; p.ent = mem_feat; p.best = best; p.tv = tv; p.ti = ti;
+  p.wjobs = wjobs_dev; p.n_wjobs = n_wjobs;
   static const int exp_win = getenv("FGVC_TC16_EXP_WIN") ? atoi(getenv("FGVC_TC16_EXP_WIN")) : 0;   // perf experiments only
   p.exp_flags = exp_win;
   // worst case (scattered arg-max keys): the entry lists every box of the frame
@@ -1152,13 +1188,35 @@ int launch_c2f_window_tc16(const void* fine_bank, int n_slots, int Hc, int Wc, i
   if (rc) return rc;
   static const bool no_floor = getenv("FGVC_C2F_NOFLOOR") != nullptr;     // perf experiments only
   if (floor_ws != nullptr && !no_floor) {
-    c2f_floor_kernel<<<Hc * Wc, 256, 0, st>>>(reinterpret_cast<const __half*>(fine_bank), Hf, Wf, Cf, Hc, Wc, scale,
-                                                      rf, job, mem_feat, best, K, floor_ws);
+    c2f_floor_kernel<<<dim3(Hc * Wc, wjobs_dev != nullptr ? n_wjobs : 1), 256, 0, st>>>(
+        reinterpret_cast<const __half*>(fine_bank), Hf, Wf, Cf, Hc, Wc, scale, rf, job, wjobs_dev, mem_feat, best, K,
+        floor_ws);
     FGVC_LAUNCH_CHECK();
     p.floor = floor_ws;
   }
   dim3 grid(cdiv(Hc, p.QH) * p.tiles_x, job.mem_end - job.mem_begin, chunks);
+  if (wjobs_dev != nullptr) grid = dim3(cdiv(Hc, p.QH) * p.tiles_x, n_y, 1);
   return launch_by_k<1, true>(mk, fine_bank, p, grid, K, st);
+}
+
+int launch_c2f_window_tc16(const void* fine_bank, int n_slots, int Hc, int Wc, int Hf, int Wf, int Cf, int scale,
+                           const fgvc_job& job, const int32_t* mem_feat, const int32_t* best, int rf, int K, int chunks,
+                           float* floor_ws, float* tv, int32_t* ti, cudaStream_t st) {
+  return launch_window(fine_bank, n_slots, Hc, Wc, Hf, Wf, Cf, scale, job, nullptr, 0, 0, mem_feat, best, rf, K, chunks,
+                       floor_ws, tv, ti, st);
+}
+
+// the fine stage of the jobs of a c2f_wjob table in one window-mode K1 launch (and one floor launch): every job gets
+// the lists, chunk for chunk, that launch_c2f_window_tc16 gives it alone
+int launch_c2f_window_tc16_jobs(const void* fine_bank, int n_slots, int Hc, int Wc, int Hf, int Wf, int Cf, int scale,
+                                const c2f_wjob* wjobs_dev, int n_wjobs, int n_y, const int32_t* mem_feat,
+                                const int32_t* best, int rf, int K, float* floor_ws, float* tv, int32_t* ti,
+                                cudaStream_t st) {
+  FGVC_CHECK_ARG(n_wjobs >= 1 && n_wjobs <= 65535 && n_y >= 1 && n_y <= 65535,
+                 "c2f window engine: %d jobs / %d (job, entry, chunk) CTAs per tile, at most 65535", n_wjobs, n_y);
+  fgvc_job none = {0, 0, 1, 0};
+  return launch_window(fine_bank, n_slots, Hc, Wc, Hf, Wf, Cf, scale, none, wjobs_dev, n_wjobs, n_y, mem_feat, best, rf,
+                       K, 1, floor_ws, tv, ti, st);
 }
 
 }  // namespace fgvc

@@ -675,6 +675,26 @@ def memory_frames(t, precede_frames, with_first=True, first=0):
     return ([first] + win) if with_first else win
 
 
+def query_job_table(t0s, T, precede_frames, with_first, bidirectional, unmasked):
+    """Jobs of point groups queried at frames ``t0s`` of a T-frame clip (the grouping of VanillaTracker.forward_test,
+    vanilla_tracker.py:249-295).  Per group the forward jobs t0+1 .. T-1 (memory_frames with first = t0), then with
+    ``bidirectional`` the backward jobs t0-1 .. 0: the forward tracker on the time-reversed clip (query frame T-1-t0)
+    mapped back to frame indices, memory [t0] + [min(t0, t + precede), ..., t + 1].  ``unmasked(mem)``: leading
+    memory entries without the radius mask.  Returns (JobTable, spans) with spans[i] = (first job, t0) of group i."""
+    table = JobTable()
+    spans = []
+    for t0 in t0s:
+        spans.append((len(table), t0))
+        for t in range(t0 + 1, T):
+            mem = memory_frames(t, precede_frames, with_first, first=t0)
+            table.add(t, mem, mem, t, unmasked=unmasked(mem))
+        if bidirectional:
+            for t in range(t0 - 1, -1, -1):
+                mem = [T - 1 - r for r in memory_frames(T - 1 - t, precede_frames, with_first, first=T - 1 - t0)]
+                table.add(t, mem, mem, t, unmasked=unmasked(mem))
+    return table, spans
+
+
 def c2f_propagate(coarse, fine, table, job_index, fine_labels, radius, radius_fine, K, temperature,
                   mask_mode="circle", engine=_lib.ENGINE_AUTO):
     dev = coarse.buf.device

@@ -20,7 +20,7 @@ import torch.nn as nn
 
 from . import _lib, engine
 from .encoder import build_backbone
-from .engine import FeatureBank, JobTable, LabelBank
+from .engine import FeatureBank, LabelBank
 
 
 class _Cfg(dict):
@@ -219,19 +219,9 @@ class VanillaTracker(nn.Module):
                 bank.load_frames(feats, 0, normalize=normalize)
 
         bidirectional = bool(cfg.get("bidirectional", False))
-        table = JobTable()
-        spans = []   # per group: (first job, t0); forward jobs t0+1 .. T-1, then (bidirectional) backward jobs t0-1 .. 0
-        for t0, _ in groups:
-            spans.append((len(table), t0))
-            for t in range(t0 + 1, T):
-                mem = engine.memory_frames(t, precede, with_first_mem, first=t0)
-                table.add(t, mem, mem, t, unmasked=len(mem) if nr is None else unmasked_first)
-            if bidirectional:
-                # the forward tracker on the time-reversed clip (query frame T-1-t0), mapped back to frame indices:
-                # memory [t0] + [min(t0, t + precede), ..., t + 1]
-                for t in range(t0 - 1, -1, -1):
-                    mem = [T - 1 - r for r in engine.memory_frames(T - 1 - t, precede, with_first_mem, first=T - 1 - t0)]
-                    table.add(t, mem, mem, t, unmasked=len(mem) if nr is None else unmasked_first)
+        # per group: (first job, t0); forward jobs t0+1 .. T-1, then (bidirectional) backward jobs t0-1 .. 0
+        table, spans = engine.query_job_table([t0 for t0, _ in groups], T, precede, with_first_mem, bidirectional,
+                                              lambda mem: len(mem) if nr is None else unmasked_first)
         outs = []
         radius = (nr // 2) if nr is not None else 1
         shared = None

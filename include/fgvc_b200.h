@@ -97,6 +97,21 @@ typedef struct fgvc_lane {
   int64_t coord_offset;  /* floats from coords to the lane's tracks */
 } fgvc_lane;
 
+/* One lane of fgvc_c2f_point_clip_tail_lanes: one coarse-to-fine recurrence of a clip (the forward or the backward
+ * track of a point group) = the consecutive jobs [job_begin, job_end) in recurrence order, with their out_slots running
+ * consecutively up or down.  Its fine label bank is fine_lab + lab_offset ([slot][Hf*Wf][Lp]), its coarse outputs go
+ * to coarse_out + out_offset ([slot][Hc*Wc][Lp]) and its tracks to coords + coord_offset ([slot][L][2]).  Two lanes
+ * may share a fine bank when neither reads a slot the other writes. */
+typedef struct fgvc_c2f_lane {
+  int32_t job_begin;
+  int32_t job_end;
+  int32_t L;             /* label channels (points) of the lane */
+  int32_t Lp;            /* bank row length: L rounded up to a multiple of 4 */
+  int64_t lab_offset;    /* floats from fine_lab to the lane's fine label bank */
+  int64_t out_offset;    /* floats from coarse_out to the lane's coarse-output bank */
+  int64_t coord_offset;  /* floats from coords to the lane's tracks */
+} fgvc_c2f_lane;
+
 /* Job-packed query tiles of the fp16 tensor engine (fgvc_affinity_topk_packed): a tile group = up to 4 jobs that
  * share most of their memory frames (consecutive query frames of a clip) and are multiplied against each key box
  * together.  Memory entries [u_begin, u_end) of the union tables list every (frame, mask flag) any job of the group
@@ -334,6 +349,43 @@ FGVC_API int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, in
                        int32_t mask_mode, int32_t radius_fine, int32_t K, float temperature,
                        const float* fine_lab_bank, int32_t Lp, float* out, float* scratch_val,
                        int32_t* scratch_idx, int64_t scratch_elems, int32_t engine, void* stream);
+
+/* Coarse-to-fine propagation of a whole clip (C2FPointTracker.track_queries), split where the recurrence is.  The
+ * coarse arg-max, the fine window top-K, the zero-padded candidates and the soft-max weights of a job depend on the
+ * features only; only the gather of fine label rows and the up-sampling of its result are recurrent.
+ *
+ * fgvc_c2f_clip_weights: for the jobs [job_begin, job_end) of jobs_host, the label-independent half of
+ * fgvc_c2f_propagate, bit for bit what that call computes for each job: (weight, fine label row) pairs
+ * weights[job - job_begin][Hc*Wc][K], rows[...] (row = mem_label_slot * Hf*Wf + fine pixel, -1 = zero-padded or empty
+ * candidate, weight 0 = unused).  Enqueued as one coarse K1 per distinct memory length (K = 1, groups = length, over a
+ * length-sorted copy of the jobs), then for all jobs at once either the floor kernel + one window-mode K1 + one weights
+ * kernel (the tensor-core fine stage) or one weights-only launch of the one-warp-per-candidate fine kernel.  The launch
+ * count does not depend on the number of jobs.  ws: fgvc_c2f_clip_workspace_bytes(...) bytes (job tables, arg-max
+ * tables, floors and fine lists of the range; a caller bounds it by calling in job slices).  jobs_host is read by the
+ * call only; the job tables it needs on the device are copied into ws. */
+FGVC_API int64_t fgvc_c2f_clip_workspace_bytes(const fgvc_job* jobs_host, int32_t job_begin, int32_t job_end,
+                       int32_t Hc, int32_t Wc, int32_t K);
+FGVC_API int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t bank_format, int32_t n_slots, int32_t Hc, int32_t Wc,
+                       int32_t C, const void* fine_bank, int32_t Hf, int32_t Wf, int32_t Cf,
+                       const fgvc_job* jobs_host, int32_t job_begin, int32_t job_end,
+                       const int32_t* mem_feat_slot, const int32_t* mem_label_slot, int32_t radius,
+                       int32_t mask_mode, int32_t radius_fine, int32_t K, float temperature, float* weights,
+                       int32_t* rows, void* ws, int64_t ws_bytes, int32_t engine, void* stream);
+
+/* The recurrent half for several lanes (fgvc_c2f_lane) at once: ONE cooperative kernel whose step s, for every lane
+ * still running, (1) gathers job s's coarse output out[q] = sum_k w * fine_lab[row] (the FMA sequence of the gather of
+ * fgvc_c2f_propagate) into the lane's coarse-output bank at the job's out_slot, grid barrier, (2) up-samples it into
+ * the job's out_slot of the lane's fine bank (the taps of fgvc_upsample_labels), grid barrier -- twice the longest
+ * lane's length in barriers.  Then per lane the NCHW copies of its coarse outputs into maps_nchw[slot][L][Hc*Wc] and
+ * ONE K3 launch over all its (frame, point) maps into coords[slot][L][2].  weights / rows: fgvc_c2f_clip_weights of
+ * the jobs from job_base on (every lane's jobs inside).  maps_nchw: scratch of (largest out_slot + 1) x (largest L) x
+ * Hc*Wc floats, reused lane after lane.  barrier_ws: 256 bytes of scratch (zeroed by the call).  Each lane's tracks
+ * and coarse outputs are bit for bit what fgvc_c2f_propagate + fgvc_upsample_labels + K3 give frame by frame. */
+FGVC_API int fgvc_c2f_point_clip_tail_lanes(const float* weights, const int32_t* rows, int32_t K, int32_t job_base,
+                       const fgvc_job* jobs_dev, const fgvc_job* jobs_host, const fgvc_c2f_lane* lanes_dev,
+                       const fgvc_c2f_lane* lanes_host, int32_t n_lanes, int32_t Hc, int32_t Wc, int32_t Hf,
+                       int32_t Wf, float* fine_lab, float* coarse_out, int32_t out_h, int32_t out_w,
+                       int32_t coord_topk, float* maps_nchw, float* coords, void* barrier_ws, void* stream);
 
 #ifdef __cplusplus
 }
