@@ -77,74 +77,61 @@ static int consecutive_slots(const fgvc_job* jobs_host, int job_begin, int job_e
   return dir > 0 ? s0 : s0 - (n - 1);
 }
 
-// Point tracking tail: the gather chain over jobs [job_begin, job_end) with an NCHW copy of every
-// propagated frame into maps_nchw[slot][L][H*W], then ONE K3 launch (fused up-sample / soft-argmax)
-// over all (frame, point) maps of the range: coords[slot][L][2].  The out_slots of the range must
-// be consecutive (they are frame indices), ascending or descending.
-static int point_clip_tail_impl(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
-                                    const fgvc_job* jobs_dev, const fgvc_job* jobs_host, int32_t job_begin,
-                                    int32_t job_end, const int32_t* mem_label_slot, int32_t H, int32_t W,
-                                    float temperature, int32_t flags, float* lab_bank, int32_t Lp, int32_t L, int32_t out_h,
-                                    int32_t out_w, int32_t coord_topk, float* maps_nchw, float* coords,
-                                    void* chain_ws, int64_t chain_ws_bytes, const int32_t* pair_ref, void* stream) {
-  FGVC_CHECK_ARG(jobs_dev && jobs_host && maps_nchw && coords && lab_bank, "fgvc_point_clip_tail: null pointer");
-  FGVC_CHECK_ARG(job_end > job_begin, "fgvc_point_clip_tail: empty job range");
+// NCHW copies of jobs [job_begin, job_end) of a label bank into maps_nchw[slot][L][H*W], then ONE K3 launch (fused
+// up-sample / soft-argmax) over all their (frame, point) maps into coords[slot][L][2].  The caller checked that the
+// out_slots are consecutive.
+static int nchw_and_coords(const float* bank, const fgvc_job* jobs_dev, const fgvc_job* jobs_host, int job_begin,
+                           int job_end, int Lp, int L, int H, int W, int out_h, int out_w, int coord_topk,
+                           float* maps_nchw, float* coords, void* stream) {
   const int n_pix = H * W;
+  int rc = launch_labels_to_nchw_jobs(bank, jobs_dev, job_begin, job_end, Lp, L, n_pix, maps_nchw, (cudaStream_t)stream);
+  if (rc) return rc;
   const int slot0 = consecutive_slots(jobs_host, job_begin, job_end);
-  FGVC_CHECK_ARG(slot0 >= 0, "fgvc_point_clip_tail: out_slots must be consecutive");
-  FGVC_CHECK_ARG(pair_ref == nullptr || chain_ws != nullptr, "fgvc_point_clip_tail_shared: needs the chain workspace");
-  if (chain_ws != nullptr && (job_end - job_begin > 1 || pair_ref != nullptr)) {
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = launch_gather_chain(topk_val, topk_idx, K, groups, jobs_dev, job_begin, job_end, mem_label_slot, pair_ref,
-                                 n_pix, temperature, flags, lab_bank, Lp, chain_ws, chain_ws_bytes, st);
-    if (rc) return rc;
-    rc = launch_labels_to_nchw_jobs(lab_bank, jobs_dev, job_begin, job_end, Lp, L, n_pix, maps_nchw, st);
-    if (rc) return rc;
-  } else {
-    for (int j = job_begin; j < job_end; ++j) {
-      const int slot = jobs_host[j].out_slot;
-      int rc = fgvc_gather_labels(topk_val, topk_idx, K, groups, jobs_dev, j, j + 1, mem_label_slot, n_pix,
-                                  temperature, flags, lab_bank, Lp, stream);
-      if (rc) return rc;
-      rc = fgvc_labels_to_nchw(lab_bank, slot, Lp, L, n_pix, maps_nchw + (int64_t)slot * L * n_pix, stream);
-      if (rc) return rc;
-    }
-  }
   return fgvc_heatmap_coords(maps_nchw + (int64_t)slot0 * L * n_pix, (job_end - job_begin) * L, H, W, out_h, out_w,
                              coord_topk, coords + (int64_t)slot0 * L * 2, stream);
 }
 
+// Point tracking tail: the gather chain over jobs [job_begin, job_end) with an NCHW copy of every
+// propagated frame into maps_nchw[slot][L][H*W], then ONE K3 launch over all (frame, point) maps of the
+// range: coords[slot][L][2].  The out_slots of the range must be consecutive (they are frame indices),
+// ascending or descending.
 extern "C" int fgvc_point_clip_tail(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
                                     const fgvc_job* jobs_dev, const fgvc_job* jobs_host, int32_t job_begin,
                                     int32_t job_end, const int32_t* mem_label_slot, int32_t H, int32_t W,
                                     float temperature, int32_t flags, float* lab_bank, int32_t Lp, int32_t L, int32_t out_h,
                                     int32_t out_w, int32_t coord_topk, float* maps_nchw, float* coords,
                                     void* chain_ws, int64_t chain_ws_bytes, void* stream) {
-  return point_clip_tail_impl(topk_val, topk_idx, K, groups, jobs_dev, jobs_host, job_begin, job_end, mem_label_slot, H, W,
-                              temperature, flags, lab_bank, Lp, L, out_h, out_w, coord_topk, maps_nchw, coords, chain_ws,
-                              chain_ws_bytes, nullptr, stream);
+  FGVC_CHECK_ARG(jobs_dev && jobs_host && maps_nchw && coords && lab_bank, "fgvc_point_clip_tail: null pointer");
+  FGVC_CHECK_ARG(job_end > job_begin, "fgvc_point_clip_tail: empty job range");
+  const int n_pix = H * W;
+  const int slot0 = consecutive_slots(jobs_host, job_begin, job_end);
+  FGVC_CHECK_ARG(slot0 >= 0, "fgvc_point_clip_tail: out_slots must be consecutive");
+  if (chain_ws != nullptr && job_end - job_begin > 1) {
+    int rc = launch_gather_chain(topk_val, topk_idx, K, groups, jobs_dev, job_begin, job_end, mem_label_slot, nullptr,
+                                 n_pix, temperature, flags, lab_bank, Lp, chain_ws, chain_ws_bytes, (cudaStream_t)stream);
+    if (rc) return rc;
+    return nchw_and_coords(lab_bank, jobs_dev, jobs_host, job_begin, job_end, Lp, L, H, W, out_h, out_w, coord_topk,
+                           maps_nchw, coords, stream);
+  }
+  for (int j = job_begin; j < job_end; ++j) {
+    const int slot = jobs_host[j].out_slot;
+    int rc = fgvc_gather_labels(topk_val, topk_idx, K, groups, jobs_dev, j, j + 1, mem_label_slot, n_pix,
+                                temperature, flags, lab_bank, Lp, stream);
+    if (rc) return rc;
+    rc = fgvc_labels_to_nchw(lab_bank, slot, Lp, L, n_pix, maps_nchw + (int64_t)slot * L * n_pix, stream);
+    if (rc) return rc;
+  }
+  return fgvc_heatmap_coords(maps_nchw + (int64_t)slot0 * L * n_pix, (job_end - job_begin) * L, H, W, out_h, out_w,
+                             coord_topk, coords + (int64_t)slot0 * L * 2, stream);
 }
 
-// Same with SHARED top-k lists: the jobs of several with_first groups that have the same query frame look at the
-// same memory frames except their first one, so K1 ran once per (query frame, memory frame) pair
-// (one list per pair) and pair_ref[e] names the list of memory entry e of these jobs (indices into
-// topk_val / topk_idx in units of H*W*K).  Needs the chain workspace.
-extern "C" int fgvc_point_clip_tail_shared(const float* topk_val, const int32_t* topk_idx, int32_t K,
-                                           const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
-                                           int32_t job_begin, int32_t job_end, const int32_t* mem_label_slot, int32_t H,
-                                           int32_t W, float temperature, int32_t flags, float* lab_bank, int32_t Lp,
-                                           int32_t L, int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
-                                           float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream) {
-  FGVC_CHECK_ARG(pair_ref != nullptr, "fgvc_point_clip_tail_shared: null pair_ref");
-  return point_clip_tail_impl(topk_val, topk_idx, K, 1, jobs_dev, jobs_host, job_begin, job_end, mem_label_slot, H, W,
-                              temperature, flags, lab_bank, Lp, L, out_h, out_w, coord_topk, maps_nchw, coords, chain_ws,
-                              chain_ws_bytes, pair_ref, stream);
-}
-
-// Several independent point tails of one clip (bidirectional tracking: the forward and the backward track of every
-// point group), each lane bit for bit its own point_clip_tail_impl: one multi-lane gather chain for all of them
-// (gather.cu), then per lane the NCHW copies and one K3 launch -- bandwidth work, where one launch per lane costs
-// nothing worth saving.
+// The point tails of the independent recurrences of a clip (every forward and backward track of every point group),
+// each lane bit for bit fgvc_point_clip_tail over its jobs with the chain workspace: one gather chain for all of them,
+// then per lane the NCHW copies and one K3 launch -- bandwidth work, where one launch per lane costs nothing worth
+// saving.  A single lane runs the multi-lane chain (gather.cu) too: with it a whole one-lane tail is not slower than
+// with gather_chain_kernel on a B200 at 1000 W (128 x 128 map, 256 points x 49 frames: 1.60 against 1.76 ms; 1024
+// points x 249 frames: 38.0 against 38.4 ms; 160 x 160, 15 points x 31 frames: 0.34 against 0.46 ms).  pair_ref names the shared per-(query frame, memory
+// frame) lists of every memory entry, or is NULL.
 extern "C" int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
                                           const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
                                           const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int32_t n_lanes,
@@ -174,12 +161,8 @@ extern "C" int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* 
   if (rc) return rc;
   for (int i = 0; i < n_lanes; ++i) {
     const fgvc_lane& ln = lanes_host[i];
-    rc = launch_labels_to_nchw_jobs(lab_bank + ln.lab_offset, jobs_dev, ln.job_begin, ln.job_end, ln.Lp, ln.L, n_pix,
-                                    maps_nchw, st);
-    if (rc) return rc;
-    const int slot0 = consecutive_slots(jobs_host, ln.job_begin, ln.job_end);
-    rc = fgvc_heatmap_coords(maps_nchw + (int64_t)slot0 * ln.L * n_pix, (ln.job_end - ln.job_begin) * ln.L, H, W, out_h,
-                             out_w, coord_topk, coords + ln.coord_offset + (int64_t)slot0 * ln.L * 2, stream);
+    rc = nchw_and_coords(lab_bank + ln.lab_offset, jobs_dev, jobs_host, ln.job_begin, ln.job_end, ln.Lp, ln.L, H, W,
+                         out_h, out_w, coord_topk, maps_nchw, coords + ln.coord_offset, stream);
     if (rc) return rc;
   }
   return FGVC_OK;
@@ -209,19 +192,14 @@ extern "C" int fgvc_c2f_point_clip_tail_lanes(const float* weights, const int32_
     FGVC_CHECK_ARG(consecutive_slots(jobs_host, ln.job_begin, ln.job_end) >= 0,
                    "fgvc_c2f_point_clip_tail_lanes: out_slots of lane %d must be consecutive", i);
   }
-  const int nc = Hc * Wc;
   cudaStream_t st = (cudaStream_t)stream;
   int rc = launch_c2f_chain_lanes(weights, rows, K, job_base, jobs_dev, lanes_dev, lanes_host, n_lanes, Hc, Wc, Hf, Wf,
                                   fine_lab, coarse_out, reinterpret_cast<unsigned int*>(barrier_ws), st);
   if (rc) return rc;
   for (int i = 0; i < n_lanes; ++i) {
     const fgvc_c2f_lane& ln = lanes_host[i];
-    rc = launch_labels_to_nchw_jobs(coarse_out + ln.out_offset, jobs_dev, ln.job_begin, ln.job_end, ln.Lp, ln.L, nc,
-                                    maps_nchw, st);
-    if (rc) return rc;
-    const int slot0 = consecutive_slots(jobs_host, ln.job_begin, ln.job_end);
-    rc = fgvc_heatmap_coords(maps_nchw + (int64_t)slot0 * ln.L * nc, (ln.job_end - ln.job_begin) * ln.L, Hc, Wc, out_h,
-                             out_w, coord_topk, coords + ln.coord_offset + (int64_t)slot0 * ln.L * 2, stream);
+    rc = nchw_and_coords(coarse_out + ln.out_offset, jobs_dev, jobs_host, ln.job_begin, ln.job_end, ln.Lp, ln.L, Hc, Wc,
+                         out_h, out_w, coord_topk, maps_nchw, coords + ln.coord_offset, stream);
     if (rc) return rc;
   }
   return FGVC_OK;

@@ -299,27 +299,18 @@ FGVC_API int fgvc_point_clip_tail(const float* topk_val, const int32_t* topk_idx
                          int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
                          float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream);
 
-/* Point tail on SHARED top-k lists (the grouping loop of VanillaTracker.forward_test, vanilla_tracker.py:249-295, which
- * re-runs forward_test_main per unique query frame).  Jobs of different with_first groups with the same query frame use the same
- * memory frames except their first one, so K1 is run once per query frame over the union of those frames with one
- * group per memory entry (fgvc_affinity_topk, groups = longest union): one list per (query frame, memory frame) pair.
- * pair_ref[e] = index of the list (in units of H*W*K elements of topk_val / topk_idx) for memory entry e of the
- * per-group job table; the tail merges each job's lists, re-basing the positions to the job's own memory list.
- * chain_ws is required. */
-FGVC_API int fgvc_point_clip_tail_shared(const float* topk_val, const int32_t* topk_idx, int32_t K,
-                         const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
-                         int32_t job_begin, int32_t job_end, const int32_t* mem_label_slot, int32_t H, int32_t W,
-                         float temperature, int32_t flags, float* lab_bank, int32_t Lp, int32_t L,
-                         int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
-                         float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream);
-
-/* Point tail of SEVERAL independent recurrences of one clip (bidirectional tracking: every point group is tracked
- * forward from its query frame and, on the time-reversed clip, backward to frame 0).  Each lane (fgvc_lane) is the
- * point tail above over its own job range, bank and tracks, and gives bit for bit what that tail gives; but the
- * chains of all lanes run together: ONE weight launch over the jobs of every lane, then ONE cooperative kernel whose
- * step s gathers job s of every lane still running, with one grid barrier per step -- the longest lane's length of
- * barriers instead of the sum over the lanes.  The NCHW copies and K3 then run per lane.  pair_ref: NULL (lists of
- * `groups` parts per job) or the shared lists of fgvc_point_clip_tail_shared (groups must be 1).
+/* Point tails of the independent recurrences of one clip: every point group tracked forward from its query frame and,
+ * with bidirectional tracking, backward to frame 0 on the time-reversed clip.  Each lane (fgvc_lane) is the point tail
+ * above over its own job range, bank and tracks, and gives bit for bit what that tail gives with the chain workspace;
+ * but the chains of all lanes run together: ONE weight launch over the jobs of every lane, then ONE cooperative kernel
+ * whose step s gathers job s of every lane still running, with one grid barrier per step -- the longest lane's length
+ * of barriers instead of the sum over the lanes.  The NCHW copies and K3 then run per lane.
+ * pair_ref: NULL (lists of `groups` parts per job) or SHARED top-k lists (groups must be 1).  Jobs of different
+ * with_first groups with the same query frame use the same memory frames except their first one, so K1 may run once
+ * per query frame over the union of those frames with one group per memory entry (fgvc_affinity_topk, groups =
+ * longest union): one list per (query frame, memory frame) pair.  pair_ref[e] = index of the list (in units of H*W*K
+ * elements of topk_val / topk_idx) for memory entry e of the per-group job table; the tail merges each job's lists,
+ * re-basing the positions to the job's own memory list.
  * lanes_dev / lanes_host: the lane table in device and host memory.  maps_nchw: scratch of (largest out_slot + 1) x
  * (largest L) x H*W floats, reused lane after lane.  chain_ws (required): fgvc_chain_workspace_bytes(je - jb, H*W, K)
  * bytes, [jb, je) = the smallest job range holding every lane. */

@@ -107,25 +107,35 @@ def test_tracks_match_the_oracle_on_both_sides():
 GEOMS = {"one_pass": (9, 24, 32, (3, 7, 13)), "short_rows": (9, 24, 32, (2, 2, 2)), "large_map": (5, 200, 200, (2, 5, 3))}
 
 
+def _per_lane(real):
+    """engine.point_tail_lanes with one call, hence one gather chain, per lane"""
+    def tail(lists, pair_ref, table, lanes, *a, **kw):
+        for lane in lanes:
+            real(lists, pair_ref, table, [lane], *a, **kw)
+    return tail
+
+
+@pytest.mark.parametrize("bidirectional", [True, False])
 @pytest.mark.parametrize("share", ["1", "0"])
 @pytest.mark.parametrize("geom", sorted(GEOMS))
-def test_lanes_are_an_exact_rescheduling(monkeypatch, geom, share):
+def test_lanes_are_an_exact_rescheduling(monkeypatch, geom, share, bidirectional):
+    from fgvc_b200 import engine
     T, H, W, sizes = GEOMS[geom]
     g = torch.Generator().manual_seed(54)
     feats = _coherent(g, T, 64, H, W).cuda()
     t0s = (0, T // 2, T - 1)
     groups = [(t0, _points(g, n, H, W)) for t0, n in zip(t0s, sizes)]
     monkeypatch.setenv("FGVC_NO_SHARE", share)
-    monkeypatch.delenv("FGVC_NO_LANES", raising=False)
-    lanes = _run(BASE, feats, groups)
-    monkeypatch.setenv("FGVC_NO_LANES", "1")
-    per_lane = _run(BASE, feats, groups)
+    lanes = _run(BASE, feats, groups, bidirectional=bidirectional)
+    monkeypatch.setattr(engine, "point_tail_lanes", _per_lane(engine.point_tail_lanes))
+    per_lane = _run(BASE, feats, groups, bidirectional=bidirectional)
     for a, b in zip(lanes, per_lane):
         assert torch.equal(a, b)
 
 
 def test_chain_is_two_launches_whatever_the_groups_and_length(monkeypatch):
-    """weights + lane chain: 2 launches; only the NCHW copy and K3 of every lane (2 each) grow with the lanes."""
+    """weights + lane chain: 2 launches, one tail call per clip, bidirectional and forward-only; only the NCHW copy and
+    K3 of every lane (2 each) grow with the lanes."""
     from fgvc_b200 import _lib, engine
     seen = []
     real = engine.point_tail_lanes
@@ -136,13 +146,15 @@ def test_chain_is_two_launches_whatever_the_groups_and_length(monkeypatch):
         seen.append((_lib.launch_count() - before, len(lanes)))
 
     monkeypatch.setattr(engine, "point_tail_lanes", counted)
-    monkeypatch.delenv("FGVC_NO_LANES", raising=False)
-    g = torch.Generator().manual_seed(55)
-    for T, t0s in ((6, (0, 3)), (12, (0, 3, 6, 9, 11)), (20, (2, 9, 17))):
-        feats = _coherent(g, T, 64, 16, 24).cuda()
-        _run(BASE, feats, [(t0, _points(g, 4, 16, 24)) for t0 in t0s])
-    assert [n for _, n in seen] == [3, 8, 6]
-    assert all(d - 2 * n == 2 for d, n in seen), seen
+    # forward-only: no lane for a group queried at the last frame
+    for bidirectional, n_lanes in ((True, [3, 8, 6]), (False, [2, 4, 3])):
+        seen.clear()
+        g = torch.Generator().manual_seed(55)
+        for T, t0s in ((6, (0, 3)), (12, (0, 3, 6, 9, 11)), (20, (2, 9, 17))):
+            feats = _coherent(g, T, 64, 16, 24).cuda()
+            _run(BASE, feats, [(t0, _points(g, 4, 16, 24)) for t0 in t0s], bidirectional=bidirectional)
+        assert [n for _, n in seen] == n_lanes, bidirectional
+        assert all(d - 2 * n == 2 for d, n in seen), (bidirectional, seen)
 
 
 def test_pinned_host_features_equal_the_resident_run():

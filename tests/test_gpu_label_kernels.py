@@ -8,6 +8,7 @@ in fp32 (in / out rounded once, then one fused multiply-add).  A float64 coordin
 8e-6 at s = 100, far more than the fp32 rounding of the values, so the references take the coordinate as the kernels
 compute it and do everything after it in float64.
 """
+import ctypes
 import math
 
 import numpy as np
@@ -213,6 +214,27 @@ def _run_tail(kind, lists, table, lab0, H, W, L, tau, flags, chain, out_hw):
     return lab, maps, out
 
 
+def _run_lanes(n_lanes, lists, table, lab0, H, W, L, tau, flags, out_hw):
+    """fgvc_point_clip_tail_lanes with ``n_lanes`` lanes over all jobs of ``table``, each on its own copy of the bank.
+    Returns (label banks [n_lanes, T, n_pix, Lp], NCHW maps of the last lane, coordinates [n_lanes, T, L, 2])."""
+    T, n_pix, Lp = lab0.shape
+    n = len(table)
+    lab = lab0.repeat(n_lanes, 1, 1)
+    jobs, _, mem_label = table.device(DEV)
+    jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4)
+    nbytes = int(_lib.load().fgvc_chain_workspace_bytes(n, n_pix, lists.K))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=DEV)
+    maps = torch.full((T, L, n_pix), NAN, device=DEV)
+    out = torch.zeros(n_lanes, T, L, 2, dtype=torch.float32, device=DEV)
+    host = (_lib.Lane * n_lanes)(*[_lib.Lane(0, n, L, Lp, i * T * n_pix * Lp, i * T * L * 2) for i in range(n_lanes)])
+    lanes = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(DEV)
+    call("fgvc_point_clip_tail_lanes", ptr(lists.val), ptr(lists.idx), lists.K, lists.groups, None, ptr(jobs),
+         ptr(jobs_host), ptr(lanes), ctypes.c_void_p(ctypes.addressof(host)), n_lanes, ptr(mem_label), H, W, float(tau),
+         int(flags), ptr(lab), out_hw[0], out_hw[1], 5, ptr(maps), ptr(out), ptr(ws), nbytes, stream_ptr())
+    torch.cuda.synchronize()
+    return lab.view(n_lanes, T, n_pix, Lp), maps, out
+
+
 def _check_chain(seed, T, H, W, L, K, groups, case):
     zp, flags, tau, lo, hi = CHAIN_CASES[case]
     flags |= _lib.zero_pad_flags(2, W) if zp else 0
@@ -243,15 +265,23 @@ def _check_chain(seed, T, H, W, L, K, groups, case):
             err = float((lab[t].double() - ref[t]).abs().max())
             assert err <= 1e-5 * scale, (kind, t, err)
             assert torch.equal(maps[t], lab[t, :, :L].t())
+        if kind == "point":
+            # the lanes entry, which the trackers call: one lane, and two lanes on two copies of the bank, give what the
+            # chained point tail gives
+            for n_lanes in (1, 2):
+                labs, maps2, outs = _run_lanes(n_lanes, lists, table, lab0, H, W, L, tau, flags, out_hw)
+                assert torch.equal(maps2[1:], maps[1:]), n_lanes
+                for i in range(n_lanes):
+                    assert torch.equal(labs[i], lab) and torch.equal(outs[i], out), (n_lanes, i)
 
 
 @pytest.mark.parametrize("case", list(CHAIN_CASES))
 @pytest.mark.parametrize("K", [1, 7, 16])
 @pytest.mark.parametrize("L", [1, 2, 3, 4, 5, 11, 70])
 def test_gather_chain_matches_per_frame_and_float64(L, K, case):
-    """Mask and point clip tails with and without the chain workspace: label bank, NCHW maps, masks and coordinates
-    bit-identical, every frame within 1e-5 of the float64 recurrence (later frames read earlier out_slots, so a missing
-    barrier or a stale read shows).  On this 13 x 17 map L <= 4 takes the multi-pass branch with a ragged last chunk
+    """Mask and point clip tails with and without the chain workspace, and the point tail's lanes entry with one and
+    two lanes: label bank, NCHW maps, masks and coordinates bit-identical, every frame within 1e-5 of the float64
+    recurrence (later frames read earlier out_slots, so a missing barrier or a stale read shows).  On this 13 x 17 map L <= 4 takes the multi-pass branch with a ragged last chunk
     and L >= 5 the one-pass branch; both follow from the launch rule without an occupancy figure."""
     H, W, T = 13, 17, 5
     ctas, per = _chain_grid(H * W, engine.pad4(L), _sms())

@@ -1,11 +1,13 @@
-"""Bidirectional point tracking at the config-3 geometry: ms per clip of K1, the recurrent tail and the whole
-propagate_points call, for forward-only tracking, bidirectional tracking with one gather chain per lane
-(FGVC_NO_LANES=1) and bidirectional tracking with the multi-lane chain, alternated in one process.
+"""Point tracking of strided query groups at the config-3 geometry: ms per clip of K1, the recurrent tail and the whole
+propagate_points call, and the peak device memory of the call, for forward-only and bidirectional tracking, each with
+every lane of the clip in one multi-lane gather chain (as the tracker runs it) and with one chain per lane, alternated
+in one process.
 
 Clip: 256 x 256 frames -> 128 x 128 x 256 features of a random-init ResNet-18 (strides 1,1,1,4), T = 50, radius 15,
 precede 5, top-k 10, temperature 0.07; TAP-Vid strided queries: 256 points at every 5th frame (10 groups).
 K1 = the affinity/top-k launches (engine.K1_TIMING); tail = CUDA events from the first point-tail call to the end of
-the last one; total = the whole call.  Prints one JSON object with the card name and its power limit.
+the last one; total = the whole call.  Prints one JSON object with the card name and its power limit, and whether
+the two schedules gave the same tracks bit for bit.
 
     python tools/bidir_bench.py [--reps 5]
 """
@@ -24,7 +26,7 @@ from fgvc_b200 import _lib, engine, synthetic as S  # noqa: E402
 
 T, HW, STEP, P = 50, 256, 5, 256
 CFG = dict(precede_frames=5, topk=10, temperature=0.07, neighbor_range=30, with_first=True, with_first_neighbor=True)
-VARIANTS = ("forward", "bidir_no_lanes", "bidir_lanes")
+VARIANTS = ("forward_lanes", "forward_per_lane", "bidir_lanes", "bidir_per_lane")
 
 
 def card():
@@ -54,16 +56,25 @@ class TailEvents:
             self.last.record()
 
 
+def per_lane(real):
+    """engine.point_tail_lanes with one call, hence one gather chain, per lane (as tests/test_gpu_bidirectional.py)"""
+    def tail(lists, pair_ref, table, lanes, *a, **kw):
+        for lane in lanes:
+            real(lists, pair_ref, table, [lane], *a, **kw)
+    return tail
+
+
 def run(variant, feats, groups):
-    os.environ.pop("FGVC_NO_LANES", None)
-    if variant == "bidir_no_lanes":
-        os.environ["FGVC_NO_LANES"] = "1"
     trk = fgvc_b200.VanillaTracker(backbone=torch.nn.Identity(),
-                                   test_cfg=dict(CFG, bidirectional=variant != "forward"))
+                                   test_cfg=dict(CFG, bidirectional=variant.startswith("bidir")))
     tail = TailEvents()
+    lanes = engine.point_tail_lanes
+    if variant.endswith("per_lane"):
+        engine.point_tail_lanes = per_lane(lanes)
     _lib.call = engine.call = tail
     engine.K1_TIMING = []
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.reset_peak_memory_stats()
     try:
         e0.record()
         out = trk.propagate_points(feats, groups, (HW, HW))
@@ -71,10 +82,10 @@ def run(variant, feats, groups):
         torch.cuda.synchronize()
     finally:
         _lib.call = engine.call = tail._call
+        engine.point_tail_lanes = lanes
         k1, engine.K1_TIMING = engine.K1_TIMING, None
-        os.environ.pop("FGVC_NO_LANES", None)
     return out, dict(k1_ms=sum(a.elapsed_time(b) for a, b in k1), tail_ms=tail.first.elapsed_time(tail.last),
-                     total_ms=e0.elapsed_time(e1))
+                     total_ms=e0.elapsed_time(e1), peak_memory_gb=torch.cuda.max_memory_allocated() / 1e9)
 
 
 def main():
@@ -97,12 +108,15 @@ def main():
             times[v].append(run(v, feats, groups)[1])
     res = dict(card=card(), feat_hw=list(feats.shape[2:]), channels=feats.shape[1], frames=T, groups=len(groups),
                points=P * len(groups), config=CFG, reps=args.reps,
-               lanes_equal_no_lanes=all(torch.equal(a, b) for a, b in zip(outs["bidir_lanes"], outs["bidir_no_lanes"])),
+               forward_lanes_equal_per_lane=all(torch.equal(a, b) for a, b in
+                                                zip(outs["forward_lanes"], outs["forward_per_lane"])),
+               bidir_lanes_equal_per_lane=all(torch.equal(a, b) for a, b in
+                                              zip(outs["bidir_lanes"], outs["bidir_per_lane"])),
                forward_half_equal=all(torch.equal(a[t0:], b[t0:]) for (t0, _), a, b in
-                                      zip(groups, outs["bidir_lanes"], outs["forward"])),
-               peak_memory_gb=torch.cuda.max_memory_allocated() / 1e9)
+                                      zip(groups, outs["bidir_lanes"], outs["forward_lanes"])))
     for v in VARIANTS:
         res[v] = {k: statistics.median(t[k] for t in times[v]) for k in ("k1_ms", "tail_ms", "total_ms")}
+        res[v]["peak_memory_gb"] = max(t["peak_memory_gb"] for t in times[v])
         res[v]["tail_ms_min_max"] = [min(t["tail_ms"] for t in times[v]), max(t["tail_ms"] for t in times[v])]
     print(json.dumps(res, indent=1))
 
