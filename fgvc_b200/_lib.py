@@ -83,9 +83,9 @@ SIGNATURES = {
     "fgvc_point_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, I, P, P, P, L64, P]),
     "fgvc_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, P, I, P, I, I, F, I, P, I, I, I, P, P, P, L64, P]),
     "fgvc_c2f_scratch_elems": (L64, [I, I]),
-    "fgvc_c2f_propagate": (I, [P, I, I, I, I, I, P, I, I, I, P, P, P, P, I, I, I, I, F, P, I, P, P, P, L64, I, P]),
+    "fgvc_c2f_propagate": (I, [P, I, I, I, I, I, P, I, I, I, I, P, P, P, P, I, I, I, I, F, P, I, P, P, P, L64, I, P]),
     "fgvc_c2f_clip_workspace_bytes": (L64, [P, I, I, I, I, I]),
-    "fgvc_c2f_clip_weights": (I, [P, I, I, I, I, I, P, I, I, I, P, I, I, P, P, I, I, I, I, F, P, P, P, L64, I, P]),
+    "fgvc_c2f_clip_weights": (I, [P, I, I, I, I, I, P, I, I, I, I, P, I, I, P, P, I, I, I, I, F, P, P, P, L64, I, P]),
     "fgvc_c2f_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, I, I, I, I, I, P, P, I, I, I, P, P, P, P]),
 }
 

@@ -16,13 +16,17 @@ around the genuine operator (tests/golden/c2f_driver.npz):
 Everything stays resident in HBM across frames: both feature banks are built once per clip (two K0 launches), the fine
 label bank holds every frame, a frame costs one coarse K1 (k = 1 per memory frame), one window-mode K1 on the tensor
 cores, the c2f tail, one up-sampling kernel and K3.
+
+``C2FTracker`` is the drop-in model around it (``eval_arc='B200C2FTracker'``): one encoder pass feeds a coarse and a
+fine bank, each in its own format, and ``C2FPointTracker.track_banks`` tracks the clip's query groups.
 """
 import ctypes
 
 import torch
 
-from . import _lib, engine
+from . import _lib, apis, engine
 from .engine import FeatureBank, JobTable, LabelBank
+from .tracker import VanillaTracker
 
 # bound of the list workspace of one fgvc_c2f_clip_weights call (the host calls it in job slices beyond): ~1.5 MB per
 # job at 32^2 coarse / 128^2 fine, precede 5, K 10 -- a strided 50-frame clip tracked both ways fits one slice
@@ -163,6 +167,28 @@ class C2FPointTracker:
         fine = FeatureBank(T, Cf, Hf, Wf, dev, split=split)
         coarse.load_frames(feats_coarse.to(dev, non_blocking=True).float(), 0, normalize=normalize)
         fine.load_frames(feats_fine.to(dev, non_blocking=True).float(), 0, normalize=normalize)
+        return self.track_banks(coarse, fine, query_points, image_hw)
+
+    @torch.no_grad()
+    def track_banks(self, coarse, fine, query_points, image_hw, shard=None):
+        """The clip path of ``track_queries`` over two loaded ``FeatureBank``s, each in its own format: coarse
+        [T, C, Hc, Wc], fine [T, Cf, s Hc, s Wc] (e.g. a TF32 coarse bank at C = 512 and an F16 fine bank at Cf = 256,
+        as ``C2FTracker`` encodes them).  query_points [P, 3] (t, x, y); returns traj [T, P, 2] float32 CUDA in the
+        input point order, with the semantics of ``track_queries``.
+
+        ``shard=(rank, world)``: the two-phase split of ``VanillaTracker.propagate_points`` over the default process
+        group.  Phase 1 runs fgvc_c2f_clip_weights for this rank's job range (``apis.frame_shard``) into its slot of the
+        (weight, row) buffers, which are all-gathered; phase 2 runs the lanes chain for this rank's slice of every
+        group's points (``apis.point_shard``), and the tracks are all-gathered.  Every rank returns the full result,
+        bit for bit that of ``world = 1``."""
+        cfg = self.cfg
+        T, Hc, Wc, Hf, Wf = coarse.n_slots, coarse.H, coarse.W, fine.H, fine.W
+        assert fine.n_slots == T and Hf % Hc == 0 and Wf % Wc == 0 and Hf // Hc == Wf // Wc, \
+            "fine grid must be s x the coarse grid"
+        h, w = image_hw
+        dev = coarse.buf.device
+        stride_f = h // Hf
+        rank, world = shard if shard is not None else (0, 1)
 
         qp = query_points.to(device=dev, dtype=torch.float32)
         qt = qp[:, 0].round().long()
@@ -174,65 +200,92 @@ class C2FPointTracker:
                                               lambda mem: unmasked_first)
         K = int(cfg["topk"])
         n_c, n_f = Hc * Wc, Hf * Wf
+        # phase 1: the (weight, fine label row) pairs of this rank's jobs, then of every job
+        lo, hi, per = apis.frame_shard(len(table), rank, world)
+        weights = torch.empty(per * world, n_c, K, dtype=torch.float32, device=dev)
+        rows = torch.empty(per * world, n_c, K, dtype=torch.int32, device=dev)
+        if hi > lo:
+            self._clip_weights(coarse, fine, table, lo, hi, K, weights, rows, dev)
+        apis.gather_job_lists(weights, per, rank, world)
+        apis.gather_job_lists(rows, per, rank, world)
+
+        # phase 2: per group, this rank's slice of its points (all of them at world = 1)
         sizes = [int(o.numel()) for o in order]
-        lab = torch.empty(sum(T * n_f * engine.pad4(P) for P in sizes), dtype=torch.float32, device=dev)
-        cout = torch.empty(sum(T * n_c * engine.pad4(P) for P in sizes), dtype=torch.float32, device=dev)
-        coords = torch.zeros(sum(T * P * 2 for P in sizes), dtype=torch.float32, device=dev)
+        parts = [apis.point_shard(P, rank, world) for P in sizes]
+        mine = [b - a for a, b in parts]
         perm = torch.cat(order) if order else torch.zeros(0, dtype=torch.long, device=dev)
         pts_all = qp[perm, 1:].contiguous()
         c0_all = engine.gaussian_coords(pts_all, (h, w)) if pts_all.shape[0] else None
+        lab = torch.empty(sum(T * n_f * engine.pad4(P) for P in mine), dtype=torch.float32, device=dev)
+        cout = torch.empty(sum(T * n_c * engine.pad4(P) for P in mine), dtype=torch.float32, device=dev)
+        coords = torch.zeros(sum(T * P * 2 for P in mine), dtype=torch.float32, device=dev)
         lanes, tracks = [], []
         lab_off = out_off = c_off = p_off = 0
-        for (j0, t0), P in zip(spans, sizes):
+        for (j0, t0), P_all, (a, _), P in zip(spans, sizes, parts, mine):
             track = coords[c_off:c_off + T * P * 2].view(T, P, 2)
             tracks.append(track)
-            labels = LabelBank(T, P, Hf, Wf, dev, buf=lab[lab_off:lab_off + T * n_f * engine.pad4(P)])
-            labels.put_gaussians(pts_all[p_off:p_off + P], t0, stride_f)
-            track[t0] = c0_all[p_off:p_off + P]
-            n_fw, n_bw = T - t0 - 1, (t0 if bidirectional else 0)
-            # forward lane, backward lane: they share the group's banks (both read slot t0, they write disjoint slots)
-            for jb, je in ((j0, j0 + n_fw), (j0 + n_fw, j0 + n_fw + n_bw)):
-                if je > jb:
-                    lanes.append(_lib.C2FLane(jb, je, P, engine.pad4(P), lab_off, out_off, c_off))
+            if P:
+                labels = LabelBank(T, P, Hf, Wf, dev, buf=lab[lab_off:lab_off + T * n_f * engine.pad4(P)])
+                labels.put_gaussians(pts_all[p_off + a:p_off + a + P], t0, stride_f)
+                track[t0] = c0_all[p_off + a:p_off + a + P]
+                n_fw, n_bw = T - t0 - 1, (t0 if bidirectional else 0)
+                # forward lane, backward lane: they share the group's banks (both read slot t0, they write disjoint
+                # slots)
+                for jb, je in ((j0, j0 + n_fw), (j0 + n_fw, j0 + n_fw + n_bw)):
+                    if je > jb:
+                        lanes.append(_lib.C2FLane(jb, je, P, engine.pad4(P), lab_off, out_off, c_off))
             lab_off += T * n_f * engine.pad4(P)
             out_off += T * n_c * engine.pad4(P)
             c_off += T * P * 2
-            p_off += P
+            p_off += P_all
         if lanes:
-            self._clip_weights_and_chain(coarse, fine, table, lanes, lab, cout, coords, K, (h, w), dev)
+            self._chain(weights, rows, table, lanes, coarse, fine, lab, cout, coords, K, (h, w), dev)
+        if world > 1:
+            pads = [-(-n // world) for n in sizes]
+            local = torch.zeros(T, sum(pads), 2, dtype=torch.float32, device=dev)
+            off = 0
+            for tr, pad in zip(tracks, pads):
+                local[:, off:off + tr.shape[1]] = tr
+                off += pad
+            tracks = apis.gather_point_tracks(local, sizes, rank, world)
         traj = torch.zeros(T, qp.shape[0], 2, dtype=torch.float32, device=dev)
         if perm.numel():
             traj[:, perm] = torch.cat(tracks, dim=1)
         return traj
 
-    def _clip_weights_and_chain(self, coarse, fine, table, lanes, lab, cout, coords, K, image_hw, dev):
-        """fgvc_c2f_clip_weights over every job of ``table`` (in job slices of bounded workspace), then
-        fgvc_c2f_point_clip_tail_lanes over ``lanes``."""
+    def _clip_weights(self, coarse, fine, table, lo, hi, K, weights, rows, dev):
+        """fgvc_c2f_clip_weights over the jobs [lo, hi) of ``table``, in job slices of bounded workspace, into rows
+        [lo, hi) of ``weights`` / ``rows``."""
         cfg = self.cfg
         n_c = coarse.H * coarse.W
-        jobs_dev, mem_feat, mem_label = table.device(dev)
+        _, mem_feat, mem_label = table.device(dev)
         jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4).contiguous()
-        n = len(table)
-        weights = torch.empty(n, n_c, K, dtype=torch.float32, device=dev)
-        rows = torch.empty(n, n_c, K, dtype=torch.int32, device=dev)
         lib = _lib.load()
-        total = int(lib.fgvc_c2f_clip_workspace_bytes(_lib.ptr(jobs_host), 0, n, coarse.H, coarse.W, K))
+        total = int(lib.fgvc_c2f_clip_workspace_bytes(_lib.ptr(jobs_host), lo, hi, coarse.H, coarse.W, K))
         # slices: bounded workspace, and at most 65535 window CTAs per coarse tile (<= 4 per memory entry)
-        n_mem = sum(j[2] - j[1] for j in table.jobs)
+        n_mem = sum(j[2] - j[1] for j in table.jobs[lo:hi])
+        n = hi - lo
         n_slices = max(-(-total // _CLIP_WS_BUDGET), -(-4 * n_mem // 65535), -(-n // 65535))
         mode = _lib.MASK_CIRCLE if cfg.get("mask_mode", "circle") == "circle" else _lib.MASK_SQUARE
         ws = None
         for i in range(n_slices):
-            a, b = (n * i) // n_slices, (n * (i + 1)) // n_slices
+            a, b = lo + (n * i) // n_slices, lo + (n * (i + 1)) // n_slices
             need = int(lib.fgvc_c2f_clip_workspace_bytes(_lib.ptr(jobs_host), a, b, coarse.H, coarse.W, K))
             if ws is None or ws.numel() < need:
                 ws = torch.empty(need, dtype=torch.uint8, device=dev)
             _lib.call("fgvc_c2f_clip_weights", _lib.ptr(coarse.buf), coarse.fmt, coarse.n_slots, coarse.H, coarse.W,
-                      coarse.C, _lib.ptr(fine.buf), fine.H, fine.W, fine.C, _lib.ptr(jobs_host), a, b, _lib.ptr(mem_feat),
-                      _lib.ptr(mem_label), int(cfg["neighbor_range"] // 2), mode, int(cfg.get("radius_fine", 12)), K,
-                      float(cfg["temperature"]), ctypes.c_void_p(weights.data_ptr() + 4 * a * n_c * K),
+                      coarse.C, _lib.ptr(fine.buf), fine.fmt, fine.H, fine.W, fine.C, _lib.ptr(jobs_host), a, b,
+                      _lib.ptr(mem_feat), _lib.ptr(mem_label), int(cfg["neighbor_range"] // 2), mode,
+                      int(cfg.get("radius_fine", 12)), K, float(cfg["temperature"]),
+                      ctypes.c_void_p(weights.data_ptr() + 4 * a * n_c * K),
                       ctypes.c_void_p(rows.data_ptr() + 4 * a * n_c * K), _lib.ptr(ws), need, int(self.engine_id),
                       _lib.stream_ptr())
+
+    def _chain(self, weights, rows, table, lanes, coarse, fine, lab, cout, coords, K, image_hw, dev):
+        """fgvc_c2f_point_clip_tail_lanes over ``lanes`` (the weights and rows of every job of ``table``)."""
+        n_c = coarse.H * coarse.W
+        jobs_dev, _, _ = table.device(dev)
+        jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4).contiguous()
         host = (_lib.C2FLane * len(lanes))(*lanes)
         lanes_dev = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(dev)
         maps = torch.empty(coarse.n_slots * max(ln.L for ln in lanes) * n_c, dtype=torch.float32, device=dev)  # NCHW scratch
@@ -242,3 +295,87 @@ class C2FPointTracker:
                   coarse.H, coarse.W, fine.H, fine.W, _lib.ptr(lab), _lib.ptr(cout), int(image_hw[0]), int(image_hw[1]), 5,
                   _lib.ptr(maps), _lib.ptr(coords), _lib.ptr(barrier), _lib.stream_ptr())
 
+
+_EXPECTED_BACKBONE = "backbone=dict(type='ResNet', depth=18, strides=(1, 1, 1, 4), out_indices=(2, 3), pool_type='none')"
+
+
+class C2FTracker(VanillaTracker):
+    """Coarse-to-fine point tracker as a drop-in model (``eval_arc='B200C2FTracker'``, BASELINE config 3-(ii)):
+    VanillaTracker's constructor and ``forward_test`` contract, the clip path of ``C2FPointTracker.track_banks``.
+
+    One encoder pass gives both levels: the backbone returns exactly two, the lower ``out_index`` is the fine level and
+    the higher the coarse level, with fine H, W = s x coarse H, W.  With the shipped eval backbone (ResNet-18,
+    ``strides=(1, 1, 1, 4)``, ``pool_type='none'``) and ``out_indices=(2, 3)``, a 256^2 clip gives layer 3 at 128^2 x
+    256 channels and layer 4 at 32^2 x 512 channels: s = 4.  Each level goes into its own FeatureBank, K0 of encoder
+    chunk i overlapped with the encoder of chunk i + 1 (``encode_to_bank``), and each bank takes its own
+    ``engine.default_split``: the coarse bank TF32 at C = 512 (the 3xTF32 engine), the fine bank F16 at Cf = 256 (the
+    tensor-core window-mode fine stage); ``test_cfg.split`` forces one format for both.
+
+    test_cfg keys: those of ``C2FPointTracker`` (precede_frames, topk, temperature, neighbor_range -- the coarse
+    radius --, radius_fine, with_first, with_first_neighbor, with_norm, split, mask_mode, bidirectional) and
+    VanillaTracker's batch_step, encoder_channels_last, engine.  ``with_first`` is also the grouping key of
+    ``forward_test``, as in VanillaTracker.  Keys of VanillaTracker that the c2f path does not implement raise
+    NotImplementedError when set to a non-default value."""
+
+    def __init__(self, backbone, head=None, train_cfg=None, test_cfg=None, init_cfg=None):
+        super().__init__(backbone, head=head, train_cfg=train_cfg, test_cfg=test_cfg, init_cfg=init_cfg)
+        cfg = self.test_cfg
+        if cfg.get("test_mode", "v1") != "v1":
+            raise NotImplementedError("C2FTracker: test_mode v2 is not built (the c2f operator is a v1 operator)")
+        if cfg.get("sim_mode", "dot_product") != "dot_product":
+            raise NotImplementedError("C2FTracker: only sim_mode='dot_product' is built")
+        for key in ("hard_prop", "stride_sample"):
+            if cfg.get(key, False):
+                raise NotImplementedError(f"C2FTracker: test_cfg.{key} is not built")
+        for key in ("topk", "neighbor_range"):
+            if cfg.get(key) is None:
+                raise NotImplementedError(f"C2FTracker needs test_cfg.{key} (the c2f path has no {key}=None form)")
+
+    def extract_feat(self, imgs):
+        """imgs [n,3,h,w] -> [fine, coarse] encoder levels; raises ValueError unless the backbone gives exactly two
+        levels with fine H, W = s x coarse H, W for one integer s."""
+        x = self.backbone(imgs)
+        levels = list(x) if isinstance(x, (tuple, list)) else [x]
+        if len(levels) != 2:
+            raise ValueError(f"C2FTracker needs a backbone with exactly two output levels (fine, coarse), got "
+                             f"{len(levels)}: use e.g. {_EXPECTED_BACKBONE}")
+        (Hf, Wf), (Hc, Wc) = levels[0].shape[-2:], levels[1].shape[-2:]
+        if Hf % Hc or Wf % Wc or Hf // Hc != Wf // Wc:
+            raise ValueError(f"C2FTracker: the fine level ({Hf}x{Wf}, lower out_index) must be s times the coarse level "
+                             f"({Hc}x{Wc}) in H and W for one integer s: use e.g. {_EXPECTED_BACKBONE}")
+        return levels
+
+    def forward_test(self, rgbs, query_points, trajectories, visibilities, save_image=False, save_path=None,
+                     iteration=None, shard=None):
+        """rgbs [1,T,3,h,w]; query_points [1,P,3] (t,x,y); trajectories [1,T,P,2]; visibilities [1,T,P].  Returns
+        VanillaTracker's 5-tuple (traj_gt, vis_gt, traj_pred, vis_pred, query_points): with ``test_cfg.with_first``
+        the points are grouped by query frame and re-ordered by group (with ``bidirectional`` each group is also
+        tracked backwards), else every point is tracked from frame 0 in input order.  ``shard=(rank, world)``: the
+        two-phase split of ``C2FPointTracker.track_banks``."""
+        _lib.require_cuda()
+        dev = torch.device("cuda", torch.cuda.current_device())
+        rgbs, query_points = rgbs.to(dev), query_points.to(dev)
+        trajectories, visibilities = trajectories.to(dev), visibilities.to(dev)
+        assert rgbs.shape[0] == 1
+        h, w = rgbs.shape[-2:]
+        fine, coarse = self.encode_to_bank(rgbs[0], n_levels=2)
+        c2f = C2FPointTracker(self.test_cfg, self.engine_id)
+        qp = query_points[0]
+        if not self.test_cfg.get("with_first", False):
+            qp = torch.cat([torch.zeros_like(qp[:, :1]), qp[:, 1:]], dim=1)
+            traj = c2f.track_banks(coarse, fine, qp, (h, w), shard=shard)
+            return trajectories, visibilities, traj.double()[None], torch.zeros_like(visibilities), query_points
+        traj = c2f.track_banks(coarse, fine, qp, (h, w), shard=shard)
+        qt = qp[:, 0]
+        perm = torch.cat([torch.nonzero(qt == t).flatten() for t in torch.unique(qt).tolist()])
+        return (trajectories[:, :, perm], visibilities[:, :, perm], traj[:, perm].to(trajectories.dtype)[None],
+                torch.zeros_like(visibilities), query_points[:, perm])
+
+    def propagate_points(self, *args, **kwargs):
+        raise NotImplementedError("C2FTracker tracks points through forward_test (C2FPointTracker.track_banks)")
+
+    def propagate_masks(self, *args, **kwargs):
+        raise NotImplementedError("C2FTracker has no mask propagation")
+
+
+B200C2FTracker = C2FTracker

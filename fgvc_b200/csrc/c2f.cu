@@ -491,9 +491,9 @@ int launch_c2f_chain_lanes(const float* cw, const int32_t* crow, int K, int job_
 }
 
 // the fine stage of fgvc_c2f_propagate runs as a window-mode K1 (+ tail) exactly when this holds (else c2f_fine_kernel)
-bool c2f_use_window(int engine, int bank_format, int Hf, int Wf, int Cf, int K, int n_mem) {
+bool c2f_use_window(int engine, int fine_format, int Hf, int Wf, int Cf, int K, int n_mem) {
   static const bool no_window = getenv("FGVC_C2F_SIMT") != nullptr;
-  return !no_window && engine != FGVC_ENGINE_SIMT && bank_format == FGVC_BANK_F16 &&
+  return !no_window && engine != FGVC_ENGINE_SIMT && fine_format == FGVC_BANK_F16 &&
          c2f_window_supported(Hf, Wf, Cf, K, n_mem);
 }
 
@@ -507,8 +507,8 @@ extern "C" int64_t fgvc_c2f_scratch_elems(int32_t n_mem, int32_t n_coarse) {
   return ((int64_t)n_mem + 1 + (int64_t)n_mem * 4 * 16) * n_coarse;
 }
 
-extern "C" int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, int32_t n_slots, int32_t Hc, int32_t Wc,
-                                  int32_t C, const void* fine_bank, int32_t Hf, int32_t Wf, int32_t Cf,
+extern "C" int fgvc_c2f_propagate(const void* coarse_bank, int32_t coarse_format, int32_t n_slots, int32_t Hc, int32_t Wc,
+                                  int32_t C, const void* fine_bank, int32_t fine_format, int32_t Hf, int32_t Wf, int32_t Cf,
                                   const fgvc_job* job_dev, const fgvc_job* job_host, const int32_t* mem_feat_slot,
                                   const int32_t* mem_label_slot, int32_t radius, int32_t mask_mode,
                                   int32_t radius_fine, int32_t K, float temperature, const float* fine_lab_bank,
@@ -526,13 +526,13 @@ extern "C" int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, 
                  "fgvc_c2f_propagate: scratch arrays need %lld elements each (fgvc_c2f_scratch_elems)",
                  (long long)fgvc_c2f_scratch_elems(n_mem, Hc * Wc));
   // coarse stage: top-1 per memory frame == groups = n_mem
-  int rc = fgvc_affinity_topk(coarse_bank, bank_format, n_slots, Hc, Wc, C, job_dev, 1, mem_feat_slot, radius, mask_mode, 1, n_mem,
+  int rc = fgvc_affinity_topk(coarse_bank, coarse_format, n_slots, Hc, Wc, C, job_dev, 1, mem_feat_slot, radius, mask_mode, 1, n_mem,
                               scratch_val, scratch_idx, engine, stream);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int scale = Hf / Hc;
   // fine stage on the tensor cores (window-mode K1 + tail) whenever the fine bank allows; else one warp per candidate
-  if (c2f_use_window(engine, bank_format, Hf, Wf, Cf, K, n_mem)) {
+  if (c2f_use_window(engine, fine_format, Hf, Wf, Cf, K, n_mem)) {
     float* floor_ws = scratch_val + (int64_t)n_mem * Hc * Wc;    // behind the coarse arg-max table: the floors,
     float* fv = floor_ws + (int64_t)Hc * Wc;                     // then the fine lists
     int32_t* fi = scratch_idx + (int64_t)(n_mem + 1) * Hc * Wc;
@@ -548,7 +548,7 @@ extern "C" int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, 
     if (rc != FGVC_ERR_UNSUPPORTED) return rc;
   }
 #define FGVC_FINE(KK)                                                                                              \
-  return bank_format == FGVC_BANK_TF32                                                                             \
+  return fine_format == FGVC_BANK_TF32                                                                             \
              ? launch_fine<KK, FGVC_BANK_TF32>(fine_bank, Hc, Wc, Hf, Wf, Cf, scale, *job_host, mem_feat_slot,      \
                                                mem_label_slot, scratch_idx, radius_fine, K, temperature,            \
                                                fine_lab_bank, Lp, out, st)                                          \
@@ -597,8 +597,9 @@ extern "C" int64_t fgvc_c2f_clip_workspace_bytes(const fgvc_job* jobs_host, int3
   return clip_layout(jobs_host, job_begin, job_end, Hc, Wc, K).total;
 }
 
-extern "C" int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t bank_format, int32_t n_slots, int32_t Hc, int32_t Wc,
-                                     int32_t C, const void* fine_bank, int32_t Hf, int32_t Wf, int32_t Cf,
+extern "C" int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t coarse_format, int32_t n_slots, int32_t Hc,
+                                     int32_t Wc, int32_t C, const void* fine_bank, int32_t fine_format, int32_t Hf, int32_t Wf,
+                                     int32_t Cf,
                                      const fgvc_job* jobs_host, int32_t job_begin, int32_t job_end,
                                      const int32_t* mem_feat_slot, const int32_t* mem_label_slot, int32_t radius,
                                      int32_t mask_mode, int32_t radius_fine, int32_t K, float temperature, float* weights,
@@ -665,7 +666,7 @@ extern "C" int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t bank_forma
     while (b < n && len(order[b]) == len(order[a])) ++b;
     const int m = len(order[a]);
     const int64_t o = wj[order[a]].best_off;
-    int rc = fgvc_affinity_topk(coarse_bank, bank_format, n_slots, Hc, Wc, C, cjobs_dev + a, b - a, mem_feat_slot, radius,
+    int rc = fgvc_affinity_topk(coarse_bank, coarse_format, n_slots, Hc, Wc, C, cjobs_dev + a, b - a, mem_feat_slot, radius,
                                 mask_mode, 1, m, best_val + o, best_idx + o, engine, stream);
     if (rc) return rc;
     a = b;
@@ -673,7 +674,7 @@ extern "C" int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t bank_forma
 
   // fine stage of every job: window-mode K1 + weights kernel on the tensor cores, else the one-warp-per-candidate
   // kernel in its weights-only form -- the choice fgvc_c2f_propagate makes for each job
-  if (c2f_use_window(engine, bank_format, Hf, Wf, Cf, K, max_mem)) {
+  if (c2f_use_window(engine, fine_format, Hf, Wf, Cf, K, max_mem)) {
     int rc = launch_c2f_window_tc16_jobs(fine_bank, n_slots, Hc, Wc, Hf, Wf, Cf, scale, wjobs_dev, n, n_y, mem_feat_slot,
                                          best_idx, radius_fine, K, floor_ws, lv, li, st);
     if (rc == FGVC_OK) {
@@ -697,7 +698,7 @@ extern "C" int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t bank_forma
       fine_bank, Hc, Wc, Hf, Wf, Cf, scale, none, mem_feat_slot, mem_label_slot, best_idx, radius_fine, K, temperature, \
       nullptr, 0, nullptr, wjobs_dev, weights, rows)
 #define FGVC_FINE_K(KK)                                               \
-  if (bank_format == FGVC_BANK_TF32) FGVC_FINE_W(KK, FGVC_BANK_TF32); \
+  if (fine_format == FGVC_BANK_TF32) FGVC_FINE_W(KK, FGVC_BANK_TF32); \
   else FGVC_FINE_W(KK, FGVC_BANK_F16)
   if (K <= 4) { FGVC_FINE_K(4); }
   else if (K <= 10) { FGVC_FINE_K(10); }

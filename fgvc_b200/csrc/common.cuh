@@ -244,7 +244,7 @@ int launch_c2f_window_tc16_jobs(const void* fine_bank, int n_slots, int Hc, int 
                                 const int32_t* best, int rf, int K, float* floor_ws, float* tv, int32_t* ti,
                                 cudaStream_t st);
 int c2f_window_chunks(int Hc, int Wc, int n_mem);
-bool c2f_use_window(int engine, int bank_format, int Hf, int Wf, int Cf, int K, int n_mem);
+bool c2f_use_window(int engine, int fine_format, int Hf, int Wf, int Cf, int K, int n_mem);
 int resident_ctas(const void* kernel, std::atomic<int>* cached, int* max_ctas);
 int launch_c2f_chain_lanes(const float* cw, const int32_t* crow, int K, int job_base, const fgvc_job* jobs_dev,
                            const fgvc_c2f_lane* lanes_dev, const fgvc_c2f_lane* lanes_host, int n_lanes, int Hc, int Wc,

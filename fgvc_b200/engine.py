@@ -708,8 +708,8 @@ def c2f_propagate(coarse, fine, table, job_index, fine_labels, radius, radius_fi
     si = torch.empty(n_scr, dtype=torch.int32, device=dev)
     mode = _lib.MASK_CIRCLE if mask_mode == "circle" else _lib.MASK_SQUARE
     jptr = ctypes.c_void_p(jobs.data_ptr() + 16 * job_index)
-    assert coarse.fmt == fine.fmt
-    call("fgvc_c2f_propagate", ptr(coarse.buf), coarse.fmt, coarse.n_slots, coarse.H, coarse.W, coarse.C, ptr(fine.buf), fine.H, fine.W, fine.C,
+    call("fgvc_c2f_propagate", ptr(coarse.buf), coarse.fmt, coarse.n_slots, coarse.H, coarse.W, coarse.C, ptr(fine.buf),
+         fine.fmt, fine.H, fine.W, fine.C,
          jptr, ctypes.byref(hj), ptr(mem_feat), ptr(mem_label), int(radius), mode, int(radius_fine), int(K),
          float(temperature), ptr(fine_labels.buf), fine_labels.Lp, ptr(out), ptr(sv), ptr(si), n_scr, int(engine),
          stream_ptr())

@@ -87,12 +87,16 @@ class VanillaTracker(nn.Module):
         return torch.cat(outs, dim=0)
 
     @torch.no_grad()
-    def encode_to_bank(self, frames):
+    def encode_to_bank(self, frames, n_levels=1):
         """frames [T,3,h,w] -> FeatureBank of the clip, encoder and K0 overlapped: the (PyTorch) encoder runs on the
         current stream in chunks of ``batch_step`` frames (vanilla_tracker.py:133-153), and K0 (normalise + split +
         pixel-major) of chunk i runs on a side stream while the encoder works on chunk i + 1.  Features go straight
         into the bank: the [T,C,Hf,Wf] fp32 tensor of the whole clip (the reference moves it to the host and back)
-        is never assembled.  ``test_cfg.encoder_channels_last`` runs the encoder in channels-last memory format."""
+        is never assembled.  ``test_cfg.encoder_channels_last`` runs the encoder in channels-last memory format.
+
+        ``n_levels > 1``: the encoder returns that many output levels (a tuple, in ``out_indices`` order), each goes
+        into a bank of its own (with its own ``engine.default_split`` unless ``test_cfg.split`` forces one), and the
+        list of banks is returned."""
         cfg = self.test_cfg
         step = cfg.get("batch_step", 5)
         T = frames.shape[0]
@@ -101,25 +105,27 @@ class VanillaTracker(nn.Module):
             self._k0_stream = torch.cuda.Stream(device=frames.device)
         side = self._k0_stream
         side.wait_stream(cur)
-        bank = None
+        banks = None
         for s0 in range(0, T, step):
             x = frames[s0:s0 + step]
             if cfg.get("encoder_channels_last", False):
                 x = x.contiguous(memory_format=torch.channels_last)
             f = self.extract_feat(x)
-            if isinstance(f, (tuple, list)):
-                f = f[0]
-            f = f.float().contiguous()
-            if bank is None:
-                bank = FeatureBank(T, f.shape[1], f.shape[2], f.shape[3], frames.device, split=cfg.get("split"))
+            fs = list(f) if isinstance(f, (tuple, list)) else [f]
+            fs = [t.float().contiguous() for t in fs[:n_levels]]
+            if banks is None:
+                banks = [FeatureBank(T, t.shape[1], t.shape[2], t.shape[3], frames.device, split=cfg.get("split"))
+                         for t in fs]
             ready = torch.cuda.Event()
             ready.record(cur)
             with torch.cuda.stream(side):
                 side.wait_event(ready)
-                bank.load_frames(f, s0, normalize=cfg.get("with_norm", cfg.get("withnorm", True)))
-            f.record_stream(side)
+                for bank, t in zip(banks, fs):
+                    bank.load_frames(t, s0, normalize=cfg.get("with_norm", cfg.get("withnorm", True)))
+            for t in fs:
+                t.record_stream(side)
         cur.wait_stream(side)
-        return bank
+        return banks[0] if n_levels == 1 else banks
 
     def _stream_in(self, feats_host, bank, table, t0, radius, mask_mode, normalize, n_chunks=6):
         """Host features of ONE clip -> feature bank and top-k lists, pipelined: the frames are copied in chunks on a
@@ -459,8 +465,11 @@ B200HRVanillaTracker = HRVanillaTracker
 
 
 def register_in_mmpt():
-    """Inside an mmpt installation: make ``eval_arc='B200VanillaTracker'`` resolvable."""
+    """Inside an mmpt installation: make ``eval_arc='B200VanillaTracker'`` (and the HR and coarse-to-fine trackers)
+    resolvable."""
     from mmpt.models.registry import MODELS
+    from .c2f_tracker import C2FTracker
     MODELS.register_module(name="B200VanillaTracker", module=VanillaTracker)
     MODELS.register_module(name="B200HRVanillaTracker", module=HRVanillaTracker)
+    MODELS.register_module(name="B200C2FTracker", module=C2FTracker)
     return MODELS

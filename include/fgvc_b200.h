@@ -328,13 +328,15 @@ FGVC_API int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* to
  * T*R^2, softmax, gather of FINE labels.  Output on the coarse grid: out[Hc*Wc][Lp].
  * job_dev / job_host: the same job in device memory (read by K1) and host memory (read by
  * the launcher); scratch_val / scratch_idx: fgvc_c2f_scratch_elems(n_mem, Hc*Wc) elements each (the coarse per-frame
- * arg-max table, one floor per coarse query, then the fine top-K lists).  With an F16 fine bank (Cf % 64 == 0,
- * Cf <= 256, n_mem <= 64) the fine stage runs on the tensor cores as a window-mode K1 (csrc/topk_tc16.cu) whose lists
- * start from the K-th best of the exactly scored window centres (+ 4 neighbours) of all memory frames; otherwise one
- * warp per candidate. */
+ * arg-max table, one floor per coarse query, then the fine top-K lists).  Each bank has its own format
+ * (fgvc_bank_format): the coarse K1 reads coarse_bank as coarse_format, everything of the fine stage reads fine_bank as
+ * fine_format -- e.g. a TF32 coarse bank at C = 512 (the 3xTF32 engine) and an F16 fine bank at Cf = 256.  With an F16
+ * fine bank (Cf % 64 == 0, Cf <= 256, n_mem <= 64) the fine stage runs on the tensor cores as a window-mode K1
+ * (csrc/topk_tc16.cu) whose lists start from the K-th best of the exactly scored window centres (+ 4 neighbours) of all
+ * memory frames; otherwise one warp per candidate. */
 FGVC_API int64_t fgvc_c2f_scratch_elems(int32_t n_mem, int32_t n_coarse);
-FGVC_API int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, int32_t n_slots, int32_t Hc, int32_t Wc,
-                       int32_t C, const void* fine_bank, int32_t Hf, int32_t Wf, int32_t Cf,
+FGVC_API int fgvc_c2f_propagate(const void* coarse_bank, int32_t coarse_format, int32_t n_slots, int32_t Hc, int32_t Wc,
+                       int32_t C, const void* fine_bank, int32_t fine_format, int32_t Hf, int32_t Wf, int32_t Cf,
                        const fgvc_job* job_dev, const fgvc_job* job_host,
                        const int32_t* mem_feat_slot, const int32_t* mem_label_slot, int32_t radius,
                        int32_t mask_mode, int32_t radius_fine, int32_t K, float temperature,
@@ -346,7 +348,8 @@ FGVC_API int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, in
  * features only; only the gather of fine label rows and the up-sampling of its result are recurrent.
  *
  * fgvc_c2f_clip_weights: for the jobs [job_begin, job_end) of jobs_host, the label-independent half of
- * fgvc_c2f_propagate, bit for bit what that call computes for each job: (weight, fine label row) pairs
+ * fgvc_c2f_propagate, bit for bit what that call computes for each job with the same two bank formats: (weight, fine
+ * label row) pairs
  * weights[job - job_begin][Hc*Wc][K], rows[...] (row = mem_label_slot * Hf*Wf + fine pixel, -1 = zero-padded or empty
  * candidate, weight 0 = unused).  Enqueued as one coarse K1 per distinct memory length (K = 1, groups = length, over a
  * length-sorted copy of the jobs), then for all jobs at once either the floor kernel + one window-mode K1 + one weights
@@ -356,8 +359,8 @@ FGVC_API int fgvc_c2f_propagate(const void* coarse_bank, int32_t bank_format, in
  * call only; the job tables it needs on the device are copied into ws. */
 FGVC_API int64_t fgvc_c2f_clip_workspace_bytes(const fgvc_job* jobs_host, int32_t job_begin, int32_t job_end,
                        int32_t Hc, int32_t Wc, int32_t K);
-FGVC_API int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t bank_format, int32_t n_slots, int32_t Hc, int32_t Wc,
-                       int32_t C, const void* fine_bank, int32_t Hf, int32_t Wf, int32_t Cf,
+FGVC_API int fgvc_c2f_clip_weights(const void* coarse_bank, int32_t coarse_format, int32_t n_slots, int32_t Hc, int32_t Wc,
+                       int32_t C, const void* fine_bank, int32_t fine_format, int32_t Hf, int32_t Wf, int32_t Cf,
                        const fgvc_job* jobs_host, int32_t job_begin, int32_t job_end,
                        const int32_t* mem_feat_slot, const int32_t* mem_label_slot, int32_t radius,
                        int32_t mask_mode, int32_t radius_fine, int32_t K, float temperature, float* weights,

@@ -53,6 +53,23 @@ def main():
         want3 = trk(test_mode=True, rgbs=rgbs, query_points=qp, trajectories=traj, visibilities=vis)
     err = max(err, (got3[2].double() - want3[2].double()).abs().max().item())
     trk.test_cfg = type(trk.test_cfg)(cfg)
+    # the coarse-to-fine model (B200C2FTracker): TAP-Vid strided query groups tracked both ways, the same split over
+    # the clip weights and the lanes chain
+    torch.manual_seed(0)
+    c2f = fgvc_b200.B200C2FTracker(backbone=dict(type="ResNet", depth=18, strides=(1, 1, 1, 4), out_indices=(2, 3),
+                                                 pool_type="none"),
+                                   test_cfg=dict(cfg, radius_fine=5, neighbor_range=6, bidirectional=True)).cuda().eval()
+    T4, P4 = 12, 5
+    qp4 = torch.cat([torch.arange(0, T4, 4).float().repeat_interleave(P4)[:, None],
+                     S.query_points(3 * P4, T4, h, w, seed=8)[:, 1:]], dim=1)[None]
+    rgbs4 = S.synthetic_video(T4, h, w, seed=9)[None]
+    z4 = (torch.zeros(1, T4, 3 * P4, 2), torch.zeros(1, T4, 3 * P4))
+    with torch.no_grad():
+        got4 = apis.sharded_forward_test(c2f, rgbs4, qp4, *z4)
+        want4 = c2f(test_mode=True, rgbs=rgbs4, query_points=qp4, trajectories=z4[0], visibilities=z4[1])
+    err_c2f = (got4[2].double() - want4[2].double()).abs().max().item()
+    err = max(err, err_c2f)
+    same_order = same_order and torch.equal(got4[4].cpu(), want4[4].cpu())
     # video-sharded driver + typed NCCL gather
     ds = [dict(rgbs=S.synthetic_video(4, 32, 48, seed=10 + i)[None], query_points=S.query_points(3, 4, 32, 48, seed=i)[None],
                trajectories=torch.zeros(1, 4, 3, 2), visibilities=torch.zeros(1, 4, 3)) for i in range(2 * world + 1)]
@@ -62,7 +79,8 @@ def main():
         ok = len(res) == len(ds) and all(r[2].shape == (1, 4, 3, 2) for r in res)
         ref = [trk(test_mode=True, **d)[2].cpu() for d in ds]
         ok = ok and all(torch.allclose(r[2].cpu().double(), g.double(), atol=1e-4) for r, g in zip(res, ref))
-        print(f"dist_check world={world}: sharded max err {err:.2e} order_ok={same_order} collect_ok={ok}")
+        print(f"dist_check world={world}: sharded max err {err:.2e} (B200C2FTracker {err_c2f:.2e}) "
+              f"order_ok={same_order} collect_ok={ok}")
         assert err < 1e-4 and same_order and ok
     dist.destroy_process_group()
 
