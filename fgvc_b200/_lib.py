@@ -42,6 +42,11 @@ class Lane(ctypes.Structure):
                 ("lab_offset", c_int64), ("coord_offset", c_int64)]
 
 
+class Cycle(ctypes.Structure):
+    """fgvc_cycle: frames and map offset of one lane of fgvc_point_cycle_lanes"""
+    _fields_ = [("t", c_int32), ("s", c_int32), ("map_offset", c_int64)]
+
+
 class C2FLane(ctypes.Structure):
     """fgvc_c2f_lane: one recurrence of fgvc_c2f_point_clip_tail_lanes (offsets in floats)"""
     _fields_ = [("job_begin", c_int32), ("job_end", c_int32), ("L", c_int32), ("Lp", c_int32),
@@ -82,6 +87,8 @@ SIGNATURES = {
     "fgvc_mask_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, P, P, P, P, L64, P]),
     "fgvc_point_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, I, P, P, P, L64, P]),
     "fgvc_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, P, I, P, I, I, F, I, P, I, I, I, P, P, P, L64, P]),
+    "fgvc_point_cycle_lanes": (I, [P, P, I, I, P, P, P, P, P, P, P, I, P, I, I, I, F, F, I, P, I, I, I, F, P, P, P, P, P,
+                                   P, L64, P]),
     "fgvc_c2f_scratch_elems": (L64, [I, I]),
     "fgvc_c2f_propagate": (I, [P, I, I, I, I, I, P, I, I, I, I, P, P, P, P, I, I, I, I, F, P, I, P, P, P, L64, I, P]),
     "fgvc_c2f_clip_workspace_bytes": (L64, [P, I, I, I, I, I]),

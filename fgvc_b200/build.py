@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libfgvc_b200.so")
 STAMP = os.path.join(HERE, ".libfgvc_b200.stamp")
-SOURCES = ["capi.cu", "prep.cu", "topk_simt.cu", "topk_tc.cu", "topk_tc16.cu", "gather.cu", "dense.cu", "coords.cu", "c2f.cu", "clip.cu"]
+SOURCES = ["capi.cu", "prep.cu", "topk_simt.cu", "topk_tc.cu", "topk_tc16.cu", "gather.cu", "dense.cu", "coords.cu", "c2f.cu", "clip.cu", "cycle.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--use_fast_math=false"]
 

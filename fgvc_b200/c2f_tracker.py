@@ -38,6 +38,8 @@ class C2FPointTracker:
     with_first_neighbor, with_norm, split, mask_mode; bidirectional (track_queries only)."""
 
     def __init__(self, cfg, engine_id=_lib.ENGINE_AUTO):
+        if cfg.get("cycle_occlusion") is not None:
+            raise NotImplementedError("C2FPointTracker: cycle_occlusion is not built")
         self.cfg = cfg
         self.engine_id = engine_id
 
@@ -327,6 +329,9 @@ class C2FTracker(VanillaTracker):
         for key in ("hard_prop", "stride_sample"):
             if cfg.get(key, False):
                 raise NotImplementedError(f"C2FTracker: test_cfg.{key} is not built")
+        if cfg.get("cycle_occlusion") is not None:
+            raise NotImplementedError("C2FTracker: test_cfg.cycle_occlusion is not built (the coarse-to-fine recurrence "
+                                      "is another operator; VanillaTracker and HRVanillaTracker have it)")
         for key in ("topk", "neighbor_range"):
             if cfg.get(key) is None:
                 raise NotImplementedError(f"C2FTracker needs test_cfg.{key} (the c2f path has no {key}=None form)")

@@ -198,6 +198,23 @@ class JobTable:
         """sizes of the union memory lists of the tile groups of jobs [j0, j1) (cost model)."""
         return [len(self._group_table(m, J, a if aligned else None)) for a, m in self._tile_groups(j0, j1, J, aligned)]
 
+    def packed_cuts(self, cuts, J, device, aligned=False):
+        """``packed`` of the consecutive job ranges ``cuts`` [(j0, j1), ...] concatenated: no tile group spans two
+        ranges, so the tile groups of each range are the ones ``packed`` gives for it alone."""
+        parts = [self.packed(a, b, J, device, aligned) for a, b in cuts if b > a]
+        if len(parts) == 1:
+            return parts[0]
+        groups, uents, upos, u = [], [], [], 0
+        for g, ue, up in parts:
+            g = g.clone()
+            g[:, 5:7] += u
+            n = int(g[:, 6].max()) - u if g.shape[0] else 0
+            groups.append(g)
+            uents.append(ue[:n])
+            upos.append(up[:n])
+            u += n
+        return torch.cat(groups), torch.cat(uents), torch.cat(upos)
+
     def packed(self, j0, j1, J, device, aligned=False):
         """Tile groups of jobs [j0, j1) for fgvc_affinity_topk_packed: (groups [n,8] int32, union entries [U] int32,
         union positions [U,4] int32) on ``device``.  A memory list is a multiset (frame 0 twice while
@@ -408,7 +425,7 @@ def pair_key(table, job):
     return q_slot, (table.mem_feat[b] & ~_lib.MEM_UNMASKED) > q_slot
 
 
-def shared_pair_table(table, spans, T):
+def shared_pair_table(table, spans, T, decide_jobs=None, max_entries=None):
     """Several ``with_first`` groups of one clip: the jobs (group g, query frame t) of different groups see the same
     memory frames except their first one, so the label-independent K1 work is shared -- run it once per query frame
     and direction over the UNION of the groups' memory entries, one list per (query frame, direction, memory entry),
@@ -417,21 +434,33 @@ def shared_pair_table(table, spans, T):
     pair_ref) or None when sharing would not pay:
       utable   : JobTable with one job per (query frame, direction), entries = sorted unique (frame, mask flag) of all
                  groups;
-      pair_ref : for every memory entry of ``table`` the index (u_job * Gmax + position in the union) of its list."""
+      pair_ref : for every memory entry of ``table`` the index (u_job * Gmax + position in the union) of its list.
+    ``decide_jobs``: whether sharing pays is judged on the first ``decide_jobs`` jobs only (the tracking jobs, when the
+    cycle checks follow them: adding the checks must not change how the tracks are computed).  ``max_entries``: a
+    (query frame, direction) with more entries is split over several utable jobs of at most that many (K1 takes at
+    most 64 lists per job); default: no split, None when a union has more than 64 entries."""
     by_key = {}
     for job in table.jobs:
         by_key.setdefault(pair_key(table, job), set()).update(table.mem_feat[job[1]:job[2]])
-    if len(table) < 1.8 * len(by_key):
+    dec = by_key
+    if decide_jobs is not None:
+        dec = {}
+        for job in table.jobs[:decide_jobs]:
+            dec.setdefault(pair_key(table, job), set()).update(table.mem_feat[job[1]:job[2]])
+    if not dec or len(table.jobs[:decide_jobs]) < 1.8 * len(dec) or max(len(v) for v in dec.values()) > 64:
         return None
     gmax = max(len(v) for v in by_key.values())
-    if gmax > 64:
+    if max_entries is None and gmax > 64:
         return None
+    gmax = min(gmax, max_entries or gmax)
     utable, where = JobTable(), {}
-    for u, key in enumerate(sorted(by_key)):
+    for key in sorted(by_key):
         ent = sorted(by_key[key], key=lambda r: (r & ~_lib.MEM_UNMASKED, 0 if (r & _lib.MEM_UNMASKED) else 1))
-        utable.add_raw(key[0], ent, key[0])
-        for i, r in enumerate(ent):
-            where[(key, r)] = u * gmax + i
+        for c in range(0, len(ent), gmax):
+            u = len(utable)
+            utable.add_raw(key[0], ent[c:c + gmax], key[0])
+            for i, r in enumerate(ent[c:c + gmax]):
+                where[(key, r)] = u * gmax + i
     pair_ref = []
     for job in table.jobs:
         key = pair_key(table, job)
@@ -487,6 +516,45 @@ def point_tail_lanes(lists, pair_ref, table, lanes, lab, maps, coords, H, W, out
          ptr(maps), ptr(coords), *chain_workspace(dev, je - jb, H * W, lists.K, flags, force=True), stream_ptr())
 
 
+def point_cycle_lanes(lists, pair_ref, table, lanes, coords, cycle_coords, vis, H, W, out_hw, stride, temperature,
+                      flags, threshold, sigma=6.0, coord_topk=5):
+    """fgvc_point_cycle_lanes: the cycle checks ``lanes`` [(job_begin, job_end, L, coord_offset, t, s)] in one call.
+    Their banks, the NCHW maps of their last slots, the K3 output and the chain workspace are allocated here, for this
+    call only: a caller bounds the memory by the checks it passes (VanillaTracker._cycle_tail)."""
+    dev = coords.device
+    n_pix = H * W
+    jobs_dev, _, mem_label = table.device(dev)
+    jobs_host = torch.tensor(table.jobs, dtype=torch.int32).reshape(-1, 4).contiguous()
+    hl, hc, lab_off, map_off = [], [], 0, 0
+    for jb, je, L, c_off, t, s in lanes:
+        hl.append(_lib.Lane(jb, je, L, pad4(L), lab_off, c_off))
+        hc.append(_lib.Cycle(t, s, map_off))
+        lab_off += (je - jb + 1) * n_pix * pad4(L)
+        map_off += L
+    host_l, host_c = (_lib.Lane * len(hl))(*hl), (_lib.Cycle * len(hc))(*hc)
+    lanes_dev = torch.frombuffer(bytearray(host_l), dtype=torch.uint8).to(dev)
+    cycles_dev = torch.frombuffer(bytearray(host_c), dtype=torch.uint8).to(dev)
+    lab = torch.empty(lab_off, dtype=torch.float32, device=dev)
+    maps = torch.empty(map_off * n_pix, dtype=torch.float32, device=dev)
+    xy = torch.empty(map_off * 2, dtype=torch.float32, device=dev)
+    jb, je = min(ln[0] for ln in lanes), max(ln[1] for ln in lanes)
+    ws_bytes = int(_lib.load().fgvc_chain_workspace_bytes(je - jb, n_pix, lists.K))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    call("fgvc_point_cycle_lanes", ptr(lists.val), ptr(lists.idx), lists.K, 1 if pair_ref is not None else lists.groups,
+         ptr(pair_ref) if pair_ref is not None else None, ptr(jobs_dev), ptr(jobs_host), ptr(lanes_dev),
+         ctypes.c_void_p(ctypes.addressof(host_l)), ptr(cycles_dev), ctypes.c_void_p(ctypes.addressof(host_c)),
+         len(lanes), ptr(mem_label), H, W, int(stride), float(sigma), float(temperature), int(flags), ptr(lab),
+         int(out_hw[0]), int(out_hw[1]), int(coord_topk), float(threshold), ptr(coords), ptr(maps), ptr(xy),
+         ptr(cycle_coords), ptr(vis), ptr(ws), ws_bytes, stream_ptr())
+
+
+def cycle_lane_bytes(n_jobs, L, n_pix, K):
+    """device bytes point_cycle_lanes allocates for a check of n_jobs jobs over L points: its bank of n_jobs + 1 slots,
+    its share of the chain workspace, its NCHW maps and K3 output"""
+    return 4 * (n_jobs + 1) * n_pix * pad4(L) + int(_lib.load().fgvc_chain_workspace_bytes(n_jobs, n_pix, K)) - 256 + \
+        4 * L * n_pix + 8 * L
+
+
 K1_TIMING = None       # bench.py: a list -> affinity_topk appends (start, end) CUDA events of every K1 launch
 
 
@@ -525,11 +593,13 @@ def plan_k1(bank, table, radius, K, mask_mode="circle", job_range=None, engine=_
 
 
 def affinity_topk(bank, table, radius, K, mask_mode="circle", groups=None, engine=_lib.ENGINE_AUTO, lists=None,
-                  job_range=None, pack=True, plan=None, floor=None):
+                  job_range=None, pack=True, plan=None, floor=None, cuts=None):
     """K1 over every job of ``table`` (or the jobs ``job_range=(begin, end)``) in one launch.  ``AUTO``
     = the tensor engine of the bank format when the shape allows, else the CUDA-core engine.  ``plan`` (plan_k1)
     fixes the tiling; the lists hold ``plan.lists_per_job`` partial lists per job, merged by the gather.
-    ``floor`` [jobs, Nq] (topk_floor): starting value of the lists, un-packed launches only (see the header)."""
+    ``floor`` [jobs, Nq] (topk_floor): starting value of the lists, un-packed launches only (see the header).
+    ``cuts``: consecutive sub-ranges of the launch whose jobs are packed into query tiles only with each other
+    (JobTable.packed_cuts): a range then gets the lists it gets in a launch of its own with the same plan."""
     dev = bank.buf.device
     jobs, mem_feat, _ = table.device(dev)
     j0, j1 = job_range if job_range is not None else (0, len(table))
@@ -548,12 +618,12 @@ def affinity_topk(bank, table, radius, K, mask_mode="circle", groups=None, engin
         ev[0].record()
         try:
             return _affinity_topk_launch(bank, table, radius, K, mode, groups, engine, lists, j0, j1, plan, per_job,
-                                         jobs, mem_feat, dev, floor)
+                                         jobs, mem_feat, dev, floor, cuts)
         finally:
             ev[1].record()
             K1_TIMING.append(ev)
     return _affinity_topk_launch(bank, table, radius, K, mode, groups, engine, lists, j0, j1, plan, per_job, jobs,
-                                 mem_feat, dev, floor)
+                                 mem_feat, dev, floor, cuts)
 
 
 def topk_floor(bank, table, seed_slots, radius, K, mask_mode="circle"):
@@ -573,10 +643,11 @@ def topk_floor(bank, table, seed_slots, radius, K, mask_mode="circle"):
 
 
 def _affinity_topk_launch(bank, table, radius, K, mode, groups, engine, lists, j0, j1, plan, per_job, jobs, mem_feat, dev,
-                          floor=None):
+                          floor=None, cuts=None):
     # fp16 tensor engine: J consecutive jobs per query tile when that saves tensor work (csrc/topk_tc16.cu)
     if (plan.J > 1 or plan.aligned) and tensor16_ok(bank, K, engine):
-        tg, uent, upos = table.packed(j0, j1, plan.J, dev, plan.aligned)
+        tg, uent, upos = table.packed(j0, j1, plan.J, dev, plan.aligned) if cuts is None else \
+            table.packed_cuts([(max(a, j0), min(b, j1)) for a, b in cuts], plan.J, dev, plan.aligned)
         try:
             call("fgvc_affinity_topk_packed", ptr(bank.buf), bank.n_slots, bank.H, bank.W, bank.C, ptr(jobs), ptr(tg),
                  int(tg.shape[0]), ptr(uent), ptr(upos), int(plan.J), int(radius), mode, int(K), int(groups),
@@ -686,13 +757,53 @@ def query_job_table(t0s, T, precede_frames, with_first, bidirectional, unmasked)
     for t0 in t0s:
         spans.append((len(table), t0))
         for t in range(t0 + 1, T):
-            mem = memory_frames(t, precede_frames, with_first, first=t0)
+            mem = track_memory(t, t0, T, precede_frames, with_first)
             table.add(t, mem, mem, t, unmasked=unmasked(mem))
         if bidirectional:
             for t in range(t0 - 1, -1, -1):
-                mem = [T - 1 - r for r in memory_frames(T - 1 - t, precede_frames, with_first, first=T - 1 - t0)]
+                mem = track_memory(t, t0, T, precede_frames, with_first)
                 table.add(t, mem, mem, t, unmasked=unmasked(mem))
     return table, spans
+
+
+def track_memory(t, t0, T, precede_frames, with_first):
+    """Memory frames of query frame t != t0 of a track that starts at t0 (query_job_table): forward (t > t0) the
+    reference's memory_frames with first = t0, backward (t < t0) the same on the time-reversed clip."""
+    if t > t0:
+        return memory_frames(t, precede_frames, with_first, first=t0)
+    return [T - 1 - r for r in memory_frames(T - 1 - t, precede_frames, with_first, first=T - 1 - t0)]
+
+
+def cycle_end(t, t0, frames):
+    """Frame where the cycle check of a prediction at t != t0 (test_cfg.cycle_occlusion) stops: ``frames`` steps from
+    t toward the query frame t0, not past it; ``frames=None``: t0."""
+    if frames is None:
+        return t0
+    return max(t0, t - frames) if t > t0 else min(t0, t + frames)
+
+
+def cycle_job_table(table, spans, T, precede_frames, with_first, bidirectional, frames, unmasked):
+    """Append the jobs of the cycle checks of every group of ``spans`` (query_job_table's (first job, t0) pairs) to
+    ``table``.  The check of (group, t) re-tracks the prediction at t toward t0 with the tracker that starts at t --
+    the backward one for t > t0, the forward one for t < t0 -- over the query frames between t and s = cycle_end(t, t0,
+    frames): the jobs query_job_table([t], ..., bidirectional=True) has for those frames, in recurrence order.  Their
+    label slots are local to the check's own bank: slot 0 = frame t, slot k = the frame of the k-th job (out_slot k).
+    Returns the checks as (group index, t, s, first job, end job), longest first (consecutive checks then have similar
+    lengths, which keeps the grid barriers of a chunk of them few)."""
+    checks = []
+    for g, (_, t0) in enumerate(spans):
+        ts = list(range(t0 + 1, T)) + (list(range(t0 - 1, -1, -1)) if bidirectional else [])
+        checks.extend((g, t, cycle_end(t, t0, frames)) for t in ts)
+    checks.sort(key=lambda c: -abs(c[1] - c[2]))
+    out = []
+    for g, t, s in checks:
+        step = -1 if s < t else 1
+        jb = len(table)
+        for q in range(t + step, s + step, step):
+            mem = track_memory(q, t, T, precede_frames, with_first)
+            table.add(q, mem, [abs(m - t) for m in mem], abs(q - t), unmasked=unmasked(mem))
+        out.append((g, t, s, jb, len(table)))
+    return out
 
 
 def c2f_propagate(coarse, fine, table, job_index, fine_labels, radius, radius_fine, K, temperature,

@@ -51,6 +51,7 @@ class VanillaTracker(nn.Module):
             else _Cfg(test_cfg or {})
         self.stride_sample = self.test_cfg.get("stride_sample", False)
         self.engine_id = self.test_cfg.get("engine", _lib.ENGINE_AUTO)
+        self.cycle_cfg()                              # a malformed cycle_occlusion fails here, not after the encoder
         self.register_buffer("iteration", torch.tensor(0, dtype=torch.float))
 
     def init_weights(self):
@@ -174,13 +175,21 @@ class VanillaTracker(nn.Module):
     local_window = False           # HRVanillaTracker: square window + zero-padded candidates
 
     @torch.no_grad()
-    def propagate_points(self, feats, groups, image_hw, shard=None):
+    def propagate_points(self, feats, groups, image_hw, shard=None, return_cycle=False):
         """feats [T,C,Hf,Wf] (CUDA); groups: list of (t0, points_xy [P',2]).
         Returns list of [T,P',2] float64 CUDA tensors (zeros before t0).
         ``shard=(rank, world)``: two-phase split of ONE video over the default process group (SURVEY 8e): K1 runs for
         this rank's frame range only and the top-k lists are all-gathered; the recurrent tail runs for this rank's
-        slice of every group's points and the tracks are all-gathered.  Every rank returns the full result."""
+        slice of every group's points and the tracks are all-gathered.  Every rank returns the full result.
+
+        ``test_cfg.cycle_occlusion = dict(frames=H, threshold=delta)``: forward-backward cycle check of every
+        prediction (INTEGRATION.md section 2).  Returns (tracks, visibility) then: visibility = per group a [T,P'] bool
+        tensor, True at the query frame and where the prediction at t, re-tracked from t toward t0 for H frames
+        (None: back to t0) and stopping at s, lands within delta image pixels of the track at s; False where there
+        is no prediction (t < t0 without ``bidirectional``).  ``return_cycle=True`` adds per group the [T,P',2]
+        float64 re-tracked positions (row t holds the one at s, zeros where there is no check)."""
         cfg = self.test_cfg
+        cyc = self.cycle_cfg()
         host_feats = False
         if isinstance(feats, FeatureBank):               # encode_to_bank: K0 already ran, overlapped with the encoder
             pre_bank = feats
@@ -225,17 +234,28 @@ class VanillaTracker(nn.Module):
 
         bidirectional = bool(cfg.get("bidirectional", False))
         # per group: (first job, t0); forward jobs t0+1 .. T-1, then (bidirectional) backward jobs t0-1 .. 0
+        unmasked = lambda mem: len(mem) if nr is None else unmasked_first       # noqa: E731
         table, spans = engine.query_job_table([t0 for t0, _ in groups], T, precede, with_first_mem, bidirectional,
-                                              lambda mem: len(mem) if nr is None else unmasked_first)
+                                              unmasked)
+        n_track = len(table)
+        # cycle checks: their jobs follow the tracking jobs in the same table, so one K1 launch covers both and a list
+        # the tracks need already is not scored twice
+        checks = None
+        if cyc is not None and n_track:
+            checks = engine.cycle_job_table(table, spans, T, precede, with_first_mem, bidirectional, cyc["frames"],
+                                            unmasked)
         radius = (nr // 2) if nr is not None else 1
         rank, world = shard if shard is not None else (0, 1)
         # several groups: the label-independent K1 work is shared between the groups (one list per (query frame,
-        # memory frame) pair); FGVC_NO_SHARE=1 keeps one K1 job per (group, frame)
+        # memory frame) pair); FGVC_NO_SHARE=1 keeps one K1 job per (group, frame).  Whether it is shared is decided
+        # on the tracking jobs alone, so that the cycle checks leave the tracks bit for bit as they are
         shared = None
-        if len(groups) > 1 and len(table) > 0 and os.environ.get("FGVC_NO_SHARE") != "1":
-            shared = engine.shared_pair_table(table, spans, T)
+        if len(groups) > 1 and n_track > 0 and os.environ.get("FGVC_NO_SHARE") != "1":
+            shared = engine.shared_pair_table(table, spans, T, decide_jobs=n_track,
+                                              max_entries=64 if checks is not None else None)
         # (the streamed path needs every job to read only earlier frames: forward jobs only)
-        streamed = host_feats and len(groups) == 1 and world == 1 and len(table) > 0 and not bidirectional
+        streamed = host_feats and len(groups) == 1 and world == 1 and len(table) > 0 and not bidirectional and \
+            checks is None
         if host_feats and not streamed and world == 1:
             bank.load_frames(feats.to(dev, non_blocking=True), 0, normalize=normalize)
         if streamed:
@@ -246,7 +266,8 @@ class VanillaTracker(nn.Module):
             from . import apis
             ktable = shared[0] if shared is not None else table
             plan = engine.plan_k1(bank, ktable, radius, cfg.topk, mask_mode, engine=self.engine_id,
-                                  groups=shared[1] if shared is not None else None, pack=shared is None)
+                                  groups=shared[1] if shared is not None else None, pack=shared is None,
+                                  job_range=(0, n_track) if (shared is None and checks is not None) else None)
             lo, hi, per = apis.frame_shard(len(ktable), rank, world)
             lists = engine.TopKLists(per * world, plan.lists_per_job, Hf * Wf, cfg.topk, dev)
             if pre_bank is None:
@@ -257,7 +278,8 @@ class VanillaTracker(nn.Module):
                     bank.load_frames(feats[a:b_].to(dev, non_blocking=True), a, normalize=normalize)
             if hi > lo:
                 engine.affinity_topk(bank, ktable, radius, cfg.topk, mask_mode, engine=self.engine_id, lists=lists,
-                                     job_range=(lo, hi), plan=plan)
+                                     job_range=(lo, hi), plan=plan,
+                                     cuts=[(0, n_track), (n_track, len(ktable))] if shared is None else None)
             apis.gather_job_lists(lists.val, per, rank, world)
             apis.gather_job_lists(lists.idx, per, rank, world)
         else:
@@ -282,33 +304,109 @@ class VanillaTracker(nn.Module):
                     floor = engine.topk_floor(bank, utable, seeds, radius, cfg.topk, mask_mode)
                 lists = engine.affinity_topk(bank, utable, radius, cfg.topk, mask_mode, groups=gmax,
                                              engine=self.engine_id, pack=False, floor=floor)
+            elif checks is not None:
+                # the tiling of the tracking jobs alone (jobs per tile, lists per job), and no query tile mixes them
+                # with the checks' jobs: the tracks get the lists they get without the checks
+                plan = engine.plan_k1(bank, table, radius, cfg.topk, mask_mode, job_range=(0, n_track),
+                                      engine=self.engine_id)
+                lists = engine.affinity_topk(bank, table, radius, cfg.topk, mask_mode, engine=self.engine_id, plan=plan,
+                                             cuts=[(0, n_track), (n_track, len(table))])
             else:
                 lists = engine.affinity_topk(bank, table, radius, cfg.topk, mask_mode, engine=self.engine_id)
         pair_ref = torch.tensor(shared[2], dtype=torch.int32, device=dev) if shared is not None else None
         # coordinates of the query frames (soft-argmax of the analytic gaussian, :321-343): one launch for all groups
         all_pts = torch.cat([pts.to(device=dev, dtype=torch.float32) for _, pts in groups], dim=0) if groups else None
         all_c0 = engine.gaussian_coords(all_pts, (h, w)) if groups and all_pts.shape[0] else None
-        outs = self._point_tail(lists, pair_ref, table, spans, groups, all_pts, all_c0, rank, world, T, Hf, Wf, (h, w),
-                                stride, temperature, flags, bidirectional, dev)
+        outs, coords, parts = self._point_tail(lists, pair_ref, table, spans, groups, all_pts, all_c0, rank, world, T,
+                                               Hf, Wf, (h, w), stride, temperature, flags, bidirectional, dev)
+        if cyc is not None:
+            # per group [T, P_rank, 2] positions and flags of the checks, cycle position in channels 2-3, flag in 4
+            cyc_xy, vis = self._cycle_tail(lists, pair_ref, table, checks, parts, coords, T, Hf, Wf, (h, w), stride,
+                                           temperature, flags, cyc["threshold"], dev)
+            outs = [torch.cat([o.double(), c.double(), v[..., None].double()], dim=-1) for o, c, v in zip(outs, cyc_xy, vis)]
+        else:
+            outs = [o.double() for o in outs]
         if world > 1:
             from . import apis
             sizes = [int(pts.shape[0]) for _, pts in groups]
             pads = [-(-n // world) for n in sizes]
-            local = torch.zeros(T, sum(pads), 2, dtype=torch.float64, device=dev)
+            local = torch.zeros(T, sum(pads), outs[0].shape[-1] if outs else 2, dtype=torch.float64, device=dev)
             off = 0
             for o, pad in zip(outs, pads):
                 local[:, off:off + o.shape[1]] = o
                 off += pad
             outs = apis.gather_point_tracks(local, sizes, rank, world)
-        return outs
+        if cyc is None:
+            return outs
+        tracks, vis = [o[..., :2].contiguous() for o in outs], [o[..., 4] != 0 for o in outs]
+        if return_cycle:
+            return tracks, vis, [o[..., 2:4].contiguous() for o in outs]
+        return tracks, vis
+
+    def cycle_cfg(self):
+        """``test_cfg.cycle_occlusion`` checked: dict(frames=positive int or None, threshold=float >= 0,
+        max_bytes=device bytes the checks of one chain call may use, default half of what is free), or None."""
+        c = self.test_cfg.get("cycle_occlusion")
+        if c is None:
+            return None
+        unknown = set(c) - {"frames", "threshold", "max_bytes"}
+        if unknown or "threshold" not in c:
+            raise TypeError(f"test_cfg.cycle_occlusion takes frames, threshold (required) and max_bytes, got {dict(c)}")
+        frames = c.get("frames")
+        if frames is not None and (isinstance(frames, bool) or int(frames) != frames or frames < 1):
+            raise ValueError(f"cycle_occlusion.frames must be a positive int or None, got {frames!r}")
+        if not float(c["threshold"]) >= 0:
+            raise ValueError(f"cycle_occlusion.threshold must be >= 0, got {c['threshold']!r}")
+        return dict(frames=None if frames is None else int(frames), threshold=float(c["threshold"]),
+                    max_bytes=c.get("max_bytes"))
+
+    def _cycle_tail(self, lists, pair_ref, table, checks, parts, coords, T, Hf, Wf, image_hw, stride, temperature, flags,
+                    threshold, dev):
+        """Cycle checks of this rank's points after the tracking tail (they start from its tracks): per check one lane
+        of a multi-lane gather chain over its own bank (engine.point_cycle_lanes), in chunks of checks whose buffers
+        fit ``max_bytes`` -- one chain call per chunk.  Returns per group the [T, P_rank, 2] float32 cycle positions and
+        the [T, P_rank] uint8 flags (1 at the query frame)."""
+        cyc_coords = torch.zeros_like(coords)
+        vis = torch.zeros(coords.numel() // 2, dtype=torch.uint8, device=dev)
+        c_offs, off = [], 0
+        for _, t0, _, P in parts:
+            c_offs.append(off)
+            vis[off // 2 + t0 * P:off // 2 + (t0 + 1) * P] = 1            # visible at the query frame
+            off += T * P * 2
+        lanes = [(jb, je, parts[g][3], c_offs[g], t, s) for g, t, s, jb, je in (checks or []) if parts[g][3]]
+        budget = self.cycle_cfg()["max_bytes"]
+        if budget is None:
+            free, _ = torch.cuda.mem_get_info(dev)
+            budget = (free + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)) // 2
+        n_pix = Hf * Wf
+        i = 0
+        while i < len(lanes):
+            # a chunk: consecutive checks (consecutive jobs) while they fit the budget (at least one)
+            j, used = i, 0
+            while j < len(lanes):
+                jb, je, L = lanes[j][:3]
+                need = engine.cycle_lane_bytes(je - jb, L, n_pix, lists.K)
+                if j > i and (used + need > budget or je - lanes[i][0] > 65535):
+                    break
+                used += need
+                j += 1
+            engine.point_cycle_lanes(lists, pair_ref, table, lanes[i:j], coords, cyc_coords, vis, Hf, Wf,
+                                     image_hw, stride, temperature, flags, threshold)
+            i = j
+        cyc_out, vis_out = [], []
+        for (_, t0, _, P), c in zip(parts, c_offs):
+            cyc_out.append(cyc_coords[c:c + T * P * 2].view(T, P, 2))
+            vis_out.append(vis[c // 2:c // 2 + T * P].view(T, P))
+        return cyc_out, vis_out
 
     def _point_tail(self, lists, pair_ref, table, spans, groups, all_pts, all_c0, rank, world, T, Hf, Wf, image_hw, stride,
                     temperature, flags, bidirectional, dev):
         """Recurrent tail: every group of this rank's points is tracked forward from its query frame and, with
         ``test_cfg.bidirectional``, backward to frame 0 -- a lane per direction over the group's label bank (both read
         slot t0 and write disjoint slots).  All banks and tracks are carved out of one allocation each, and every lane
-        of the clip runs in ONE gather chain (engine.point_tail_lanes).  Returns per group the [T, P_rank, 2] float64
-        tracks; rows that no lane writes stay zero."""
+        of the clip runs in ONE gather chain (engine.point_tail_lanes).  Returns per group the [T, P_rank, 2] float32
+        tracks (rows that no lane writes stay zero), the flat buffer they are views of, and per group (first job, t0,
+        first point in all_pts, points of this rank)."""
         n_pix = Hf * Wf
         parts, p_off = [], 0               # per group: (first job, t0, first point in all_pts, points of this rank)
         for (j0, t0), (_, pts) in zip(spans, groups):
@@ -336,7 +434,7 @@ class VanillaTracker(nn.Module):
         if lanes:
             maps = torch.empty(T * max(ln[2] for ln in lanes) * n_pix, dtype=torch.float32, device=dev)   # NCHW scratch
             engine.point_tail_lanes(lists, pair_ref, table, lanes, lab, maps, coords, Hf, Wf, image_hw, temperature, flags)
-        return [o.double() for o in outs]
+        return outs, coords, parts
 
     def forward_test(self, rgbs, query_points, trajectories, visibilities, save_image=False, save_path=None,
                      iteration=None, shard=None):
@@ -352,18 +450,22 @@ class VanillaTracker(nn.Module):
         B, T = rgbs.shape[:2]
         h, w = rgbs.shape[-2:]
         feats = self.encode_to_bank(rgbs[0])           # FeatureBank: encoder chunks overlapped with K0
+        cycle = self.cycle_cfg() is not None
         if not self.test_cfg.get("with_first", False):
-            traj = self.propagate_points(feats, [(0, query_points[0, :, 1:])], (h, w), shard=shard)[0]
-            return trajectories, visibilities, traj[None], torch.zeros_like(visibilities), query_points
+            out = self.propagate_points(feats, [(0, query_points[0, :, 1:])], (h, w), shard=shard)
+            traj, vis_pred = (out[0][0], out[1][0][None].to(visibilities.dtype)) if cycle else \
+                (out[0], torch.zeros_like(visibilities))
+            return trajectories, visibilities, traj[None], vis_pred, query_points
         qt = query_points[0, :, 0]
         ts = torch.unique(qt).tolist()
         order = [torch.nonzero(qt == t).flatten() for t in ts]
         groups = [(int(t), query_points[0, idx, 1:]) for t, idx in zip(ts, order)]
-        trajs = self.propagate_points(feats, groups, (h, w), shard=shard)
+        out = self.propagate_points(feats, groups, (h, w), shard=shard)
+        trajs = out[0] if cycle else out
         perm = torch.cat(order)
         pred = torch.cat(trajs, dim=1).to(trajectories.dtype)[None]
-        return (trajectories[:, :, perm], visibilities[:, :, perm], pred, torch.zeros_like(visibilities),
-                query_points[:, perm])
+        vis_pred = torch.cat(out[1], dim=1)[None].to(visibilities.dtype) if cycle else torch.zeros_like(visibilities)
+        return (trajectories[:, :, perm], visibilities[:, :, perm], pred, vis_pred, query_points[:, perm])
 
     # -------------------------------------------------- VOS-style entry (mask labels)
     @torch.no_grad()

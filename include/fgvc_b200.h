@@ -97,6 +97,15 @@ typedef struct fgvc_lane {
   int64_t coord_offset;  /* floats from coords to the lane's tracks */
 } fgvc_lane;
 
+/* What fgvc_point_cycle_lanes adds to a fgvc_lane: a forward-backward check of one point group's track from frame t
+ * back toward its query frame, ending at frame s.  map_offset: the lane's L maps start map_offset maps (of H*W floats)
+ * into maps_nchw, and its L cycle positions map_offset points (of 2 floats) into xy_scratch. */
+typedef struct fgvc_cycle {
+  int32_t t;             /* frame the re-track starts from (slot 0 of the lane's bank) */
+  int32_t s;             /* frame it ends at (the lane's last slot) */
+  int64_t map_offset;
+} fgvc_cycle;
+
 /* One lane of fgvc_c2f_point_clip_tail_lanes: one coarse-to-fine recurrence of a clip (the forward or the backward
  * track of a point group) = the consecutive jobs [job_begin, job_end) in recurrence order, with their out_slots running
  * consecutively up or down.  Its fine label bank is fine_lab + lab_offset ([slot][Hf*Wf][Lp]), its coarse outputs go
@@ -320,6 +329,30 @@ FGVC_API int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* to
                          const int32_t* mem_label_slot, int32_t H, int32_t W, float temperature, int32_t flags,
                          float* lab_bank, int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
                          float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream);
+
+/* Forward-backward cycle consistency of point tracks (test_cfg.cycle_occlusion): every (group, frame t) prediction is
+ * re-tracked toward the group's query frame, and the point is visible at t iff the re-track lands within `threshold`
+ * image pixels of the group's own prediction at the frame s where it stops.  Lane i = lanes[i] + cycles[i]:
+ *   - its bank lab_bank + lab_offset holds job_end - job_begin + 1 slots of [H*W][Lp]: slot 0 is frame t, slot k the
+ *     frame of the lane's k-th job; the jobs' out_slots are 1, 2, ..., n and their memory label slots index this bank;
+ *   - its group's tracks are coords + coord_offset ([frame][L][2], read only) and its outputs go to the same places of
+ *     cycle_coords ([frame][L][2]: the re-tracked position at s, stored at row t) and vis ([frame][L] bytes, at
+ *     coord_offset / 2: 1 = visible at t).
+ * Enqueued as a constant number of launches whatever the number of lanes: ONE launch writes the gaussian labels
+ * (fgvc_gaussian_labels' arithmetic, `stride`, `sigma`) of every lane's points at coords[t] into its slot 0; the
+ * multi-lane gather chain of fgvc_point_clip_tail_lanes runs every lane's jobs (max (job_end - job_begin) grid
+ * barriers); ONE launch copies every lane's LAST slot to NCHW (maps_nchw, sum of L maps of H*W floats); ONE K3
+ * launch turns those maps into positions (xy_scratch, sum of L points); ONE launch compares them with coords[s] and
+ * writes cycle_coords and vis.  Each position is bit for bit what fgvc_point_clip_tail_lanes gives at s for a group
+ * queried at t with the same jobs.  The other arguments are fgvc_point_clip_tail_lanes'. */
+FGVC_API int fgvc_point_cycle_lanes(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
+                         const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
+                         const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, const fgvc_cycle* cycles_dev,
+                         const fgvc_cycle* cycles_host, int32_t n_lanes, const int32_t* mem_label_slot, int32_t H,
+                         int32_t W, int32_t stride, float sigma, float temperature, int32_t flags, float* lab_bank,
+                         int32_t out_h, int32_t out_w, int32_t coord_topk, float threshold, const float* coords,
+                         float* maps_nchw, float* xy_scratch, float* cycle_coords, uint8_t* vis, void* chain_ws,
+                         int64_t chain_ws_bytes, void* stream);
 
 /* K2 -- coarse-to-fine propagation (local_attention.py:721-880), single query frame.
  * Coarse stage = per-memory-frame masked argmax on the coarse bank (K1 with K=1 per
