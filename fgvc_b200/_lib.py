@@ -87,6 +87,7 @@ SIGNATURES = {
     "fgvc_mask_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, P, P, P, P, L64, P]),
     "fgvc_point_clip_tail": (I, [P, P, I, I, P, P, I, I, P, I, I, F, I, P, I, I, I, I, I, P, P, P, L64, P]),
     "fgvc_point_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, P, I, P, I, I, F, I, P, I, I, I, P, P, P, L64, P]),
+    "fgvc_mask_clip_tail_lanes": (I, [P, P, I, I, P, P, P, P, P, I, P, I, I, F, I, P, I, I, P, P, P, P, L64, P]),
     "fgvc_point_cycle_lanes": (I, [P, P, I, I, P, P, P, P, P, P, P, I, P, I, I, I, F, F, I, P, I, I, I, F, P, P, P, P, P,
                                    P, L64, P]),
     "fgvc_c2f_scratch_elems": (L64, [I, I]),

@@ -5,6 +5,35 @@
 
 using namespace fgvc;
 
+// Hard propagation over jobs [job_begin, job_end) of one label bank: the memory keeps one_hot(argmax) of every
+// propagated frame, the prediction is decoded from the soft labels first (vanilla_tracker.py:762-798) -- so gather,
+// NCHW copy, decode and hardening frame by frame.  scratch_minmax: 2L words.
+static int hard_prop_tail(const float* topk_val, const int32_t* topk_idx, int K, int groups, const fgvc_job* jobs_dev,
+                          const fgvc_job* jobs_host, int job_begin, int job_end, const int32_t* mem_label_slot, int H,
+                          int W, float temperature, int flags, float* lab_bank, int Lp, int L, int out_h, int out_w,
+                          float* scratch_minmax, uint8_t* masks, float* maps_nchw, void* stream) {
+  const int n_pix = H * W;
+  const int64_t mask_elems = (int64_t)out_h * out_w;
+  cudaStream_t st = (cudaStream_t)stream;
+  for (int j = job_begin; j < job_end; ++j) {
+    int rc = fgvc_gather_labels(topk_val, topk_idx, K, groups, jobs_dev, j, j + 1, mem_label_slot, n_pix,
+                                temperature, flags, lab_bank, Lp, stream);
+    if (rc) return rc;
+    const int slot = jobs_host[j].out_slot;
+    float* lab_slot = lab_bank + (int64_t)slot * n_pix * Lp;
+    if (maps_nchw) {
+      rc = fgvc_labels_to_nchw(lab_bank, slot, Lp, L, n_pix, maps_nchw + (int64_t)slot * L * n_pix, stream);
+      if (rc) return rc;
+    }
+    rc = launch_decode(lab_slot, true, L, Lp, H, W, out_h, out_w, reinterpret_cast<uint32_t*>(scratch_minmax),
+                       masks + slot * mask_elems, st);
+    if (rc) return rc;
+    rc = launch_labels_harden(lab_slot, n_pix, L, Lp, st);
+    if (rc) return rc;
+  }
+  return FGVC_OK;
+}
+
 // After K0 + K1 ran for the whole clip: for every job j (in order) gather the labels of its
 // query frame (K1b) and decode them to a uint8 mask of the image size.
 extern "C" int fgvc_mask_clip_tail(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
@@ -17,29 +46,10 @@ extern "C" int fgvc_mask_clip_tail(const float* topk_val, const int32_t* topk_id
   FGVC_CHECK_ARG(jobs_dev && jobs_host && masks && scratch_minmax && lab_bank, "fgvc_mask_clip_tail: null pointer");
   FGVC_CHECK_ARG(L > 0 && L <= 255 && Lp >= L && Lp % 4 == 0, "fgvc_mask_clip_tail: bad label sizes");
   const int n_pix = H * W;
-  const int64_t mask_elems = (int64_t)out_h * out_w;
   cudaStream_t st = (cudaStream_t)stream;
-  if (flags & FGVC_HARD_PROP) {
-    // hard propagation: the memory keeps one_hot(argmax) of every propagated frame, the prediction is
-    // decoded from the soft labels first (vanilla_tracker.py:762-798) -- so decode per frame
-    for (int j = job_begin; j < job_end; ++j) {
-      int rc = fgvc_gather_labels(topk_val, topk_idx, K, groups, jobs_dev, j, j + 1, mem_label_slot, n_pix,
-                                  temperature, flags, lab_bank, Lp, stream);
-      if (rc) return rc;
-      const int slot = jobs_host[j].out_slot;
-      float* lab_slot = lab_bank + (int64_t)slot * n_pix * Lp;
-      if (maps_nchw) {
-        rc = fgvc_labels_to_nchw(lab_bank, slot, Lp, L, n_pix, maps_nchw + (int64_t)slot * L * n_pix, stream);
-        if (rc) return rc;
-      }
-      rc = launch_decode(lab_slot, true, L, Lp, H, W, out_h, out_w, reinterpret_cast<uint32_t*>(scratch_minmax),
-                         masks + slot * mask_elems, st);
-      if (rc) return rc;
-      rc = launch_labels_harden(lab_slot, n_pix, L, Lp, st);
-      if (rc) return rc;
-    }
-    return FGVC_OK;
-  }
+  if (flags & FGVC_HARD_PROP)
+    return hard_prop_tail(topk_val, topk_idx, K, groups, jobs_dev, jobs_host, job_begin, job_end, mem_label_slot, H, W,
+                          temperature, flags, lab_bank, Lp, L, out_h, out_w, scratch_minmax, masks, maps_nchw, stream);
   // the recurrence lives only in the gather: run the chain first ...
   if (chain_ws != nullptr && job_end - job_begin > 1) {
     // ... as ONE persistent kernel with a grid barrier per frame (gather.cu)
@@ -65,6 +75,61 @@ extern "C" int fgvc_mask_clip_tail(const float* topk_val, const int32_t* topk_id
   // ... then decode every frame of the range in two batched launches (scratch: [n_jobs][2L] words)
   return launch_decode_jobs(lab_bank, jobs_dev, job_begin, job_end, L, Lp, H, W, out_h, out_w,
                             reinterpret_cast<uint32_t*>(scratch_minmax), masks, st);
+}
+
+// The mask tails of the independent recurrences of a clip (the forward and the backward propagation from an annotated
+// frame), each lane bit for bit fgvc_mask_clip_tail over its jobs and its bank with the chain workspace: ONE
+// multi-lane gather chain, ONE NCHW copy over every job of every lane, ONE batched decode (min-max + arg-max) over
+// every job of every lane.  With FGVC_HARD_PROP every lane runs the per-frame loop of fgvc_mask_clip_tail instead.
+extern "C" int fgvc_mask_clip_tail_lanes(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
+                                         const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
+                                         const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int32_t n_lanes,
+                                         const int32_t* mem_label_slot, int32_t H, int32_t W, float temperature,
+                                         int32_t flags, float* lab_bank, int32_t out_h, int32_t out_w,
+                                         float* scratch_minmax, uint8_t* masks, float* maps_nchw, void* chain_ws,
+                                         int64_t chain_ws_bytes, void* stream) {
+  const bool hard = (flags & FGVC_HARD_PROP) != 0;
+  FGVC_CHECK_ARG(topk_val && topk_idx && jobs_dev && jobs_host && lanes_dev && lanes_host && mem_label_slot &&
+                     lab_bank && scratch_minmax && masks && (chain_ws || hard),
+                 "fgvc_mask_clip_tail_lanes: null pointer");
+  FGVC_CHECK_ARG(K >= 1 && K <= 16, "fgvc_mask_clip_tail_lanes: topk=%d not in [1,16]", K);
+  FGVC_CHECK_ARG(n_lanes >= 1 && H > 0 && W > 0 && out_h > 0 && out_w > 0 && groups >= 1,
+                 "fgvc_mask_clip_tail_lanes: bad sizes");
+  FGVC_CHECK_ARG(pair_ref == nullptr || groups == 1, "fgvc_mask_clip_tail_lanes: shared lists need groups == 1");
+  FGVC_CHECK_ARG(pair_ref == nullptr || !hard, "fgvc_mask_clip_tail_lanes: hard propagation takes no shared lists");
+  FGVC_CHECK_ARG(temperature > 0.f, "fgvc_mask_clip_tail_lanes: temperature must be > 0");
+  int64_t n_jobs = 0;
+  for (int i = 0; i < n_lanes; ++i) {
+    const fgvc_lane& ln = lanes_host[i];
+    FGVC_CHECK_ARG(ln.job_begin >= 0 && ln.job_end > ln.job_begin, "fgvc_mask_clip_tail_lanes: lane %d is empty", i);
+    FGVC_CHECK_ARG(ln.L > 0 && ln.L <= 255 && ln.Lp >= ln.L && ln.Lp % 4 == 0 && ln.lab_offset >= 0 &&
+                       ln.lab_offset % 4 == 0 && ln.coord_offset == 0,
+                   "fgvc_mask_clip_tail_lanes: bad label sizes or offsets in lane %d", i);
+    n_jobs += ln.job_end - ln.job_begin;
+  }
+  FGVC_CHECK_ARG(n_jobs <= 65535, "fgvc_mask_clip_tail_lanes: %lld jobs in all, at most 65535", (long long)n_jobs);
+  if (hard) {
+    for (int i = 0; i < n_lanes; ++i) {
+      const fgvc_lane& ln = lanes_host[i];
+      int rc = hard_prop_tail(topk_val, topk_idx, K, groups, jobs_dev, jobs_host, ln.job_begin, ln.job_end,
+                              mem_label_slot, H, W, temperature, flags, lab_bank + ln.lab_offset, ln.Lp, ln.L, out_h,
+                              out_w, scratch_minmax, masks, maps_nchw, stream);
+      if (rc) return rc;
+    }
+    return FGVC_OK;
+  }
+  const int n_pix = H * W;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = launch_gather_chain_lanes(topk_val, topk_idx, K, groups, jobs_dev, lanes_dev, lanes_host, n_lanes,
+                                     mem_label_slot, pair_ref, n_pix, temperature, flags, lab_bank, chain_ws,
+                                     chain_ws_bytes, st);
+  if (rc) return rc;
+  if (maps_nchw) {
+    rc = launch_labels_to_nchw_lanes(lab_bank, jobs_dev, lanes_dev, lanes_host, n_lanes, n_pix, maps_nchw, st);
+    if (rc) return rc;
+  }
+  return launch_decode_lanes(lab_bank, jobs_dev, lanes_dev, lanes_host, n_lanes, H, W, out_h, out_w,
+                             reinterpret_cast<uint32_t*>(scratch_minmax), masks, st);
 }
 
 // Lowest out_slot of jobs [job_begin, job_end) when their out_slots run consecutively up (a forward track) or down (a

@@ -205,6 +205,52 @@ struct c2f_wjob {
   int64_t list_off;     // elements: lists [Hc * Wc][n_mem * chunks][K]
 };
 
+// Batched label-side launches (NCHW copy, mask decode) over a list of jobs: grid index z -> the job's label bank, its
+// out_slot, its label sizes and its decode min-max keys.  One kernel body serves both forms below.
+struct JobRef {
+  const float* lab;      // the job's label bank ([slot][H*W][Lp])
+  int slot, L, Lp;
+  uint32_t* mn;          // [L] min keys of the job's decode
+  uint32_t* mx;          // [L] max keys
+};
+// jobs [job_begin, job_begin + n) of one bank; min-max keys interleaved per job: minmax[z][2L]
+struct RangeJobs {
+  const float* lab;
+  const fgvc_job* jobs;
+  int job_begin, L, Lp;
+  uint32_t* minmax;
+  __device__ __forceinline__ JobRef at(int z) const {
+    uint32_t* mm = minmax + (int64_t)z * 2 * L;
+    return JobRef{lab, jobs[job_begin + z].out_slot, L, Lp, mm, mm + L};
+  }
+};
+// every job of lanes[0, n_lanes), lane after lane, each lane over its bank lab + lab_offset; min keys of all jobs first
+// (minmax[0, n_keys)), then their max keys (minmax[n_keys, 2 n_keys)), job after job with the lane's L keys each
+struct LaneJobs {
+  const float* lab;
+  const fgvc_job* jobs;
+  const fgvc_lane* lanes;
+  int n_lanes;
+  uint32_t* minmax;
+  int64_t n_keys;
+  __device__ __forceinline__ JobRef at(int z) const {
+    int l = 0;
+    int64_t key = 0;
+    for (;;) {
+      const int n = __ldg(&lanes[l].job_end) - __ldg(&lanes[l].job_begin), L = __ldg(&lanes[l].L);
+      if (z < n || l == n_lanes - 1) break;
+      z -= n;
+      key += (int64_t)n * L;
+      ++l;
+    }
+    const fgvc_lane& ln = lanes[l];
+    const int L = __ldg(&ln.L);
+    key += (int64_t)z * L;
+    return JobRef{lab + __ldg(&ln.lab_offset), jobs[__ldg(&ln.job_begin) + z].out_slot, L, __ldg(&ln.Lp), minmax + key,
+                  minmax + n_keys + key};
+  }
+};
+
 // host launchers implemented in the .cu files -------------------------------------------
 int launch_affinity_topk_simt(const void* bank, int fmt, int H, int W, int C, const fgvc_job* jobs, int n_jobs,
                               const int32_t* mem_feat, int radius, int mode, int K, int groups,
@@ -251,6 +297,11 @@ int launch_c2f_chain_lanes(const float* cw, const int32_t* crow, int K, int job_
                            int Hf, int Wf, float* fine_lab, float* coarse_out, unsigned int* barrier, cudaStream_t st);
 int launch_decode_jobs(const float* lab, const fgvc_job* jobs_dev, int job_begin, int job_end, int L, int Lp, int H,
                        int W, int out_h, int out_w, uint32_t* minmax, uint8_t* masks, cudaStream_t st);
+int launch_labels_to_nchw_lanes(const float* lab, const fgvc_job* jobs_dev, const fgvc_lane* lanes_dev,
+                                const fgvc_lane* lanes_host, int n_lanes, int n_pix, float* maps_nchw, cudaStream_t st);
+int launch_decode_lanes(const float* lab, const fgvc_job* jobs_dev, const fgvc_lane* lanes_dev,
+                        const fgvc_lane* lanes_host, int n_lanes, int H, int W, int out_h, int out_w, uint32_t* minmax,
+                        uint8_t* masks, cudaStream_t st);
 int launch_labels_harden(float* lab_slot, int n_pix, int L, int Lp, cudaStream_t st);
 int launch_decode(const float* src, bool pixmajor, int L, int Lp, int H, int W, int out_h, int out_w,
                   uint32_t* minmax, uint8_t* out, cudaStream_t st);

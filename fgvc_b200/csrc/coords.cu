@@ -477,19 +477,20 @@ decode_argmax_kernel(const float* __restrict__ src, int L, int H, int W, int str
   out[o] = (uint8_t)arg;
 }
 
-// batched form for a clip: blockIdx.y walks jobs [job_begin, job_end); each decodes the label-bank
-// slot jobs[j].out_slot into masks[slot] using minmax[j - job_begin][2L]
+// batched form for a clip: blockIdx.y walks a list of jobs (a job range of one bank, or every job of several lanes);
+// each decodes the label-bank slot of its out_slot into masks[slot] using its own min-max keys
 // Per-channel min / max of the up-sampled map.  Within one source cell the bilinear value is
 // monotone along each axis, so its extremes over the output pixels of that cell sit on the four
 // corner-most output pixels: 4 evaluations per cell instead of (out/in)^2.  One thread per source
 // cell; the values are produced by the same tap arithmetic as the arg-max pass.
+// Jobs: RangeJobs or LaneJobs (common.cuh), blockIdx.y = job.
+template <class Jobs>
 __global__ void __launch_bounds__(256)
-decode_minmax_jobs_kernel(const float* __restrict__ lab, const fgvc_job* __restrict__ jobs, int job_begin, int L,
-                          int Lp, int H, int W, int out_h, int out_w, uint32_t* __restrict__ minmax) {
+decode_minmax_jobs_kernel(const Jobs jobs, int H, int W, int out_h, int out_w) {
   extern __shared__ uint32_t skey[];   // [2L]
-  const int slot = jobs[job_begin + blockIdx.y].out_slot;
-  const float* src = lab + (int64_t)slot * H * W * Lp;
-  uint32_t* mm = minmax + (int64_t)blockIdx.y * 2 * L;
+  const JobRef jr = jobs.at(blockIdx.y);
+  const int L = jr.L, Lp = jr.Lp;
+  const float* src = jr.lab + (int64_t)jr.slot * H * W * Lp;
   for (int i = threadIdx.x; i < 2 * L; i += 256) skey[i] = i < L ? 0xffffffffu : 0u;
   __syncthreads();
   const int cell = blockIdx.x * 256 + threadIdx.x;
@@ -527,26 +528,26 @@ decode_minmax_jobs_kernel(const float* __restrict__ lab, const fgvc_job* __restr
   }
   __syncthreads();
   for (int i = threadIdx.x; i < 2 * L; i += 256) {
-    if (i < L) atomicMin(mm + i, skey[i]);
-    else atomicMax(mm + i, skey[i]);
+    if (i < L) atomicMin(jr.mn + i, skey[i]);
+    else atomicMax(jr.mx + (i - L), skey[i]);
   }
 }
 
 // One CTA = a 64 x 4 tile of output pixels of one frame (blockIdx.z): no index division, neighbouring threads share
 // their source taps.  Per-channel constants in shared memory as (min, max, reciprocal of the range, -).
+template <class Jobs>
 __global__ void __launch_bounds__(256)
-decode_argmax_jobs_kernel(const float* __restrict__ lab, const fgvc_job* __restrict__ jobs, int job_begin, int L,
-                          int Lp, int H, int W, int out_h, int out_w, const uint32_t* __restrict__ minmax,
-                          uint8_t* __restrict__ masks) {
+decode_argmax_jobs_kernel(const Jobs jobs, int H, int W, int out_h, int out_w, uint8_t* __restrict__ masks) {
   // [Lp] (min, divisor, reciprocal of the divisor, -) with divisor = (max - min) + 1e-12.  Channels that are not
   // normalised (max <= 0: the map stays as it is) get (0, 1, 1): (v - 0) / 1 = v exactly; the pad channels get
   // min = +inf: their value becomes -inf and can never win.  The inner loop then has no per-channel case split.
   extern __shared__ float4 scst[];
-  const uint32_t* mm = minmax + (int64_t)blockIdx.z * 2 * L;
+  const JobRef jr = jobs.at(blockIdx.z);
+  const int L = jr.L, Lp = jr.Lp;
   for (int i = threadIdx.x; i < Lp; i += 256) {
     float4 cs = make_float4(INFINITY, 1.f, 1.f, 0.f);
     if (i < L) {
-      const float mn = key2f(__ldg(mm + i)), mx = key2f(__ldg(mm + L + i));
+      const float mn = key2f(__ldg(jr.mn + i)), mx = key2f(__ldg(jr.mx + i));
       const float dv = (mx - mn) + 1e-12f;
       cs = mx > 0.f ? make_float4(mn, dv, __frcp_rn(dv), 0.f) : make_float4(0.f, 1.f, 1.f, 0.f);
     }
@@ -555,8 +556,8 @@ decode_argmax_jobs_kernel(const float* __restrict__ lab, const fgvc_job* __restr
   __syncthreads();
   const int ox = blockIdx.x * 64 + (threadIdx.x & 63), oy = blockIdx.y * 4 + (threadIdx.x >> 6);
   if (ox >= out_w || oy >= out_h) return;
-  const int slot = jobs[job_begin + blockIdx.z].out_slot;
-  const float4* src = reinterpret_cast<const float4*>(lab + (int64_t)slot * H * W * Lp);
+  const int slot = jr.slot;
+  const float4* src = reinterpret_cast<const float4*>(jr.lab + (int64_t)slot * H * W * Lp);
   const int l4n = Lp / 4;
   const Tap t = make_tap(oy, ox, H, W, (float)H / (float)out_h, (float)W / (float)out_w);
   const float4* s00 = src + (int64_t)t.p00 * l4n;
@@ -598,11 +599,36 @@ int launch_decode_jobs(const float* lab, const fgvc_job* jobs_dev, int job_begin
   init_minmax_kernel<<<cdiv(n * 2 * L, 256), 256, 0, st>>>(minmax, n, L);
   FGVC_LAUNCH_CHECK();
   dim3 grid(cdiv(out_w, 64), cdiv(out_h, 4), n), grid_cells(cdiv(H * W, 256), n);
-  decode_minmax_jobs_kernel<<<grid_cells, 256, 2 * L * 4, st>>>(lab, jobs_dev, job_begin, L, Lp, H, W, out_h, out_w,
-                                                               minmax);
+  const RangeJobs jobs{lab, jobs_dev, job_begin, L, Lp, minmax};
+  decode_minmax_jobs_kernel<<<grid_cells, 256, 2 * L * 4, st>>>(jobs, H, W, out_h, out_w);
   FGVC_LAUNCH_CHECK();
-  decode_argmax_jobs_kernel<<<grid, 256, Lp * 16, st>>>(lab, jobs_dev, job_begin, L, Lp, H, W, out_h, out_w, minmax,
-                                                       masks);
+  decode_argmax_jobs_kernel<<<grid, 256, Lp * 16, st>>>(jobs, H, W, out_h, out_w, masks);
+  FGVC_LAUNCH_CHECK();
+  return FGVC_OK;
+}
+
+// The decode of every job of every lane (LaneJobs) in the two launches above; the min-max keys are initialised by two
+// memsets (min keys first, then max keys), so the decode is two kernel launches whatever the number of lanes.
+int launch_decode_lanes(const float* lab, const fgvc_job* jobs_dev, const fgvc_lane* lanes_dev,
+                        const fgvc_lane* lanes_host, int n_lanes, int H, int W, int out_h, int out_w, uint32_t* minmax,
+                        uint8_t* masks, cudaStream_t st) {
+  int n = 0, max_L = 1, max_Lp = 4;
+  int64_t n_keys = 0;
+  for (int i = 0; i < n_lanes; ++i) {
+    const int len = lanes_host[i].job_end - lanes_host[i].job_begin;
+    n += len;
+    n_keys += (int64_t)len * lanes_host[i].L;
+    max_L = max(max_L, lanes_host[i].L);
+    max_Lp = max(max_Lp, lanes_host[i].Lp);
+  }
+  if (n <= 0) return FGVC_OK;
+  FGVC_CUDA(cudaMemsetAsync(minmax, 0xff, (size_t)n_keys * 4, st));
+  FGVC_CUDA(cudaMemsetAsync(minmax + n_keys, 0x00, (size_t)n_keys * 4, st));
+  dim3 grid(cdiv(out_w, 64), cdiv(out_h, 4), n), grid_cells(cdiv(H * W, 256), n);
+  const LaneJobs jobs{lab, jobs_dev, lanes_dev, n_lanes, minmax, n_keys};
+  decode_minmax_jobs_kernel<<<grid_cells, 256, 2 * max_L * 4, st>>>(jobs, H, W, out_h, out_w);
+  FGVC_LAUNCH_CHECK();
+  decode_argmax_jobs_kernel<<<grid, 256, max_Lp * 16, st>>>(jobs, H, W, out_h, out_w, masks);
   FGVC_LAUNCH_CHECK();
   return FGVC_OK;
 }

@@ -122,15 +122,18 @@ labels_to_nchw_kernel(const float* __restrict__ src, int Lp, int L, int n_pix, f
   }
 }
 
-// the same for the out_slots of jobs [job_begin, job_begin + gridDim.z): dst[slot][L][n_pix]
+// the same for the out_slots of a list of jobs (Jobs: RangeJobs or LaneJobs of common.cuh, job = blockIdx.z):
+// dst[slot][L][n_pix] with the job's L
+template <class Jobs>
 __global__ void __launch_bounds__(256)
-labels_to_nchw_jobs_kernel(const float* __restrict__ lab, const fgvc_job* __restrict__ jobs, int job_begin, int Lp, int L,
-                           int n_pix, float* __restrict__ maps) {
+labels_to_nchw_jobs_kernel(const Jobs jobs, int n_pix, float* __restrict__ maps) {
   __shared__ float t[32][33];
-  const int slot = jobs[job_begin + blockIdx.z].out_slot;
-  const float* src = lab + (int64_t)slot * n_pix * Lp;
+  const JobRef jr = jobs.at(blockIdx.z);
+  const int slot = jr.slot, L = jr.L, Lp = jr.Lp;
+  const float* src = jr.lab + (int64_t)slot * n_pix * Lp;
   float* dst = maps + (int64_t)slot * L * n_pix;
   const int p0 = blockIdx.x * 32, l0 = blockIdx.y * 32;
+  if (l0 >= L) return;                                     // (whole block: a lane with fewer channels)
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   for (int j = ty; j < 32; j += 8) {
     int p = p0 + j, l = l0 + tx;
@@ -145,14 +148,16 @@ labels_to_nchw_jobs_kernel(const float* __restrict__ lab, const fgvc_job* __rest
 
 // wide variant (n_pix % 4 == 0): 64 pixels x 64 channels per CTA, 16-byte loads along the channels and 16-byte
 // stores along the pixels
+template <class Jobs>
 __global__ void __launch_bounds__(256)
-labels_to_nchw_jobs_wide_kernel(const float* __restrict__ lab, const fgvc_job* __restrict__ jobs, int job_begin, int Lp,
-                                int L, int n_pix, float* __restrict__ maps) {
+labels_to_nchw_jobs_wide_kernel(const Jobs jobs, int n_pix, float* __restrict__ maps) {
   __shared__ float t[64][65];
-  const int slot = jobs[job_begin + blockIdx.z].out_slot;
-  const float* src = lab + (int64_t)slot * n_pix * Lp;
+  const JobRef jr = jobs.at(blockIdx.z);
+  const int slot = jr.slot, L = jr.L, Lp = jr.Lp;
+  const float* src = jr.lab + (int64_t)slot * n_pix * Lp;
   float* dst = maps + (int64_t)slot * L * n_pix;
   const int p0 = blockIdx.x * 64, l0 = blockIdx.y * 64;
+  if (l0 >= L) return;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
 #pragma unroll
   for (int j = ty; j < 64; j += 16) {
@@ -234,15 +239,36 @@ int launch_labels_to_nchw_jobs(const float* lab, const fgvc_job* jobs_dev, int j
   if (n <= 0) return FGVC_OK;
   const bool wide = n_pix % 4 == 0 && L >= 32 && (reinterpret_cast<uintptr_t>(maps_nchw) & 15) == 0;
   for (int z0 = 0; z0 < n; z0 += 65535) {
+    const RangeJobs jobs{lab, jobs_dev, job_begin + z0, L, Lp, nullptr};
     if (wide) {
       dim3 grid(cdiv(n_pix, 64), cdiv(L, 64), min(65535, n - z0));
-      labels_to_nchw_jobs_wide_kernel<<<grid, 256, 0, st>>>(lab, jobs_dev, job_begin + z0, Lp, L, n_pix, maps_nchw);
+      labels_to_nchw_jobs_wide_kernel<<<grid, 256, 0, st>>>(jobs, n_pix, maps_nchw);
     } else {
       dim3 grid(cdiv(n_pix, 32), cdiv(L, 32), min(65535, n - z0));
-      labels_to_nchw_jobs_kernel<<<grid, 256, 0, st>>>(lab, jobs_dev, job_begin + z0, Lp, L, n_pix, maps_nchw);
+      labels_to_nchw_jobs_kernel<<<grid, 256, 0, st>>>(jobs, n_pix, maps_nchw);
     }
     FGVC_LAUNCH_CHECK();
   }
+  return FGVC_OK;
+}
+
+// the NCHW copies of every job of every lane in ONE launch (at most 65535 jobs in all, checked by the caller)
+int launch_labels_to_nchw_lanes(const float* lab, const fgvc_job* jobs_dev, const fgvc_lane* lanes_dev,
+                                const fgvc_lane* lanes_host, int n_lanes, int n_pix, float* maps_nchw, cudaStream_t st) {
+  int n = 0, min_L = lanes_host[0].L, max_L = 1;
+  for (int i = 0; i < n_lanes; ++i) {
+    n += lanes_host[i].job_end - lanes_host[i].job_begin;
+    min_L = min(min_L, lanes_host[i].L);
+    max_L = max(max_L, lanes_host[i].L);
+  }
+  if (n <= 0) return FGVC_OK;
+  const LaneJobs jobs{lab, jobs_dev, lanes_dev, n_lanes, nullptr, 0};
+  if (n_pix % 4 == 0 && min_L >= 32 && (reinterpret_cast<uintptr_t>(maps_nchw) & 15) == 0) {
+    labels_to_nchw_jobs_wide_kernel<<<dim3(cdiv(n_pix, 64), cdiv(max_L, 64), n), 256, 0, st>>>(jobs, n_pix, maps_nchw);
+  } else {
+    labels_to_nchw_jobs_kernel<<<dim3(cdiv(n_pix, 32), cdiv(max_L, 32), n), 256, 0, st>>>(jobs, n_pix, maps_nchw);
+  }
+  FGVC_LAUNCH_CHECK();
   return FGVC_OK;
 }
 

@@ -827,24 +827,43 @@ def c2f_propagate(coarse, fine, table, job_index, fine_labels, radius, radius_fi
     return out
 
 
+def check_ref_frame(ref_frame, T):
+    """``ref_frame`` of a T-frame mask clip as an int in [0, T); ValueError otherwise."""
+    if isinstance(ref_frame, bool) or not isinstance(ref_frame, (int, np.integer)) or not 0 <= int(ref_frame) < T:
+        raise ValueError(f"ref_frame must be an int in [0, {T}), got {ref_frame!r}")
+    return int(ref_frame)
+
+
 class MaskClipPropagator:
     """VOS-style propagation of one clip with pre-allocated banks (the loop of
     vanilla_tracker.py:345-412 / :730-798 for mask labels): K0 over all frames, ONE K1 launch
     over all frames' jobs, then per frame K1b gather -> NCHW -> decode (bilinear up-sample,
-    min-max normalise, argmax).  ``events=True`` records CUDA events around K1."""
+    min-max normalise, argmax).  ``events=True`` records CUDA events around K1.
 
-    def __init__(self, T, C, H, W, L, out_hw, cfg, device, engine_id=_lib.ENGINE_AUTO, split=None):
+    ``ref_frame`` = t0: the annotated frame.  The masks of frames t0+1 .. T-1 are the propagation of the clip from t0
+    on (memory_frames with first = t0), those of frames t0-1 .. 0 the propagation of the time-reversed clip from t0
+    (track_memory); each half is bit for bit the run of this class with ref_frame = 0 on the sliced / the flipped clip
+    when that run tiles K1 the same way (a shorter clip may pick more partial lists per job, plan_k1; exactly tied
+    affinities may then be merged in another order).
+    K1 runs once over both directions (no query tile mixes them), and the two tails are the two lanes of one
+    fgvc_mask_clip_tail_lanes call: max(t0, T-1-t0) grid barriers instead of T-1.  ref_frame = 0 is the plain forward
+    propagation through fgvc_mask_clip_tail."""
+
+    def __init__(self, T, C, H, W, L, out_hw, cfg, device, engine_id=_lib.ENGINE_AUTO, split=None, ref_frame=0):
         self.T, self.C, self.H, self.W, self.L, self.out_hw, self.cfg = T, C, H, W, L, tuple(out_hw), cfg
+        self.ref_frame = t0 = check_ref_frame(ref_frame, T)
         self.engine_id = engine_id
         self.device = device
         self.bank = FeatureBank(T, C, H, W, device, split=split or cfg.get("split"))
         self.labels = LabelBank(T, L, H, W, device)
-        self.table = JobTable()
         nr = cfg.get("neighbor_range", None)
         unmasked_first = 0 if cfg.get("with_first_neighbor", True) else 1
-        for t in range(1, T):
-            mem = memory_frames(t, cfg["precede_frames"], cfg.get("with_first", True))
-            self.table.add(t, mem, mem, t, unmasked=len(mem) if nr is None else unmasked_first)
+        # forward jobs t0+1 .. T-1, then backward jobs t0-1 .. 0 (with t0 = 0: today's jobs 1 .. T-1)
+        self.table, _ = query_job_table([t0], T, cfg["precede_frames"], cfg.get("with_first", True), True,
+                                        lambda mem: len(mem) if nr is None else unmasked_first)
+        self.n_fwd = T - 1 - t0
+        # the lanes of the tail: (job_begin, job_end) of each non-empty direction
+        self.lanes = [(a, b) for a, b in ((0, self.n_fwd), (self.n_fwd, len(self.table))) if b > a]
         self.radius = (nr // 2) if nr is not None else 1
         # the tiling of K1 (jobs per tile, aligned memory classes, parts) is fixed per clip: it sizes the lists
         self.plan = plan_k1(self.bank, self.table, self.radius, cfg["topk"], cfg.get("mask_mode", "circle"),
@@ -858,9 +877,15 @@ class MaskClipPropagator:
         self.k1_events = None
         self._tail_stream = None
         # optional: K1 in a few launches with the gather chain of chunk i on a side stream under K1 of chunk
-        # i+1.  Measured on config 2 it does not pay (the tail is real SM work, not latency): off by default.
+        # i+1.  Measured on config 2 it does not pay (the tail is real SM work, not latency): off by default, and
+        # forward propagation (ref_frame = 0) only.
         self._overlap = (plan_overlap_chunks(len(self.table), (-(-H // 8)) * (-(-W // 16)))
-                         if (T > 1 and cfg.get("overlap_tail", False)) else [])
+                         if (T > 1 and t0 == 0 and cfg.get("overlap_tail", False)) else [])
+        self._lanes_dev = None
+        if t0 > 0:
+            host = (_lib.Lane * len(self.lanes))(*[_lib.Lane(a, b, L, self.labels.Lp, 0, 0) for a, b in self.lanes])
+            self._lanes_host = host
+            self._lanes_dev = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(device)
         self.temperature, self.flags = sim_params(cfg, C, cfg["temperature"], sim_mode=cfg.get("sim_mode", "dot_product"),
                                                   normalize=cfg.get("with_norm", True))
         if cfg.get("hard_prop", False):
@@ -873,6 +898,18 @@ class MaskClipPropagator:
         masks = self.masks if masks is None else masks
         call("fgvc_decode_masks_pixmajor", ptr(self.labels.buf), t, self.labels.Lp, self.L, self.H, self.W,
              self.out_hw[0], self.out_hw[1], ptr(self.scratch), ptr(masks[t]), stream_ptr())
+
+    def _tail_lanes(self, want_maps):
+        """both directions from ref_frame > 0: the two lanes of one fgvc_mask_clip_tail_lanes call over the one bank"""
+        lists = self.lists
+        jobs, _, mem_label = self.table.device(self.device)
+        call("fgvc_mask_clip_tail_lanes", ptr(lists.val), ptr(lists.idx), lists.K, lists.groups, None, ptr(jobs),
+             ptr(self.jobs_host), ptr(self._lanes_dev), ctypes.c_void_p(ctypes.addressof(self._lanes_host)),
+             len(self.lanes), ptr(mem_label), self.H, self.W, self.temperature, self.flags, ptr(self.labels.buf),
+             self.out_hw[0], self.out_hw[1], ptr(self.scratch), ptr(self.masks),
+             ptr(self.maps) if want_maps else None,
+             *chain_workspace(self.device, len(self.table), self.H * self.W, lists.K, self.flags,
+                              force=not (self.flags & _lib.HARD_PROP)), stream_ptr())
 
     def _tail(self, j0, j1, want_maps, lists=None, masks=None):
         lists = lists or self.lists
@@ -887,23 +924,31 @@ class MaskClipPropagator:
     def _k1(self, j0, j1, lists=None):
         cfg = self.cfg
         lists = lists or self.lists
+        # both directions: no query tile mixes them, so each gets the lists (and the K1 cost) of a run of its own
         affinity_topk(self.bank, self.table, self.radius, cfg["topk"], cfg.get("mask_mode", "circle"),
-                      engine=self.engine_id, lists=lists, job_range=(j0, j1), plan=self.plan)
+                      engine=self.engine_id, lists=lists, job_range=(j0, j1), plan=self.plan,
+                      cuts=self.lanes if self.ref_frame > 0 else None)
 
-    def run(self, feats, onehot0, events=False, want_maps=True):
-        """feats [T,C,H,W] fp32 CUDA; onehot0 [L,H,W] fp32 CUDA.  Returns (maps, masks);
-        ``want_maps=False`` skips the NCHW copies of the propagated label maps."""
+    def run(self, feats, onehot, events=False, want_maps=True):
+        """feats [T,C,H,W] fp32 CUDA; onehot [L,H,W] fp32 CUDA, the labels of frame ``ref_frame``.  Returns (maps,
+        masks); ``want_maps=False`` skips the NCHW copies of the propagated label maps."""
         cfg = self.cfg
+        t0 = self.ref_frame
         self.bank.load_frames(feats, 0, normalize=cfg.get("with_norm", True))
-        self.labels.put_nchw(onehot0, 0)
+        self.labels.put_nchw(onehot, t0)
         if want_maps:
-            self.maps[0].copy_(onehot0)
-        self._decode(0)
+            self.maps[t0].copy_(onehot)
+        self._decode(t0)
         if self.T > 1:
             if events:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-            if len(self._overlap) <= 1:
+            if t0 > 0:
+                self._k1(0, len(self.table))
+                if events:
+                    e1.record()
+                self._tail_lanes(want_maps)
+            elif len(self._overlap) <= 1:
                 self._k1(0, len(self.table))
                 if events:
                     e1.record()
@@ -939,7 +984,11 @@ class MaskClipPropagator:
           * across clips the staging buffers are double-buffered, so the copies of the NEXT call start while this
             call still computes (they only wait for the K0 launches that read the same staging buffer two calls
             ago).  For a stream of clips ``chunks=[(0, n_jobs)]`` is then the fastest plan: the copies are
-            hidden behind the previous clip and K1 runs as one launch."""
+            hidden behind the previous clip and K1 runs as one launch.
+        The chunked upload relies on every job reading earlier frames only: ``ref_frame > 0`` (backward jobs read
+        later frames) raises NotImplementedError; use ``run`` for it."""
+        if self.ref_frame != 0:
+            raise NotImplementedError("run_host propagates from frame 0 only; use run() for ref_frame > 0")
         cfg = self.cfg
         if not hasattr(self, "_stage"):
             self._stage = [torch.empty(self.T, self.C, self.H, self.W, dtype=torch.float32, device=self.device)

@@ -469,14 +469,17 @@ class VanillaTracker(nn.Module):
 
     # -------------------------------------------------- VOS-style entry (mask labels)
     @torch.no_grad()
-    def propagate_masks(self, feats, ref_seg, out_hw, num_classes=None):
-        """feats [T,C,Hf,Wf]; ref_seg int [Hf,Wf] (first-frame mask already at feature
-        resolution).  Returns (label maps [T,L,Hf,Wf], uint8 masks [T,h,w]) with the
-        decode of vanilla_tracker.py:769-798."""
+    def propagate_masks(self, feats, ref_seg, out_hw, num_classes=None, ref_frame=0):
+        """feats [T,C,Hf,Wf]; ref_seg int [Hf,Wf]: the mask of frame ``ref_frame`` (default: the first frame), already
+        at feature resolution.  Returns (label maps [T,L,Hf,Wf], uint8 masks [T,h,w]) with the decode of
+        vanilla_tracker.py:769-798.  With ref_frame = t0 > 0 the frames after t0 are propagated forward from t0 and
+        the frames before it backward (the forward propagation of the time-reversed clip from t0), in one call."""
         T, C, Hf, Wf = feats.shape
+        ref_frame = engine.check_ref_frame(ref_frame, T)
         dev = feats.device
         onehot = torch.nn.functional.one_hot(ref_seg.long().to(dev), num_classes).permute(2, 0, 1).float().contiguous()
-        clip = engine.MaskClipPropagator(T, C, Hf, Wf, onehot.shape[0], out_hw, self.test_cfg, dev, self.engine_id)
+        clip = engine.MaskClipPropagator(T, C, Hf, Wf, onehot.shape[0], out_hw, self.test_cfg, dev, self.engine_id,
+                                         ref_frame=ref_frame)
         return clip.run(feats.float().contiguous(), onehot)
 
 
@@ -518,16 +521,20 @@ class HRVanillaTracker(VanillaTracker):
         self.hard_prop = self.test_cfg.get("hard_prop", False)
 
     @torch.no_grad()
-    def forward_test_vos(self, imgs, ref_seg_map, img_meta, save_image=False, save_path=None, iteration=None):
-        """imgs [1, n, 3, T, h, w] (or [1, 3, T, h, w]); ref_seg_map [1, h, w] integer labels of frame 0;
-        img_meta[0]['original_shape'].  Returns a list with one uint8/int array [T, H0, W0] of per-frame label
-        masks (frame 0 = the given mask), as the reference's ``list(all_seg_preds)`` for integer input."""
+    def forward_test_vos(self, imgs, ref_seg_map, img_meta, save_image=False, save_path=None, iteration=None,
+                         ref_frame=0):
+        """imgs [1, n, 3, T, h, w] (or [1, 3, T, h, w]); ref_seg_map [1, h, w] integer labels of frame ``ref_frame``
+        (default 0); img_meta[0]['original_shape'].  Returns a list with one uint8/int array [T, H0, W0] of per-frame
+        label masks (frame ``ref_frame`` = the given mask), as the reference's ``list(all_seg_preds)`` for integer
+        input.  With ref_frame = t0 > 0 the frames after t0 are propagated forward from t0 and the frames before it
+        backward, as the reference does on the time-reversed clip from t0."""
         _lib.require_cuda()
         dev = torch.device("cuda", torch.cuda.current_device())
         imgs = imgs.to(dev)
         if imgs.ndim == 6:
             imgs = imgs.reshape((-1,) + imgs.shape[2:])
         assert imgs.shape[0] == 1 and ref_seg_map.ndim == 3, "one clip, integer reference mask"
+        ref_frame = engine.check_ref_frame(ref_frame, imgs.shape[2])
         h, w = imgs.shape[-2:]
         imgs, _ = pad_divide_by(imgs, self.stride)
         seg, pa = pad_divide_by(ref_seg_map.to(dev), self.stride)
@@ -544,7 +551,8 @@ class HRVanillaTracker(VanillaTracker):
         cfg.update(mask_mode="square", local_window=True, with_first_neighbor=True,
                    with_norm=self.test_cfg.get("with_norm", True))
         direct = sum(pa) == 0 and (oh, ow) == (h, w)
-        clip = engine.MaskClipPropagator(T, C, Hf, Wf, L, (oh, ow) if direct else pad_shape, cfg, dev, self.engine_id)
+        clip = engine.MaskClipPropagator(T, C, Hf, Wf, L, (oh, ow) if direct else pad_shape, cfg, dev, self.engine_id,
+                                         ref_frame=ref_frame)
         maps, masks = clip.run(feats.float().contiguous(), onehot, want_maps=not direct)
         if direct:
             out = masks.clone()
@@ -558,7 +566,7 @@ class HRVanillaTracker(VanillaTracker):
             lo, hi = p.amin(dim=(2, 3), keepdim=True), p.amax(dim=(2, 3), keepdim=True)
             p = torch.where(hi > 0, (p - lo) / (hi - lo + 1e-12), p)
             out = p.argmax(dim=1).to(torch.uint8)
-        out[0] = first.to(out.dtype)
+        out[ref_frame] = first.to(out.dtype)
         return [out.cpu().numpy()]
 
 

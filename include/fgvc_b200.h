@@ -87,7 +87,8 @@ typedef struct fgvc_job {
 /* One lane of fgvc_point_clip_tail_lanes: one recurrence of a clip (the forward or the backward track of a point group)
  * = the consecutive jobs [job_begin, job_end) in recurrence order, with their out_slots running consecutively up or
  * down, over its own label bank lab_bank + lab_offset ([slot][H*W][Lp]) and its own tracks coords + coord_offset
- * ([slot][L][2]).  Two lanes may share a bank when neither reads a slot the other writes. */
+ * ([slot][L][2]).  Two lanes may share a bank when neither reads a slot the other writes.  fgvc_mask_clip_tail_lanes
+ * takes the same table with coord_offset = 0. */
 typedef struct fgvc_lane {
   int32_t job_begin;
   int32_t job_end;
@@ -329,6 +330,27 @@ FGVC_API int fgvc_point_clip_tail_lanes(const float* topk_val, const int32_t* to
                          const int32_t* mem_label_slot, int32_t H, int32_t W, float temperature, int32_t flags,
                          float* lab_bank, int32_t out_h, int32_t out_w, int32_t coord_topk, float* maps_nchw,
                          float* coords, void* chain_ws, int64_t chain_ws_bytes, void* stream);
+
+/* Mask tails of the independent recurrences of one clip: the propagation from an annotated frame t0 forward to T-1
+ * and backward to 0 (the forward propagation of the time-reversed clip), or any other set of job ranges.  Each lane
+ * (fgvc_lane; coord_offset unused, must be 0) is the mask tail above over its own job range and its own label bank
+ * lab_bank + lab_offset, and gives bit for bit what fgvc_mask_clip_tail gives for it with the chain workspace: masks
+ * into masks[slot][out_h][out_w] and, when maps_nchw is given, NCHW copies into maps_nchw + slot * L * H*W (the lane's
+ * L).  Two lanes may share a bank when neither reads a slot the other writes (the two directions of one annotated
+ * frame both read slot t0); lanes write distinct out_slots of masks / maps_nchw.  Enqueued as ONE multi-lane gather
+ * chain (one weight launch + one cooperative kernel, the longest lane's length of grid barriers, as in
+ * fgvc_point_clip_tail_lanes), ONE NCHW-copy launch over every job of every lane (when maps_nchw is given) and ONE
+ * batched decode over every job of every lane (min-max launch + arg-max launch).  pair_ref: NULL or shared lists, as in
+ * fgvc_point_clip_tail_lanes.  scratch_minmax: 2 L words per job, summed over all lanes.  chain_ws (required without
+ * FGVC_HARD_PROP): fgvc_chain_workspace_bytes(je - jb, H*W, K) bytes, [jb, je) = the smallest job range holding every
+ * lane.  With FGVC_HARD_PROP every lane runs the per-frame loop of fgvc_mask_clip_tail (decode before hardening: not
+ * batched), lane after lane; pair_ref must then be NULL.  At most 65535 jobs in all, L <= 255. */
+FGVC_API int fgvc_mask_clip_tail_lanes(const float* topk_val, const int32_t* topk_idx, int32_t K, int32_t groups,
+                         const int32_t* pair_ref, const fgvc_job* jobs_dev, const fgvc_job* jobs_host,
+                         const fgvc_lane* lanes_dev, const fgvc_lane* lanes_host, int32_t n_lanes,
+                         const int32_t* mem_label_slot, int32_t H, int32_t W, float temperature, int32_t flags,
+                         float* lab_bank, int32_t out_h, int32_t out_w, float* scratch_minmax, uint8_t* masks,
+                         float* maps_nchw, void* chain_ws, int64_t chain_ws_bytes, void* stream);
 
 /* Forward-backward cycle consistency of point tracks (test_cfg.cycle_occlusion): every (group, frame t) prediction is
  * re-tracked toward the group's query frame, and the point is visible at t iff the re-track lands within `threshold`
